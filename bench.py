@@ -1,7 +1,7 @@
 """bench.py -- cPongDouble env-steps/s at 84x84x4 observations (BASELINE.json metric), plus the car-racing
 configurations (BASELINE configs 4 and 5) as sub-records of the same JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs-per-gpu E] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs-per-gpu E] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one vec-env step of the whole shard: every env advances 4 game frames and both
 agents' (4, 84, 84) uint8 observations are produced (56 448 B per env-step).  Workload =
@@ -50,6 +50,8 @@ def parse_args():
     ap.add_argument("--car-single-envs", type=int, default=1024)
     ap.add_argument("--car-double-envs", type=int, default=16384)
     ap.add_argument("--no-modes", action="store_true", help="skip the ring / 42x42 / api_step side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed cPongDouble step returned to "
+                    "DIR/<name>.npy (float32 / float64), so that two builds can be compared output for output")
     return ap.parse_args()
 
 
@@ -256,8 +258,32 @@ def P(t):
 
 
 # --------------------------------------------------------------------------- Pong: the headline leg
-def pong_leg(cx, a, N, dim=84, stack_mode="stack", steps=None, warmup=None, with_e2e=True, with_clocks=True):
-    """Device-timed rollout through the C ABI (random actions + game core + rasteriser); returns a record."""
+DUMP_ENVS = 1 << 19          # per-env arrays: 32 B per env with its index, 16.8 MB at most
+DUMP_OBS_ENVS = 128          # both agents' (4, 84, 84) stacks as float32: 28.9 MB
+
+
+def dump_outputs(d, N, obs0, obs1, rew, done, steps_t, real):
+    """The arrays crl_pong_step_state + crl_pong_render_obs wrote, as float32 .npy files under d (under 64 MB in all).
+    Envs are a fixed seeded sample: every env up to DUMP_ENVS for the per-env arrays, DUMP_OBS_ENVS of them for the
+    observations; env_index / obs_env_index name the envs kept."""
+    import numpy as np
+    import torch
+    perm = np.random.default_rng(0).permutation(N)
+    env_idx, obs_idx = np.sort(perm[:DUMP_ENVS]), np.sort(perm[:DUMP_OBS_ENVS])
+
+    def take(t, idx):
+        return t.index_select(0, torch.from_numpy(idx).to(t.device)).to(torch.float32).cpu().numpy()
+    out = {"env_index": env_idx.astype(np.float64), "reward": take(rew, env_idx), "done": take(done, env_idx),
+           "num_steps": take(steps_t, env_idx), "real_reward": take(real, env_idx),
+           "obs_env_index": obs_idx.astype(np.float64), "obs_agent0": take(obs0, obs_idx), "obs_agent1": take(obs1, obs_idx)}
+    os.makedirs(d, exist_ok=True)
+    for name, x in out.items():
+        np.save(os.path.join(d, name + ".npy"), x)
+
+
+def pong_leg(cx, a, N, dim=84, stack_mode="stack", steps=None, warmup=None, with_e2e=True, with_clocks=True, dump_dir=None):
+    """Device-timed rollout through the C ABI (random actions + game core + rasteriser); returns a record.  With
+    dump_dir, the outputs of the last timed step are written there (dump_outputs) before anything else runs."""
     import numpy as np
     from competitive_rl_b200 import _native, make_envs
     torch = cx.torch
@@ -308,6 +334,8 @@ def pong_leg(cx, a, N, dim=84, stack_mode="stack", steps=None, warmup=None, with
         sampler.mark_stop()
     launches = _native.launch_count() - l0
     clocks = sampler.stop() if sampler else None
+    if dump_dir:
+        dump_outputs(dump_dir, N, obs0, obs1, rew, done, steps_t, real)
     ms = e0.elapsed_time(e1)
     raster_ms = sum(x.elapsed_time(y) for x, y in kern_ev) / steps
     rec = {"ms": ms, "raster_ms": raster_ms, "launches": launches, "clocks": clocks, "steps": steps, "warmup": warmup,
@@ -565,7 +593,7 @@ def run_ours(a):
     world, rank = cx.world, cx.rank
     N = a.envs_per_gpu
 
-    r = pong_leg(cx, a, N)
+    r = pong_leg(cx, a, N, dump_dir=a.dump_outputs if rank == 0 else None)
     ms, raster_ms, e2e_s, e2e_obs_s = cx.max_over_ranks([r["ms"], r["raster_ms"], r["e2e_s"], r["e2e_obs_s"]])
     total_envs = N * world
     value = total_envs * a.steps / (ms / 1e3)
@@ -657,7 +685,7 @@ def run_reference(a):
     if rank != 0:
         return
     threads = host_threads()
-    # one "step" here = one vec-step of the bounded sample; K steps timed after W warm-up, and at least 2 s of CPU time
+    # one "step" here = one vec-step of the bounded sample; K steps timed after W warm-up
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import numpy as np
     import pong_oracle
@@ -670,14 +698,10 @@ def run_reference(a):
     acts = rng.integers(0, 3, (64, E, 2)).astype(np.int32)
     for t in range(max(3, a.warmup)):
         v.step(acts[t % 64])
-    steps = 0
+    steps = a.steps
     t0 = time.perf_counter()
-    while True:
-        v.step(acts[steps % 64])
-        steps += 1
-        el = time.perf_counter() - t0
-        if (steps >= a.steps and el >= 2.0) or el > 150:   # bounded above, and never shorter than 2 s of CPU work
-            break
+    for t in range(steps):
+        v.step(acts[t % 64])
     dt = time.perf_counter() - t0
     val = E * steps / dt
     cb = {"value": val, "unit": UNIT, "cores": threads, "kind": "port",
@@ -701,7 +725,11 @@ def run_reference(a):
 
 if __name__ == "__main__":
     args = parse_args()
+    if args.steps < 1:
+        sys.exit("bench.py: --steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            sys.exit("bench.py: --dump-outputs writes the device path's outputs; it does not apply to --impl reference")
         run_reference(args)
     else:
         run_ours(args)

@@ -3,11 +3,11 @@ driving its OWN policy_serving.Policy objects (utils/policy_serving.py:10-66, ne
 reference's cPongDouble vec-env, with serves injected.  Build container only.
 
 The reference's trained checkpoints (resources/pong/checkpoint-*.pkl) are its data and are not vendored, so the network
-opponents of this fixture carry SYNTHETIC weights given by a closed formula (synthetic_state_dict below) that the GPU
+opponents of this fixture carry SYNTHETIC weights given by a closed formula (synthetic_state_dict in tests/conftest.py) that the GPU
 test re-creates: what is pinned is everything around the weights -- the opponent sees obs[1] of the PREVIOUS step, its
 own FrameStackTensor is rolled on every call and never reset on done or on reset_opponent, inputs / 255, greedy argmax,
 action 999 for RULE_BASED, the (N, 1) reward / done shapes -- and the two network definitions themselves.
-(The real WEAK / MEDIUM checkpoints are compared, where the reference tree is present, by tests/test_builtin_policies.py.)
+(tests/test_builtin_policies.py replays this fixture on the CPU oracle to check both network classes without a GPU.)
 
 Two modifications to the reference objects, both forced by the tree itself: get_builtin_agent_names is narrowed (the
 wrapper's constructor builds every agent and asserts on the STRONG / ALPHA_PONG checkpoint files, which the reference
@@ -19,20 +19,12 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
+sys.path.insert(0, os.path.join(os.path.dirname(HERE), "tests"))
 import ref_loader  # noqa: E402
+from conftest import synthetic_state_dict  # noqa: E402
 from pong_oracle import make_serve_table  # noqa: E402
 
 OUT = os.path.join(os.path.dirname(HERE), "tests", "golden")
-
-
-def synthetic_state_dict(model):
-    """parameter k (state_dict order), element i: 0.08 * sin(0.37 * i + k) -- float64 -> float32"""
-    import torch
-    sd = {}
-    for k, (name, p) in enumerate(model.state_dict().items()):
-        i = np.arange(p.numel(), dtype=np.float64)
-        sd[name] = torch.from_numpy((0.08 * np.sin(0.37 * i + k)).astype(np.float32).reshape(tuple(p.shape)))
-    return sd
 
 
 def main():
@@ -64,7 +56,7 @@ def main():
     w.agents["STRONG"] = Policy(BP.single_obs_space, BP.single_act_space, N, "", use_light_model=False)
     w.agent_names.append("STRONG")
     for n in ("WEAK", "MEDIUM", "STRONG"):
-        w.agents[n].model.load_state_dict(synthetic_state_dict(w.agents[n].model))
+        w.agents[n].model.load_state_dict(synthetic_state_dict([(k, p.shape) for k, p in w.agents[n].model.state_dict().items()]))
     schedule = [(0, "RULE_BASED"), (40, "WEAK"), (90, "STRONG"), (130, "WEAK"), (155, "RULE_BASED")]
     rng = np.random.default_rng(77)
     actions = rng.integers(0, 3, (T, N)).astype(np.int32)

@@ -25,3 +25,23 @@ def atlas():
 def load_golden(name):
     import numpy as np
     return np.load(os.path.join(GOLDEN, name + ".npz"))
+
+
+def reference_layout(key):
+    """[(parameter name, shape)] in state-dict order of the reference's network or checkpoint `key`
+    (tests/golden/reference_networks.json, oracle/gen_golden_networks.py)."""
+    import json
+    with open(os.path.join(GOLDEN, "reference_networks.json")) as f:
+        return [(name, tuple(shape)) for name, shape in json.load(f)[key]]
+
+
+def synthetic_state_dict(layout):
+    """The weights of tests/golden/tournament_synth.npz: parameter k of `layout` ([(name, shape)] in state-dict order),
+    element i = float32(0.08 * sin(0.37 * i + k))."""
+    import numpy as np
+    import torch
+    sd = {}
+    for k, (name, shape) in enumerate(layout):
+        i = np.arange(int(np.prod(shape)), dtype=np.float64)
+        sd[name] = torch.from_numpy((0.08 * np.sin(0.37 * i + k)).astype(np.float32).reshape(tuple(shape)))
+    return sd

@@ -1,55 +1,70 @@
-"""Built-in tournament opponents (competitive-rl_b200/builtin_policies.py): the network definitions against the
-reference's own utils/network.py and its shipped checkpoints (CPU, only where /root/reference exists), and the device
-policy against a CPU evaluation of the same weights (GPU)."""
-import importlib.util
-import os
-
+"""Built-in tournament opponents (competitive-rl_b200/builtin_policies.py): the two network definitions against the
+reference's own networks (utils/network.py) and shipped checkpoints -- their state-dict layouts
+(tests/golden/reference_networks.json) and the logits they recorded in tests/golden/tournament_synth.npz (CPU) -- and
+the device policy against a CPU evaluation of the same weights (GPU)."""
 import numpy as np
 import pytest
 
+from conftest import load_golden, reference_layout, synthetic_state_dict
+
 torch = pytest.importorskip("torch")
-
-REF = "/root/reference"
-
-
-def _ref_network():
-    path = os.path.join(REF, "competitive_rl", "utils", "network.py")
-    if not os.path.isfile(path):
-        pytest.skip("reference sources not available")
-    spec = importlib.util.spec_from_file_location("_ref_network", path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)            # the file imports torch only
-    return mod
 
 
 @pytest.mark.parametrize("name", ["weak", "medium"])
-def test_light_network_matches_reference_checkpoint(name):
-    from competitive_rl_b200.builtin_policies import LightActorCritic
-    R = _ref_network()
-    ckpt = os.path.join(REF, "resources", "pong", "checkpoint-%s.pkl" % name)
-    if not os.path.isfile(ckpt):
-        pytest.skip("checkpoint not available")
-    state = torch.load(ckpt, map_location="cpu", weights_only=False)["model"]
-    ours, ref = LightActorCritic((4, 42, 42), 3), R.LightActorCritic((4, 42, 42), 3)
-    ours.load_state_dict(state, strict=True)
-    ref.load_state_dict(state, strict=True)
-    x = torch.from_numpy(np.random.default_rng(0).integers(0, 256, (64, 4, 42, 42)).astype(np.float32))
+def test_light_network_matches_reference_checkpoint(name, tmp_path):
+    """A checkpoint with the layout of the reference's checkpoint-<name>.pkl (its "model" state dict: every parameter
+    name and shape) loads strictly into LightActorCritic, and DevicePolicy, which loads the real file the same way,
+    computes exactly what the network computes with those weights."""
+    from competitive_rl_b200.builtin_policies import DevicePolicy, LightActorCritic
+    sd = synthetic_state_dict(reference_layout("checkpoint-%s.pkl" % name))
+    ours = LightActorCritic((4, 42, 42), 3)
+    ours.load_state_dict(sd, strict=True)
+    path = str(tmp_path / ("checkpoint-%s.pkl" % name))
+    torch.save({"model": sd, "optimizer": {}}, path)
+    pol = DevicePolicy(64, path, use_light_model=True, device="cpu")
+    x = torch.from_numpy(np.random.default_rng(0).integers(0, 256, (64, 4, 1, 42, 42)).astype(np.float32))
+    for k in range(4):                           # four frames fill the policy's stack
+        got = pol.logits(x[:, k])
     with torch.no_grad():
-        lo, vo = ours(x)
-        lr, vr = ref(x)
-    assert torch.equal(lo, lr) and torch.equal(vo, vr)
+        want = ours(x[:, :, 0])[0]
+    assert torch.equal(got, want)
 
 
-def test_full_network_matches_reference_definition():
-    from competitive_rl_b200.builtin_policies import ActorCritic
-    R = _ref_network()
-    torch.manual_seed(0)
-    ref = R.ActorCritic((4, 42, 42), 3)
-    ours = ActorCritic((4, 42, 42), 3)
-    ours.load_state_dict(ref.state_dict(), strict=True)          # same parameter names and shapes
-    x = torch.from_numpy(np.random.default_rng(1).integers(0, 256, (16, 4, 42, 42)).astype(np.float32))
-    with torch.no_grad():
-        assert torch.equal(ours(x)[0], ref(x)[0]) and torch.equal(ours(x)[1], ref(x)[1])
+def test_full_network_matches_reference_definition(atlas):
+    """Replays the fixture's rollout on the CPU oracle (bit-exact to the reference's frames, checked on agent 0's
+    observation every step) with the recorded opponent actions, and feeds the opponent's observations to LightActorCritic
+    (WEAK) and ActorCritic (STRONG).  Their weights are the fixture's synthetic ones, built on the reference networks'
+    own state-dict layouts and loaded strictly, so every parameter name, shape and the parameter order are pinned.
+    WEAK's logits equal the recorded ones bit for bit; STRONG's 11x11x32 convolution sums in a library-chosen order, so
+    its logits are held to a few fp32 ulps."""
+    from competitive_rl_b200.builtin_policies import DevicePolicy
+    from pong_oracle import PongOracleVec
+    g = load_golden("tournament_synth")
+    T, N = g["actions"].shape
+    pols = {}
+    for name, light in (("WEAK", True), ("STRONG", False)):
+        pols[name] = DevicePolicy(N, "", use_light_model=light, device="cpu")
+        layout = reference_layout("LightActorCritic" if light else "ActorCritic")
+        pols[name].model.load_state_dict(synthetic_state_dict(layout), strict=True)
+    orc = PongOracleVec("cPongDouble-v0", N, 42, None, 21, atlas, g["serves"])
+    obs = orc.reset()
+    assert np.array_equal(obs[0], g["obs0"][0])
+    checked = {name: 0 for name in pols}
+    for t in range(T):
+        name = str(g["agent_at"][t])
+        if name in pols:            # the opponent acts on the previous step's obs[1]; its stack rolls only when it acts
+            got = pols[name].logits(torch.from_numpy(obs[1])).numpy()
+            want = g["opp_logits"][t]
+            if name == "WEAK":
+                assert np.array_equal(got, want), (t, got, want)
+            else:
+                assert np.abs(got - want).max() <= 2e-6 * max(1.0, float(np.abs(want).max())), (t, got, want)
+            checked[name] += 1
+        obs, rew, done, _ = orc.step(np.stack([g["actions"][t], g["opp_actions"][t]], axis=1))
+        assert np.array_equal(obs[0], g["obs0"][t + 1]) and np.array_equal(rew[:, :1], g["rew"][t]), t
+        assert np.array_equal(done, g["done"][t][:, 0]), t
+    orc.close()
+    assert checked == {"WEAK": 75, "STRONG": 40}
 
 
 def test_agent_names_follow_available_checkpoints(tmp_path):

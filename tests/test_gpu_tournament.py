@@ -11,18 +11,10 @@ reset_opponent; inputs / 255; argmax."""
 import numpy as np
 import pytest
 
-from conftest import load_golden
+from conftest import load_golden, reference_layout, synthetic_state_dict
 
 torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
-
-
-def synthetic_state_dict(model):
-    sd = {}
-    for k, (name, p) in enumerate(model.state_dict().items()):
-        i = np.arange(p.numel(), dtype=np.float64)
-        sd[name] = torch.from_numpy((0.08 * np.sin(0.37 * i + k)).astype(np.float32).reshape(tuple(p.shape)))
-    return sd
 
 
 class CheckedOpponent(object):
@@ -55,7 +47,8 @@ def test_tournament_replays_reference_rollout():
     checked = {}
     for name, light in (("WEAK", True), ("STRONG", False)):
         pol = DevicePolicy(N, "", use_light_model=light, device=env.env.device)
-        pol.model.load_state_dict(synthetic_state_dict(pol.model))
+        pol.model.load_state_dict(synthetic_state_dict(reference_layout("LightActorCritic" if light else "ActorCritic")),
+                                  strict=True)
         checked[name] = CheckedOpponent(pol, g)
         env.agents[name] = checked[name]
         if name not in env.agent_names:
