@@ -24,6 +24,7 @@ EXPORTS = [
     "crl_car_step", "crl_car_step_state", "crl_car_render_obs", "crl_car_get_state", "crl_car_get_track",
     "crl_car_random_actions", "crl_car_get_stats", "crl_car_get_contacts", "crl_car_check",
     "crl_car_seed", "crl_car_step_host", "crl_car_set_elapsed", "crl_car_set_state", "crl_car_ring_phase", "crl_car_render_state", "crl_car_set_obs_rotation",
+    "crl_obs_alloc", "crl_obs_free",
 ]
 
 
@@ -117,6 +118,8 @@ def load():
     L.crl_pong_render_obs_f32.argtypes = [vp, i32, vp, vp, vp, vp]
     L.crl_pong_reset_state.argtypes = [vp, vp]
     L.crl_pong_get_stats.argtypes = [vp, vp, vp]
+    L.crl_obs_alloc.argtypes = [i32, ctypes.c_size_t, ctypes.POINTER(vp), ctypes.POINTER(i32)]
+    L.crl_obs_free.argtypes = [vp]
     L.crl_car_create.argtypes = [ctypes.POINTER(CarConfig), ctypes.POINTER(vp)]
     L.crl_car_destroy.argtypes = [vp]
     L.crl_car_load_glyphs.argtypes = [vp, vp, ctypes.c_size_t, vp]

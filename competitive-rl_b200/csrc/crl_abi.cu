@@ -7,7 +7,11 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <cuda.h>
+
 #include <atomic>
+#include <mutex>
+#include <unordered_map>
 #include <vector>
 
 #include "../../include/crl_b200.h"
@@ -489,6 +493,140 @@ int crl_pong_check(crl_pong* h, void* stream) {
     }
     if (flag & 2) return fail(CRL_E_INVALID, "an action outside {0, 1, 2} (cPongDouble: or 999) was passed to step; it was played as 1 (stay)");
     if (flag & 1) return fail(CRL_E_SERVES, "injected serve table exhausted");
+    return CRL_OK;
+}
+
+// ---- observation buffers in compressible memory (crl_obs_alloc / crl_obs_free) ----
+// The driver calls come through cudaGetDriverEntryPointByVersion, so the library has no link dependency on libcuda.
+struct ObsDriver {
+    decltype(&::cuMemCreate) create = nullptr;
+    decltype(&::cuMemRelease) release = nullptr;
+    decltype(&::cuMemGetAllocationGranularity) granularity = nullptr;
+    decltype(&::cuMemGetAllocationPropertiesFromHandle) properties = nullptr;
+    decltype(&::cuMemAddressReserve) reserve = nullptr;
+    decltype(&::cuMemAddressFree) address_free = nullptr;
+    decltype(&::cuMemMap) map = nullptr;
+    decltype(&::cuMemUnmap) unmap = nullptr;
+    decltype(&::cuMemSetAccess) set_access = nullptr;
+    bool ok = false;
+};
+
+static const ObsDriver& obs_driver() {
+    static const ObsDriver d = [] {
+        ObsDriver r;
+        auto get = [](const char* name, auto& fn) {
+            void* p = nullptr;
+            cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+            if (cudaGetDriverEntryPointByVersion(name, &p, 12000, cudaEnableDefault, &q) != cudaSuccess ||
+                q != cudaDriverEntryPointSuccess)
+                return false;
+            fn = reinterpret_cast<std::remove_reference_t<decltype(fn)>>(p);
+            return p != nullptr;
+        };
+        r.ok = get("cuMemCreate", r.create) && get("cuMemRelease", r.release) &&
+               get("cuMemGetAllocationGranularity", r.granularity) &&
+               get("cuMemGetAllocationPropertiesFromHandle", r.properties) && get("cuMemAddressReserve", r.reserve) &&
+               get("cuMemAddressFree", r.address_free) && get("cuMemMap", r.map) && get("cuMemUnmap", r.unmap) &&
+               get("cuMemSetAccess", r.set_access);
+        return r;
+    }();
+    return d;
+}
+
+struct ObsAlloc {
+    int device;
+    size_t bytes;   // mapped size (VMM) or 0 (cudaMalloc)
+};
+static std::mutex g_obs_mu;
+static std::unordered_map<void*, ObsAlloc> g_obs;
+
+// A compressible VMM mapping of `bytes` on `device`, or nullptr when the driver does not provide one.
+static void* obs_map_compressible(int device, size_t bytes, size_t* mapped, int32_t* compressed) {
+    const ObsDriver& d = obs_driver();
+    if (!d.ok) return nullptr;
+    CUmemAllocationProp prop;
+    memset(&prop, 0, sizeof prop);
+    prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    prop.location.id = device;
+    prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+    size_t g = 0;
+    if (d.granularity(&g, &prop, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED) != CUDA_SUCCESS || g == 0) return nullptr;
+    const size_t sz = (bytes + g - 1) / g * g;
+    CUmemGenericAllocationHandle h;
+    if (d.create(&h, sz, &prop, 0) != CUDA_SUCCESS) return nullptr;
+    CUmemAllocationProp got;
+    memset(&got, 0, sizeof got);
+    CUdeviceptr va = 0;
+    CUmemAccessDesc acc;
+    memset(&acc, 0, sizeof acc);
+    acc.location = prop.location;
+    acc.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+    if (d.properties(&got, h) != CUDA_SUCCESS || d.reserve(&va, sz, g, 0, 0) != CUDA_SUCCESS) {
+        d.release(h);
+        return nullptr;
+    }
+    if (d.map(va, sz, 0, h, 0) != CUDA_SUCCESS) {
+        d.address_free(va, sz);
+        d.release(h);
+        return nullptr;
+    }
+    d.release(h);   // the mapping keeps the memory until it is unmapped
+    if (d.set_access(va, sz, &acc, 1) != CUDA_SUCCESS) {
+        d.unmap(va, sz);
+        d.address_free(va, sz);
+        return nullptr;
+    }
+    *mapped = sz;
+    // the driver may grant an ordinary allocation (for instance when the device's compression resources are used up)
+    *compressed = got.allocFlags.compressionType == CU_MEM_ALLOCATION_COMP_GENERIC ? 1 : 0;
+    return reinterpret_cast<void*>(va);
+}
+
+int crl_obs_alloc(int32_t device, size_t bytes, void** ptr, int32_t* compressed) {
+    if (!ptr || !compressed || bytes == 0) return fail(CRL_E_INVALID, "crl_obs_alloc: null output pointer or zero bytes");
+    *ptr = nullptr;
+    *compressed = 0;
+    CrlDeviceGuard guard(device);
+    CUDA_TRY(guard.err);
+    int supported = 0;
+    CUDA_TRY(cudaDeviceGetAttribute(&supported, (cudaDeviceAttr)CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, device));
+    void* p = nullptr;
+    size_t mapped = 0;
+    if (supported) p = obs_map_compressible(device, bytes, &mapped, compressed);
+    if (p == nullptr) {
+        *compressed = 0;
+        CUDA_TRY(cudaMalloc(&p, bytes));
+    }
+    {
+        std::lock_guard<std::mutex> lk(g_obs_mu);
+        g_obs[p] = ObsAlloc{device, mapped};
+    }
+    *ptr = p;
+    return CRL_OK;
+}
+
+int crl_obs_free(void* ptr) {
+    if (!ptr) return CRL_OK;
+    ObsAlloc a;
+    {
+        std::lock_guard<std::mutex> lk(g_obs_mu);
+        auto it = g_obs.find(ptr);
+        if (it == g_obs.end()) return fail(CRL_E_INVALID, "crl_obs_free: %p was not returned by crl_obs_alloc", ptr);
+        a = it->second;
+        g_obs.erase(it);
+    }
+    CrlDeviceGuard guard(a.device);
+    CUDA_TRY(guard.err);
+    if (a.bytes == 0) {
+        CUDA_TRY(cudaFree(ptr));
+        return CRL_OK;
+    }
+    CUDA_TRY(cudaDeviceSynchronize());   // a kernel may still be writing the buffer
+    const ObsDriver& d = obs_driver();
+    CUresult r = d.unmap(reinterpret_cast<CUdeviceptr>(ptr), a.bytes);
+    if (r == CUDA_SUCCESS) r = d.address_free(reinterpret_cast<CUdeviceptr>(ptr), a.bytes);
+    if (r != CUDA_SUCCESS) return fail(CRL_E_CUDA, "crl_obs_free: cuMemUnmap / cuMemAddressFree failed (CUresult %d)", (int)r);
     return CRL_OK;
 }
 

@@ -8,8 +8,10 @@
 #include <c10/cuda/CUDAStream.h>
 #include <torch/extension.h>
 
+#include <algorithm>
 #include <stdexcept>
 #include <string>
+#include <vector>
 
 #include "../../include/crl_b200.h"
 
@@ -250,6 +252,23 @@ struct Car {
     uint64_t raw_handle() const { return (uint64_t)(uintptr_t)h; }
 };
 
+// An uninitialised observation buffer: crl_obs_alloc's memory (compressible where the device grants it) viewed as a tensor
+// that gives the memory back through crl_obs_free when its storage is released; with compressible=False, torch.empty.
+// Returns (tensor, whether the memory is compressible).
+std::pair<at::Tensor, bool> obs_empty(const std::vector<int64_t>& shape, at::ScalarType dtype, int64_t device, bool compressible) {
+    const auto opts = at::TensorOptions().dtype(dtype).device(at::kCUDA, (c10::DeviceIndex)device);
+    if (!compressible) return {at::empty(shape, opts), false};
+    int64_t numel = 1;
+    for (int64_t d : shape) {
+        TORCH_CHECK(d >= 0, "obs_empty: negative dimension");
+        numel *= d;
+    }
+    void* p = nullptr;
+    int32_t compressed = 0;
+    check_rc(crl_obs_alloc((int32_t)device, std::max<size_t>((size_t)numel * c10::elementSize(dtype), 1), &p, &compressed));
+    return {torch::from_blob(p, shape, [](void* q) { crl_obs_free(q); }, opts), compressed != 0};
+}
+
 }  // namespace
 
 PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
@@ -257,6 +276,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
     py::register_exception<CrlError>(m, "CrlError", PyExc_RuntimeError);
     m.def("abi_version", []() { return crl_abi_version(); });
     m.def("launch_count", []() { return crl_launch_count(); });
+    m.def("obs_empty", &obs_empty, py::arg("shape"), py::arg("dtype"), py::arg("device"), py::arg("compressible") = true);
     py::class_<Pong>(m, "Pong")
         .def(py::init<int64_t, int64_t, int64_t, int64_t, int64_t, int64_t, int64_t, bool, uint64_t, int64_t>())
         .def("close", &Pong::close)

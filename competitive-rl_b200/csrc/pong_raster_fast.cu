@@ -36,9 +36,13 @@ template <> struct alignas(16) TapEnt<3> { uint32_t meta; float w[3]; };
 template <> struct alignas(16) TapEnt<5> { uint32_t meta; float w[5]; uint32_t pad[2]; };
 // meta: src0 | tapmask<<8 | (y only) mask of taps lying in the white border rows <<16
 
+#ifndef CRL_FAST84_CTAS
+#define CRL_FAST84_CTAS 3    // resident CTAs per SM of the 84x84 kernel: see pong_raster_init
+#endif
+// CTAS: resident CTAs per SM the kernel is compiled for (__launch_bounds__) and launched with
 template <int DIM> struct FastCfg;
-template <> struct FastCfg<84> { static constexpr int TAPS = 3, VEC = 16; };
-template <> struct FastCfg<42> { static constexpr int TAPS = 5, VEC = 4; };
+template <> struct FastCfg<84> { static constexpr int TAPS = 3, VEC = 16, CTAS = CRL_FAST84_CTAS; };
+template <> struct FastCfg<42> { static constexpr int TAPS = 5, VEC = 4, CTAS = 3; };
 
 constexpr int FAST_WARPS = 8;
 constexpr int FIRST_PAD = 224;   // y_first/y_last padded to a multiple of 16 bytes
@@ -182,8 +186,10 @@ __device__ __forceinline__ uint8_t eval_text_pixel(const AreaTabs* __restrict__ 
     return (uint8_t)min(max(__float2int_rn(sum), 0), 255);
 }
 
-template <int DIM>
-__global__ void __launch_bounds__(FAST_WARPS * 32, 3)
+// RING: the ring observation mode (crl_pong_config::stack_mode 1).  A template parameter, so that the plain-stack
+// instantiation carries none of the ring's run-time branches and state in its hot loop.
+template <int DIM, bool RING>
+__global__ void __launch_bounds__(FAST_WARPS * 32, FastCfg<DIM>::CTAS)
 pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* __restrict__ obs0,
                         uint8_t* __restrict__ obs1, const FastTabs<DIM>* __restrict__ gtabs) {
     constexpr int TAPS = FastCfg<DIM>::TAPS, VEC = FastCfg<DIM>::VEC;
@@ -234,8 +240,8 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
     // makes the counter itself the bottleneck (2.7 TB/s in the probe).
     const long long n_stacks = (long long)p.n * p.n_agents;
     // frames a stack writes: c (plain stack), or the newest frame twice (ring; all 2c slots only after a reset)
-    const int per_ticket = max(1, 4 / (p.ring ? 2 : p.c));
-    const int out_slots = p.ring ? 2 * p.c : p.c;
+    const int per_ticket = max(1, 4 / (RING ? 2 : p.c));
+    const int out_slots = RING ? 2 * p.c : p.c;
     long long s = 0, s_end = 0;
     for (;;) {
         if (s >= s_end) {
@@ -251,7 +257,7 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
         FrameSpec my_spec = make_uint4(0u, 0u, 0u, 0u);
         if (lane < p.c) my_spec = hist[(size_t)lane * p.n + env];
         // ring: only the newest frame is new, unless the env was just reset (its whole history changed)
-        const int first_slot = (p.ring && !p.fill_all && !p.last_done[env]) ? p.c - 1 : 0;
+        const int first_slot = (RING && !p.fill_all && !p.last_done[env]) ? p.c - 1 : 0;
 
         for (int slot = first_slot; slot < p.c; ++slot) {
             FrameSpec f;
@@ -263,7 +269,7 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
             // c slots before or after it, whichever exists (the newest frame: ring_phase + c and ring_phase)
             uint8_t* out8 = out_stack + (size_t)slot * DD;
             uint8_t* out8b = nullptr;
-            if (p.ring) {
+            if (RING) {
                 const int pos = p.ring_phase + 1 + slot;
                 out8 = out_stack + (size_t)pos * DD;
                 out8b = out_stack + (size_t)(pos >= p.c ? pos - p.c : pos + p.c) * DD;
@@ -293,7 +299,7 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
                 memset(&z, 0, sizeof z);
                 V* out = reinterpret_cast<V*>(out8);
                 for (int k = lane; k < NCH; k += 32) st_stream(out + k, z);
-                if (out8b != nullptr) {
+                if (RING) {
                     V* outb = reinterpret_cast<V*>(out8b);
                     for (int k = lane; k < NCH; k += 32) st_stream(outb + k, z);
                 }
@@ -441,13 +447,13 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
                 __syncwarp();
                 if (lane == 0) {
                     bulk_store(out8, sm8, DD);
-                    if (out8b != nullptr) bulk_store(out8b, sm8, DD);
+                    if (RING) bulk_store(out8b, sm8, DD);
                 }
                 pending = true;
             } else {
                 __syncwarp();
                 V* out = reinterpret_cast<V*>(out8);
-                if (out8b == nullptr) {
+                if (!RING) {
 #pragma unroll
                     for (int j = 0; j < (NCH + 31) / 32; ++j)
                         if ((j + 1) * 32 <= NCH || lane + 32 * j < NCH) st_stream(out + lane + 32 * j, sm[lane + 32 * j]);
@@ -913,20 +919,23 @@ cudaError_t pong_raster_init(int g_grid[3]) {
     int dev = 0, sms = 0, nb = 0;
     if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
     if ((e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(pong_raster_fast_kernel<84>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)fast_smem_bytes<84>());
+    // both instantiations (plain stack, ring) of a size share the shared-memory size and the register budget
+    // (__launch_bounds__), so one occupancy query per size sizes the grid for both
+    const void* fast[2][2] = {{(const void*)pong_raster_fast_kernel<84, false>, (const void*)pong_raster_fast_kernel<84, true>},
+                              {(const void*)pong_raster_fast_kernel<42, false>, (const void*)pong_raster_fast_kernel<42, true>}};
+    const int smem[2] = {(int)fast_smem_bytes<84>(), (int)fast_smem_bytes<42>()};
+    for (int d = 0; d < 2; ++d)
+        for (int r = 0; r < 2; ++r)
+            if ((e = cudaFuncSetAttribute(fast[d][r], cudaFuncAttributeMaxDynamicSharedMemorySize, smem[d])) != cudaSuccess) return e;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, pong_raster_fast_kernel<84, false>, FAST_WARPS * 32, smem[0]);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(pong_raster_fast_kernel<42>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)fast_smem_bytes<42>());
-    if (e != cudaSuccess) return e;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, pong_raster_fast_kernel<84>, FAST_WARPS * 32,
-                                                      fast_smem_bytes<84>());
-    if (e != cudaSuccess) return e;
-    // 84x84 is bound by the DRAM write path, which prefers fewer concurrent write streams: 2 CTAs (16 warps) per SM
-    // measured 0.523 ms per launch against 0.535 ms with the 3 that fit (1 CTA: 0.621 ms)
-    g_grid[0] = sms * max(min(nb, 2), 1);
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, pong_raster_fast_kernel<42>, FAST_WARPS * 32,
-                                                      fast_smem_bytes<42>());
+    // 84x84: FastCfg<84>::CTAS per SM.  With uncompressed observation buffers the DRAM write path preferred fewer
+    // concurrent write streams (2 CTAs: 0.523 ms per launch, 3: 0.535 ms).  With compressible buffers DRAM is no longer
+    // the limit and the kernel gains from the warps that hide its own latency: 3 CTAs 0.4886 ms against 0.4963 ms with 2
+    // (B200, 65 536 envs, stack mode; the ring instantiation spills 8 bytes at 3 and lost 2 %, 192.5 against 196.2 M
+    // env-steps/s, less than the headline gains)
+    g_grid[0] = sms * max(min(nb, FastCfg<84>::CTAS), 1);
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, pong_raster_fast_kernel<42, false>, FAST_WARPS * 32, smem[1]);
     if (e != cudaSuccess) return e;
     g_grid[1] = sms * max(nb, 1);
     e = cudaFuncSetAttribute(pong_raster_quad_kernel<42>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)quad_smem_bytes<42>());
@@ -948,8 +957,9 @@ cudaError_t launch_pong_raster(const PongDev& p, const FrameSpec* hist, uint8_t*
     if (me != cudaSuccess) return me;
     if (p.dim == 84) {
         const unsigned grid = (unsigned)min((long long)p.raster_grid[0], want);
-        pong_raster_fast_kernel<84><<<grid, FAST_WARPS * 32, fast_smem_bytes<84>(), s>>>(
-            p, hist, obs0, obs1, reinterpret_cast<const FastTabs<84>*>(p.fast_tabs));
+        const FastTabs<84>* tabs = reinterpret_cast<const FastTabs<84>*>(p.fast_tabs);
+        if (p.ring) pong_raster_fast_kernel<84, true><<<grid, FAST_WARPS * 32, fast_smem_bytes<84>(), s>>>(p, hist, obs0, obs1, tabs);
+        else pong_raster_fast_kernel<84, false><<<grid, FAST_WARPS * 32, fast_smem_bytes<84>(), s>>>(p, hist, obs0, obs1, tabs);
     } else if (p.quad_ok && !p.ring && (long long)p.n * p.c * p.n_agents < (1LL << 31)) {
         const long long quads = (((long long)p.n * p.c + 3) / 4) * p.n_agents;
         const unsigned grid = (unsigned)min((long long)p.raster_grid[2], (quads + 4 * QUAD_WARPS - 1) / (4 * QUAD_WARPS));
@@ -957,8 +967,9 @@ cudaError_t launch_pong_raster(const PongDev& p, const FrameSpec* hist, uint8_t*
             p, hist, obs0, obs1, reinterpret_cast<const FastTabs<42>*>(p.fast_tabs));
     } else {
         const unsigned grid = (unsigned)min((long long)p.raster_grid[1], want);
-        pong_raster_fast_kernel<42><<<grid, FAST_WARPS * 32, fast_smem_bytes<42>(), s>>>(
-            p, hist, obs0, obs1, reinterpret_cast<const FastTabs<42>*>(p.fast_tabs));
+        const FastTabs<42>* tabs = reinterpret_cast<const FastTabs<42>*>(p.fast_tabs);
+        if (p.ring) pong_raster_fast_kernel<42, true><<<grid, FAST_WARPS * 32, fast_smem_bytes<42>(), s>>>(p, hist, obs0, obs1, tabs);
+        else pong_raster_fast_kernel<42, false><<<grid, FAST_WARPS * 32, fast_smem_bytes<42>(), s>>>(p, hist, obs0, obs1, tabs);
     }
     return cudaGetLastError();
 }

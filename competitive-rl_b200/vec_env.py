@@ -284,13 +284,23 @@ class CudaPongVecEnv(VecEnv):
 
         dev = self.device
         shape = (n, self.c, self.dim, self.dim)
+        # Observation stacks and rings live in compressible memory where the device grants it (crl_obs_alloc): the frames
+        # are mostly constant runs, so the rasteriser's writes reach DRAM in fewer bytes.  obs_compressed says whether
+        # every one of them was granted compressible memory.
+        self.obs_compressed = True
+
+        def obs_buffer(shape, dtype):
+            t, compressed = ext.obs_empty(list(shape), dtype, dev.index)
+            self.obs_compressed = self.obs_compressed and compressed
+            return t
+
         # the ring (one per agent) carries the frame history, so there is exactly one; the small outputs still rotate
-        self._ring = [torch.empty((n, 2 * self.c, self.dim, self.dim), dtype=torch.uint8, device=dev)
+        self._ring = [obs_buffer((n, 2 * self.c, self.dim, self.dim), torch.uint8)
                       for _ in range(self.n_agents)] if self.ring else None
         self._sets = []
         for _ in range(max(1, int(n_buffers))):
             self._sets.append(dict(
-                obs=None if self.ring else [torch.empty(shape, dtype=torch.float32 if self.f32 else torch.uint8, device=dev)
+                obs=None if self.ring else [obs_buffer(shape, torch.float32 if self.f32 else torch.uint8)
                                             for _ in range(self.n_agents)],
                 rew=torch.zeros((n, 2), dtype=torch.float32, device=dev),
                 real=torch.zeros((n, 2), dtype=torch.float32, device=dev),
@@ -443,6 +453,8 @@ class CudaPongVecEnv(VecEnv):
                 torch.cuda.synchronize(self.device)
             self._impl.close()
             self._h = None
+            # the env's references to its buffers: the observation memory goes back once the caller's are gone too
+            self._ring, self._sets, self._obs = None, [], None
         self.closed = True
 
     def __del__(self):

@@ -171,6 +171,17 @@ int crl_pong_get_stats(crl_pong* h, uint64_t* stats_host, void* stream);
 uint64_t crl_launch_count(void);
 int crl_pong_check(crl_pong* h, void* stream);
 
+/* Observation buffers.  crl_obs_alloc allocates `bytes` of device memory on `device` for the observations the
+ * rasterisers write (crl_pong_*: obs0_dev / obs1_dev, and the rings of stack_mode 1).  Where the device supports generic
+ * memory compression (CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED) the memory is a compressible mapping
+ * (cuMemCreate with CU_MEM_ALLOCATION_COMP_GENERIC, size rounded up to the allocation granularity): Pong frames are
+ * mostly constant runs, which the memory system then moves to and from DRAM in fewer bytes.  Contents and addressing
+ * are those of any device memory.  *compressed is 1 when the driver granted compressible memory, 0 when the buffer is
+ * an ordinary allocation (no support, or the request was refused).  crl_obs_free synchronises the device, then
+ * releases a buffer crl_obs_alloc returned (NULL: no-op). */
+int crl_obs_alloc(int32_t device, size_t bytes, void** ptr, int32_t* compressed);
+int crl_obs_free(void* ptr);
+
 /* ======================================================================================
  * cCarRacing-v0 / cCarRacingDouble-v0
  * Replaces the env stack built by make_car_racing / make_car_racing_double

@@ -12,7 +12,8 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "competitive-rl_b200", "libcrl_b200.so")
-KERNELS = ["pong_step_kernel", "pong_raster_fast_kernelILi84", "pong_raster_fast_kernelILi42", "pong_raster_quad_kernelILi42",
+KERNELS = ["pong_step_kernel", "pong_raster_fast_kernelILi84ELb0", "pong_raster_fast_kernelILi84ELb1",
+           "pong_raster_fast_kernelILi42ELb0", "pong_raster_fast_kernelILi42ELb1", "pong_raster_quad_kernelILi42",
            "car_step_kernel", "car_sensor_kernel", "car_collide_kernel", "car_render_kernel", "car_frame_setup_kernel", "car_frame_aux_kernel",
            "car_stack_shift_kernel", "car_reset_kernel", "car_pregen_kernel"]
 
@@ -55,7 +56,7 @@ def main():
             if op.split(".")[0] in ("LDG", "STG", "LDS", "STS", "LDL", "STL", "ATOMG", "ATOMS", "RED", "LDC", "UBLKCP", "UTMASTG", "CCTL"):
                 mem[op] += 1
         n_inst = sum(ops.values())
-        short = key.replace("ILi", "_")
+        short = key.replace("ILi", "_").replace("ELb0", "").replace("ELb1", "_ring")   # <DIM, RING> of the fast kernel
         fn = "%s_sass_%s.txt" % (prefix, short)
         head = ["# %s" % name, "# resources: %s" % usage.get(name, "?"), "# instructions: %d" % n_inst,
                 "# opcode histogram: " + ", ".join("%s %d" % kv for kv in ops.most_common(28)),
