@@ -20,6 +20,7 @@ EXPORTS = [
     "crl_pong_render_obs", "crl_pong_render_obs_generic", "crl_pong_terminal_obs", "crl_pong_step_host",
     "crl_pong_get_state", "crl_pong_set_state", "crl_pong_render_raw", "crl_pong_random_actions",
     "crl_launch_count", "crl_pong_check", "crl_pong_get_stats", "crl_pong_ring_phase", "crl_pong_render_obs_f32", "crl_pong_reset_state",
+    "crl_pong_set_obs_buffers", "crl_pong_forget_obs",
     "crl_car_create", "crl_car_destroy", "crl_car_load_glyphs", "crl_car_inject_tracks", "crl_car_load_tracks", "crl_car_reset",
     "crl_car_step", "crl_car_step_state", "crl_car_render_obs", "crl_car_get_state", "crl_car_get_track",
     "crl_car_random_actions", "crl_car_get_stats", "crl_car_get_contacts", "crl_car_check",
@@ -118,6 +119,8 @@ def load():
     L.crl_pong_render_obs_f32.argtypes = [vp, i32, vp, vp, vp, vp]
     L.crl_pong_reset_state.argtypes = [vp, vp]
     L.crl_pong_get_stats.argtypes = [vp, vp, vp]
+    L.crl_pong_set_obs_buffers.argtypes = [vp, ctypes.POINTER(vp), ctypes.POINTER(vp), i32, vp]
+    L.crl_pong_forget_obs.argtypes = [vp]
     L.crl_obs_alloc.argtypes = [i32, ctypes.c_size_t, ctypes.POINTER(vp), ctypes.POINTER(i32)]
     L.crl_obs_free.argtypes = [vp]
     L.crl_car_create.argtypes = [ctypes.POINTER(CarConfig), ctypes.POINTER(vp)]

@@ -73,7 +73,30 @@ struct crl_pong {
     // crl_pong_step_host: the small results go back to the host on a side stream while the rasteriser runs
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_state = nullptr, ev_copied = nullptr;
+    // crl_pong_set_obs_buffers: observation buffers whose contents the library tracks.  shown ([agent][c][n] FrameSpecs per
+    // set) describes what the set's buffers hold while `valid`; renders into a valid set store only what changed.
+    struct ObsSet {
+        uint8_t* obs[2];
+        FrameSpec* shown;
+        bool valid;
+    };
+    std::vector<ObsSet> sets;
+    FrameSpec* shown_dev = nullptr;
+    bool full_obs = false;      // CRL_PONG_FULL_OBS: every render stores whole stacks
 };
+
+static size_t obs_bytes(const crl_pong* h) {
+    return (size_t)h->dev.n * (h->dev.ring ? 2 * h->dev.c : h->dev.c) * h->dev.dim * h->dev.dim;
+}
+
+// [p, p + bytes) was written by something other than a tracked render: the sets it overlaps no longer know their contents
+static void obs_written(crl_pong* h, const void* p, size_t bytes) {
+    if (!p) return;
+    const uintptr_t a = (uintptr_t)p, b = a + bytes, ob = obs_bytes(h);
+    for (auto& st : h->sets)
+        for (int k = 0; k < h->dev.n_agents; ++k)
+            if (a < (uintptr_t)st.obs[k] + ob && (uintptr_t)st.obs[k] < b) st.valid = false;
+}
 
 // OpenCV computeResizeAreaTab (SURVEY.md A.2): scale and cell in double, alpha stored as float.
 static bool build_axis(int ssize, int dsize, uint8_t* src0, uint8_t* cnt, float (*alpha)[MAX_TAPS], uint8_t* first,
@@ -143,6 +166,7 @@ int crl_pong_destroy(crl_pong* h) {
     if (!h) return CRL_OK;
     CrlDeviceGuard guard(h->cfg.device);
     for (void* p : h->allocs) cudaFree(p);
+    if (h->shown_dev) cudaFree(h->shown_dev);
     if (h->ev_state) cudaEventDestroy(h->ev_state);
     if (h->ev_copied) cudaEventDestroy(h->ev_copied);
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
@@ -228,6 +252,7 @@ int crl_pong_create(const crl_pong_config* cfg, crl_pong** out) {
             g_launches += 1;
             d.fast_tabs = h->fast_tabs_dev;
             d.quad_ok = (pong_quad_ok(tabs) && getenv("CRL_PONG_NO_QUAD") == nullptr) ? 1 : 0;
+            h->full_obs = getenv("CRL_PONG_FULL_OBS") != nullptr;   // A/B switch: no incremental stacks
         }
     }
     d.tabs = h->tabs_dev;
@@ -296,6 +321,7 @@ int crl_pong_load_atlas(crl_pong* h, const uint8_t* strips_host, size_t bytes, v
         h->dev.text_w0 = w0; h->dev.text_w1 = w1;
     }
     h->atlas_loaded = true;
+    for (auto& st : h->sets) st.valid = false;   // every frame may look different now
     return CRL_OK;
 }
 
@@ -332,7 +358,67 @@ int crl_pong_render_obs(crl_pong* h, uint8_t* obs0_dev, uint8_t* obs1_dev, void*
     if (int r = need_ready(h, true)) return r;
     if (!obs0_dev || (h->dev.n_agents == 2 && !obs1_dev)) return fail(CRL_E_INVALID, "null observation buffer");
     if (h->dev.n_agents == 1) obs1_dev = obs0_dev;
-    LAUNCH(launch_pong_raster(h->dev, h->dev.hist, obs0_dev, obs1_dev, (cudaStream_t)stream));
+    cudaStream_t s = (cudaStream_t)stream;
+    crl_pong::ObsSet* set = nullptr;
+    for (auto& st : h->sets)
+        if (st.obs[0] == obs0_dev && (h->dev.n_agents == 1 || st.obs[1] == obs1_dev)) set = &st;
+    const bool incremental = !h->full_obs && pong_raster_incremental_ok(h->dev, obs0_dev, obs1_dev);
+    if (set && set->valid && incremental) {
+        LAUNCH(launch_pong_raster(h->dev, h->dev.hist, obs0_dev, obs1_dev, set->shown, s));
+        return CRL_OK;
+    }
+    LAUNCH(launch_pong_raster(h->dev, h->dev.hist, obs0_dev, obs1_dev, nullptr, s));
+    if (!set) {
+        obs_written(h, obs0_dev, obs_bytes(h));
+        obs_written(h, obs1_dev, obs_bytes(h));
+    } else if (incremental) {   // the set now holds hist: later renders into it can be incremental
+        const size_t per_agent = (size_t)h->dev.c * h->dev.n;
+        for (int k = 0; k < h->dev.n_agents; ++k)
+            CUDA_TRY(cudaMemcpyAsync(set->shown + k * per_agent, h->dev.hist, per_agent * sizeof(FrameSpec),
+                                     cudaMemcpyDeviceToDevice, s));
+        set->valid = true;
+    } else {
+        set->valid = false;
+    }
+    return CRL_OK;
+}
+
+int crl_pong_set_obs_buffers(crl_pong* h, uint8_t* const* obs0_devs_host, uint8_t* const* obs1_devs_host, int32_t count,
+                             void* stream) {
+    CHECK_HANDLE(h);
+    const int na = h->dev.n_agents;
+    if (count != 0) {
+        if (h->dev.ring) return fail(CRL_E_STATE, "stack_mode ring keeps its own frames: there are no buffer sets to register");
+        if (count < 0 || count > CRL_PONG_MAX_OBS_SETS || !obs0_devs_host || (na == 2 && !obs1_devs_host))
+            return fail(CRL_E_INVALID, "need 1 .. %d buffer sets (and obs1 buffers for cPongDouble), got %d",
+                        CRL_PONG_MAX_OBS_SETS, count);
+        std::vector<uint8_t*> all;
+        for (int i = 0; i < count; ++i)
+            for (int k = 0; k < na; ++k) {
+                uint8_t* b = k ? obs1_devs_host[i] : obs0_devs_host[i];
+                if (!b) return fail(CRL_E_INVALID, "null buffer in set %d", i);
+                for (uint8_t* o : all)
+                    if (o == b) return fail(CRL_E_INVALID, "a buffer appears twice in the sets");
+                all.push_back(b);
+            }
+    }
+    CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));   // no render in flight reads the old specs
+    h->sets.clear();
+    if (h->shown_dev) {
+        CUDA_TRY(cudaFree(h->shown_dev));
+        h->shown_dev = nullptr;
+    }
+    if (count == 0) return CRL_OK;
+    const size_t per_set = (size_t)na * h->dev.c * h->dev.n;
+    CUDA_TRY(cudaMalloc(&h->shown_dev, (size_t)count * per_set * sizeof(FrameSpec)));
+    for (int i = 0; i < count; ++i)
+        h->sets.push_back({{obs0_devs_host[i], na == 2 ? obs1_devs_host[i] : obs0_devs_host[i]}, h->shown_dev + i * per_set, false});
+    return CRL_OK;
+}
+
+int crl_pong_forget_obs(crl_pong* h) {
+    if (!h) return fail(CRL_E_INVALID, "null handle");
+    for (auto& st : h->sets) st.valid = false;
     return CRL_OK;
 }
 
@@ -341,6 +427,8 @@ int crl_pong_render_obs_generic(crl_pong* h, uint8_t* obs0_dev, uint8_t* obs1_de
     if (int r = need_ready(h, true)) return r;
     if (!obs0_dev || (h->dev.n_agents == 2 && !obs1_dev)) return fail(CRL_E_INVALID, "null observation buffer");
     LAUNCH(launch_pong_raster_generic(h->dev, h->dev.hist, nullptr, h->dev.ring, obs0_dev, obs1_dev, (cudaStream_t)stream));
+    obs_written(h, obs0_dev, obs_bytes(h));
+    obs_written(h, obs1_dev, obs_bytes(h));
     return CRL_OK;
 }
 
@@ -350,6 +438,8 @@ int crl_pong_render_obs_f32(crl_pong* h, int32_t terminal, const uint8_t* only_d
     if (h->dev.ring) return fail(CRL_E_STATE, "float32 observations are plain stacks: create the handle with stack_mode 0");
     if (!obs0_dev || (h->dev.n_agents == 2 && !obs1_dev)) return fail(CRL_E_INVALID, "null observation buffer");
     LAUNCH(launch_pong_raster_f32(h->dev, terminal ? h->dev.term_hist : h->dev.hist, only_done_dev, obs0_dev, obs1_dev, (cudaStream_t)stream));
+    obs_written(h, obs0_dev, 4 * obs_bytes(h));
+    obs_written(h, obs1_dev, 4 * obs_bytes(h));
     return CRL_OK;
 }
 
@@ -398,6 +488,8 @@ int crl_pong_terminal_obs(crl_pong* h, const uint8_t* done_dev, uint8_t* term0_d
     if (int r = need_ready(h, true)) return r;
     if (!done_dev || !term0_dev || (h->dev.n_agents == 2 && !term1_dev)) return fail(CRL_E_INVALID, "null buffer");
     LAUNCH(launch_pong_raster_generic(h->dev, h->dev.term_hist, done_dev, 0, term0_dev, term1_dev, (cudaStream_t)stream));
+    obs_written(h, term0_dev, obs_bytes(h));
+    obs_written(h, term1_dev, obs_bytes(h));
     return CRL_OK;
 }
 

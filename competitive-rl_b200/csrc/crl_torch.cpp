@@ -143,6 +143,16 @@ struct Pong {
                                      opt_dev_ptr<uint8_t>(rgb1, at::kByte, dev(), 210 * 160 * 3, "rgb1"), stream_of(dev())));
     }
     void check() { check_rc(crl_pong_check(handle(), stream_of(dev()))); }
+    // observation buffer sets whose contents the library tracks (crl_pong_set_obs_buffers); empty lists unregister
+    void set_obs_buffers(const std::vector<at::Tensor>& obs0, const std::vector<at::Tensor>& obs1) {
+        TORCH_CHECK(cfg.n_agents == 1 || obs1.size() == obs0.size(), "cPongDouble needs an obs1 buffer per set");
+        std::vector<uint8_t*> p0, p1;
+        for (const at::Tensor& t : obs0) p0.push_back(dev_ptr<uint8_t>(t, at::kByte, dev(), obs_numel, "obs0 buffer of a set"));
+        for (const at::Tensor& t : obs1) p1.push_back(dev_ptr<uint8_t>(t, at::kByte, dev(), obs_numel, "obs1 buffer of a set"));
+        check_rc(crl_pong_set_obs_buffers(handle(), p0.data(), cfg.n_agents == 2 ? p1.data() : nullptr, (int32_t)p0.size(),
+                                          stream_of(dev())));
+    }
+    void forget_obs() { check_rc(crl_pong_forget_obs(handle())); }
     std::vector<uint64_t> stats() {
         std::vector<uint64_t> s(8);
         check_rc(crl_pong_get_stats(handle(), s.data(), stream_of(dev())));
@@ -295,6 +305,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
         .def("set_state", &Pong::set_state)
         .def("render_raw", &Pong::render_raw)
         .def("check", &Pong::check)
+        .def("set_obs_buffers", &Pong::set_obs_buffers)
+        .def("forget_obs", &Pong::forget_obs)
         .def("stats", &Pong::stats)
         .def("raw_handle", &Pong::raw_handle);
     py::class_<Car>(m, "Car")

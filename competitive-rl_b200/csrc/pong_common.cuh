@@ -151,7 +151,11 @@ cudaError_t launch_pong_set_state(const PongDev& p, const double* state, cudaStr
 cudaError_t launch_pong_random_actions(int32_t* actions, int n_values, uint64_t seed, uint64_t step, cudaStream_t s);
 
 cudaError_t launch_pong_build_tables(const PongDev& p, uint8_t* text_tab, uint8_t* tmpl, cudaStream_t s);
-cudaError_t launch_pong_raster(const PongDev& p, const FrameSpec* hist, uint8_t* obs0, uint8_t* obs1, cudaStream_t s);
+// shown != nullptr: incremental 84x84 stack render (pong_raster_incremental_ok must hold): obs* hold the frames shown
+// ([agent][c][n]) describes; afterwards shown = hist
+cudaError_t launch_pong_raster(const PongDev& p, const FrameSpec* hist, uint8_t* obs0, uint8_t* obs1, FrameSpec* shown,
+                               cudaStream_t s);
+bool pong_raster_incremental_ok(const PongDev& p, const void* obs0, const void* obs1);
 // ring = 1: obs* are 2c-slot rings, rewritten completely (terminal observations are always plain stacks: ring = 0)
 cudaError_t launch_pong_raster_generic(const PongDev& p, const FrameSpec* hist, const uint8_t* only_done, int ring,
                                        uint8_t* obs0, uint8_t* obs1, cudaStream_t s);

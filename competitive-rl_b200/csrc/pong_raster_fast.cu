@@ -23,7 +23,9 @@
 //   C. hands the buffer to the TMA engine: one cp.async.bulk shared->global of 7 056 bytes
 //      (fence.proxy.async first), so the drain costs one instruction and overlaps step A of
 //      the next frame.
-// HBM traffic = the observation bytes, written once; ~100 B/env of state are read.
+// HBM traffic = the observation bytes, written once; ~100 B/env of state are read.  Into buffers whose contents the
+// library tracks (crl_pong_set_obs_buffers), the incremental instantiation stores only the 16-byte chunks a frame can
+// have changed since the buffer's last render (INC below).
 // The grid is persistent: SMs x resident CTAs, warps stride over the stacks.
 #include <type_traits>
 
@@ -186,22 +188,100 @@ __device__ __forceinline__ uint8_t eval_text_pixel(const AreaTabs* __restrict__ 
     return (uint8_t)min(max(__float2int_rn(sum), 0), 255);
 }
 
+// ---- incremental stacks (INC): what a frame buffer already holds decides what is stored ----
+// (env, agent) stacks per work ticket of the incremental kernel: its stacks store ~1/20 of the bytes, so one atomic per
+// stack would make the counter a bottleneck
+#ifndef CRL_INC_TICKET
+#define CRL_INC_TICKET 4
+#endif
+
+__device__ __forceinline__ uint32_t spec_diff(const FrameSpec& a, const FrameSpec& b) {
+    const uint32_t nr = ~(1u << 17);   // the raw bit only matters to the float32 mode
+    return (a.x ^ b.x) | ((a.y ^ b.y) & nr) | (a.z ^ b.z) | ((a.w ^ b.w) & nr);
+}
+
+// scoreboard entry of a frame (the kernel's text_id), -2 when its score combination is outside text_tab; any_valid = 0: the
+// all-zero frame
+__device__ __forceinline__ int frame_text_id(FrameSpec f, int agent, bool& any_valid) {
+    const bool va = (f.y >> 16) & 1u, vb = (f.w >> 16) & 1u;
+    any_valid = va || vb;
+    if (!va) f.y = f.w;
+    if (!vb) f.w = f.y;
+    const int pairA = (int)(f.y & 255u) * ATLAS_SCORES + (int)((f.y >> 8) & 255u);
+    const int pairB = (int)(f.w & 255u) * ATLAS_SCORES + (int)((f.w >> 8) & 255u);
+    int base = pairA, kind = 0;
+    if (pairA != pairB) {
+        const int d = pairB - pairA;
+        if (d == ATLAS_SCORES) kind = 1;
+        else if (d == 1 && (pairA % ATLAS_SCORES) != ATLAS_SCORES - 1) kind = 2;
+        else if (d == -ATLAS_SCORES) { base = pairB; kind = 1; }
+        else if (d == -1 && (pairB % ATLAS_SCORES) != ATLAS_SCORES - 1) { base = pairB; kind = 2; }
+        else return -2;
+    }
+    return (base * 3 + kind) * 2 + agent;
+}
+
+// Byte offsets of the bat word and the ball pixel this lane patches for frame f (-1: none): the offset arithmetic of phases
+// A2 / A3 of pong_raster_fast_kernel, without the pixel values.  For a frame that has valid render states.
+template <int DIM>
+__device__ __forceinline__ void frame_patch_offsets(const FastTabs<DIM>* T, FrameSpec f, int agent, int lane, int& bat_off,
+                                                    int& ball_off) {
+    const int cL = (int)T->bat_c0[0], cR = (int)T->bat_c0[1];
+    const int b_side = lane >> 4, b_which = (lane >> 3) & 1, b_row = lane & 7;
+    const int p_which = lane >> 4, p_col = lane & 3, p_row = (lane >> 2) & 3;
+    if (!((f.y >> 16) & 1u)) { f.x = f.z; f.y = f.w; }
+    if (!((f.w >> 16) & 1u)) { f.z = f.x; f.w = f.y; }
+    const bool same = (f.x == f.z);
+    const int lyA = (f.x >> 16) & 255u, ryA = f.x >> 24, lyB = (f.z >> 16) & 255u, ryB = f.z >> 24;
+    const int vlA = agent ? ryA : lyA, vrA = agent ? lyA : ryA;
+    const int vlB = agent ? ryB : lyB, vrB = agent ? lyB : ryB;
+    bat_off = -1;
+    {
+        const int y0 = b_which ? (b_side ? vrB : vlB) : (b_side ? vrA : vlA);
+        const int c0 = max(y0, ARENA_TOP), c1 = min(y0 + BAT_H, ARENA_BOTTOM);
+        if (c1 > c0 && !(b_which && same)) {
+            const int dy = (int)T->y_first[c0] + b_row;
+            if (dy <= (int)T->y_last[c1 - 1]) bat_off = dy * DIM + (b_side ? cR : cL);
+        }
+    }
+    ball_off = -1;
+    {
+        const FrameSpec& g = f;
+        const uint32_t bx = p_which ? g.z : g.x;
+        int x0 = bx & 255u, x1 = min(x0 + BALL_SIZE, SCREEN_W);
+        int y0 = (bx >> 8) & 255u, y1 = min(y0 + BALL_SIZE, ARENA_BOTTOM);
+        y0 = max(y0, ARENA_TOP);
+        if (agent) { const int t = SCREEN_W - x1; x1 = SCREEN_W - x0; x0 = t; }
+        if (x1 > x0 && y1 > y0 && !(p_which && same)) {
+            const int dx = (int)T->x_first[x0] + p_col, dy = (int)T->y_first[y0] + p_row;
+            if (dx <= (int)T->x_last[x1 - 1] && dy <= (int)T->y_last[y1 - 1]) ball_off = dy * DIM + dx;
+        }
+    }
+}
+
 // RING: the ring observation mode (crl_pong_config::stack_mode 1).  A template parameter, so that the plain-stack
 // instantiation carries none of the ring's run-time branches and state in its hot loop.
-template <int DIM, bool RING>
+// INC (plain stacks only): the output buffers hold the frames `shown` ([agent][c][n] FrameSpecs) describes; a frame is
+// stored only where it can differ from the one it replaces.  A frame equals the template outside its patches (bat
+// words, ball pixels) and its scoreboard words [text_w0, text_w1), so the chunks touched by the old frame's patches,
+// the new frame's patches and, when the scoreboard entries differ, the scoreboard words cover every changed byte.
+// Frames whose specs are equal (ignoring the raw bit) are not stored at all; the all-zero frame and scoreboards outside
+// text_tab are stored whole.  Afterwards `shown` holds hist.
+template <int DIM, bool RING, bool INC>
 __global__ void __launch_bounds__(FAST_WARPS * 32, FastCfg<DIM>::CTAS)
 pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* __restrict__ obs0,
-                        uint8_t* __restrict__ obs1, const FastTabs<DIM>* __restrict__ gtabs) {
+                        uint8_t* __restrict__ obs1, const FastTabs<DIM>* __restrict__ gtabs, FrameSpec* __restrict__ shown) {
     constexpr int TAPS = FastCfg<DIM>::TAPS, VEC = FastCfg<DIM>::VEC;
     constexpr int DD = DIM * DIM, FB = ((DD + 15) / 16) * 16, NCH = DD / VEC;
 #ifndef CRL_RASTER_TMA
 #define CRL_RASTER_TMA 0
 #endif
-    constexpr bool USE_TMA = (DD % 16 == 0) && (CRL_RASTER_TMA != 0);
+    constexpr bool USE_TMA = (DD % 16 == 0) && (CRL_RASTER_TMA != 0) && !INC;
     constexpr int TEXT_ITERS = 3;   // text_stride <= 96 vectors (checked on the host)
     typedef typename VecT<VEC>::type V;
     typedef FastTabs<DIM> Tabs;
     static_assert(DD % VEC == 0, "frame must be a whole number of store vectors");
+    static_assert(!INC || (!RING && VEC == 16), "incremental stacks: 16-byte chunks, plain stacks");
 
     extern __shared__ uint4 smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(smem_raw);
@@ -231,6 +311,8 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
     uint32_t prev_bat_rest = 0u, prev_ball_old = 0u;
     int cur_text = -1;          // text_tab entry whose rows are in the buffer (-1: template's)
     bool pending = false;       // a bulk store may still be reading the buffer
+    FrameSpec prev_spec = make_uint4(0u, 0u, 0u, 0u);   // INC: the frame whose patches prev_bat_off / prev_ball_off are
+    bool prev_known = false;
 
     // Stacks are handed out by a global counter, not by a static grid stride: all resident warps then write within one
     // compact window of the observation buffers that advances front to back, like the CTA dispatcher of a non-persistent
@@ -240,7 +322,7 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
     // makes the counter itself the bottleneck (2.7 TB/s in the probe).
     const long long n_stacks = (long long)p.n * p.n_agents;
     // frames a stack writes: c (plain stack), or the newest frame twice (ring; all 2c slots only after a reset)
-    const int per_ticket = max(1, 4 / (RING ? 2 : p.c));
+    const int per_ticket = INC ? CRL_INC_TICKET : max(1, 4 / (RING ? 2 : p.c));
     const int out_slots = RING ? 2 * p.c : p.c;
     long long s = 0, s_end = 0;
     for (;;) {
@@ -254,8 +336,12 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
         const long long s_cur = s++;
         const int env = (int)(s_cur / p.n_agents), agent = (int)(s_cur % p.n_agents);
         uint8_t* out_stack = (agent ? obs1 : obs0) + (size_t)env * out_slots * DD;
-        FrameSpec my_spec = make_uint4(0u, 0u, 0u, 0u);
-        if (lane < p.c) my_spec = hist[(size_t)lane * p.n + env];
+        FrameSpec my_spec = make_uint4(0u, 0u, 0u, 0u), my_shown = make_uint4(0u, 0u, 0u, 0u);
+        FrameSpec* shown_at = INC ? shown + ((size_t)agent * p.c + lane) * p.n + env : nullptr;
+        if (lane < p.c) {
+            my_spec = hist[(size_t)lane * p.n + env];
+            if (INC) my_shown = *shown_at;
+        }
         // ring: only the newest frame is new, unless the env was just reset (its whole history changed)
         const int first_slot = (RING && !p.fill_all && !p.last_done[env]) ? p.c - 1 : 0;
 
@@ -265,6 +351,15 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
             f.y = __shfl_sync(0xffffffffu, my_spec.y, slot);
             f.z = __shfl_sync(0xffffffffu, my_spec.z, slot);
             f.w = __shfl_sync(0xffffffffu, my_spec.w, slot);
+            const FrameSpec f_raw = f;
+            FrameSpec o = f;   // INC: what the buffer's slot holds
+            if (INC) {
+                o.x = __shfl_sync(0xffffffffu, my_shown.x, slot);
+                o.y = __shfl_sync(0xffffffffu, my_shown.y, slot);
+                o.z = __shfl_sync(0xffffffffu, my_shown.z, slot);
+                o.w = __shfl_sync(0xffffffffu, my_shown.w, slot);
+                if (spec_diff(f, o) == 0u) continue;   // the slot already holds this frame
+            }
             // plain stack: frame `slot` goes to channel `slot`.  Ring: to slot ring_phase + 1 + slot and to its double
             // c slots before or after it, whichever exists (the newest frame: ring_phase + c and ring_phase)
             uint8_t* out8 = out_stack + (size_t)slot * DD;
@@ -395,6 +490,21 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
                 }
             }
 
+            // ---- A4 (INC). what to store: the whole frame, or the chunks under both frames' patches and, when the
+            //      scoreboard entries differ, the chunks [ta, tb) of the scoreboard words ----
+            bool whole = true;
+            int ta = 0, tb = 0, old_bat = -1, old_ball = -1;
+            if (INC) {
+                bool old_valid;
+                const int old_text = frame_text_id(o, agent, old_valid);
+                whole = !old_valid || old_text == -2 || !text_ok;
+                if (!whole && old_text != text_id) { ta = p.text_w0 * 4 >> 4; tb = min((p.text_w1 * 4 + 15) >> 4, NCH); }
+                if (!whole) {
+                    if (prev_known && spec_diff(o, prev_spec) == 0u) { old_bat = prev_bat_off; old_ball = prev_ball_off; }
+                    else frame_patch_offsets<DIM>(T, o, agent, lane, old_bat, old_ball);
+                }
+            }
+
             // ======== B. the buffer: wait for the previous drain, restore, patch ========
             if (pending) {
                 if (lane == 0) bulk_wait_read();
@@ -440,9 +550,26 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
             if (ball_off >= 0) sm8[ball_off] = (uint8_t)ball_val;   // overrides the strip LUT where the ball is near
             prev_bat_off = bat_off; prev_bat_rest = bat_rest;
             prev_ball_off = ball_off; prev_ball_old = ball_old;
+            prev_spec = f_raw; prev_known = true;
 
             // ======== C. drain ========
-            if (USE_TMA) {
+#ifdef CRL_RASTER_NO_DRAIN
+            // measurement build: everything but the stores (the kernel's compute floor); the output is left unwritten
+            continue;
+#endif
+            if (INC && !whole) {
+                // Every lane stores the chunk under each of its patch offsets.  Lanes that hit the same chunk in one
+                // instruction store the same 16 bytes and coalesce; a chunk stored by two instructions gets the same bytes
+                // twice.  (A shared-memory bitmap that deduplicated the chunks first cost more in atomics than it saved.)
+                __syncwarp();
+                V* out = reinterpret_cast<V*>(out8);
+                for (int u = ta + lane; u < tb; u += 32) st_stream(out + u, sm[u]);
+                const int offs[4] = {old_bat, old_ball, bat_off, ball_off};
+#pragma unroll
+                for (int k = 0; k < 4; ++k)
+                    if (offs[k] >= 0) st_stream(out + (offs[k] >> 4), sm[offs[k] >> 4]);
+                __syncwarp();
+            } else if (USE_TMA) {
                 fence_proxy_async_smem();    // generic-proxy writes -> visible to the async proxy
                 __syncwarp();
                 if (lane == 0) {
@@ -470,6 +597,8 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
                 __syncwarp();
             }
         }
+        if (INC && lane < p.c) *shown_at = my_spec;
+        prev_known = false;   // patch offsets depend on the agent too
     }
     if (USE_TMA && lane == 0) bulk_wait_all();   // the buffer must outlive the last drain
 }
@@ -919,15 +1048,17 @@ cudaError_t pong_raster_init(int g_grid[3]) {
     int dev = 0, sms = 0, nb = 0;
     if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
     if ((e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-    // both instantiations (plain stack, ring) of a size share the shared-memory size and the register budget
-    // (__launch_bounds__), so one occupancy query per size sizes the grid for both
-    const void* fast[2][2] = {{(const void*)pong_raster_fast_kernel<84, false>, (const void*)pong_raster_fast_kernel<84, true>},
-                              {(const void*)pong_raster_fast_kernel<42, false>, (const void*)pong_raster_fast_kernel<42, true>}};
+    // the instantiations of a size (plain stack, ring; 84x84 also incremental) share the shared-memory size and the
+    // register budget (__launch_bounds__), so one occupancy query per size sizes the grid for all of them
+    const void* fast[2][2] = {{(const void*)pong_raster_fast_kernel<84, false, false>, (const void*)pong_raster_fast_kernel<84, true, false>},
+                              {(const void*)pong_raster_fast_kernel<42, false, false>, (const void*)pong_raster_fast_kernel<42, true, false>}};
     const int smem[2] = {(int)fast_smem_bytes<84>(), (int)fast_smem_bytes<42>()};
     for (int d = 0; d < 2; ++d)
         for (int r = 0; r < 2; ++r)
             if ((e = cudaFuncSetAttribute(fast[d][r], cudaFuncAttributeMaxDynamicSharedMemorySize, smem[d])) != cudaSuccess) return e;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, pong_raster_fast_kernel<84, false>, FAST_WARPS * 32, smem[0]);
+    e = cudaFuncSetAttribute(pong_raster_fast_kernel<84, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem[0]);
+    if (e != cudaSuccess) return e;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, pong_raster_fast_kernel<84, false, false>, FAST_WARPS * 32, smem[0]);
     if (e != cudaSuccess) return e;
     // 84x84: FastCfg<84>::CTAS per SM.  With uncompressed observation buffers the DRAM write path preferred fewer
     // concurrent write streams (2 CTAs: 0.523 ms per launch, 3: 0.535 ms).  With compressible buffers DRAM is no longer
@@ -935,7 +1066,7 @@ cudaError_t pong_raster_init(int g_grid[3]) {
     // (B200, 65 536 envs, stack mode; the ring instantiation spills 8 bytes at 3 and lost 2 %, 192.5 against 196.2 M
     // env-steps/s, less than the headline gains)
     g_grid[0] = sms * max(min(nb, FastCfg<84>::CTAS), 1);
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, pong_raster_fast_kernel<42, false>, FAST_WARPS * 32, smem[1]);
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, pong_raster_fast_kernel<42, false, false>, FAST_WARPS * 32, smem[1]);
     if (e != cudaSuccess) return e;
     g_grid[1] = sms * max(nb, 1);
     e = cudaFuncSetAttribute(pong_raster_quad_kernel<42>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)quad_smem_bytes<42>());
@@ -946,20 +1077,34 @@ cudaError_t pong_raster_init(int g_grid[3]) {
     return cudaSuccess;
 }
 
-cudaError_t launch_pong_raster(const PongDev& p, const FrameSpec* hist, uint8_t* obs0, uint8_t* obs1, cudaStream_t s) {
+static bool fast_path(const PongDev& p, const void* obs0, const void* obs1) {
+    const bool aligned = ((uintptr_t)obs0 % 16 == 0) && ((uintptr_t)obs1 % 16 == 0);
+    return p.fast_tabs != nullptr && p.fast_ok && aligned && (p.dim == 84 || p.dim == 42);
+}
+
+bool pong_raster_incremental_ok(const PongDev& p, const void* obs0, const void* obs1) {
+    return fast_path(p, obs0, obs1) && p.dim == 84 && !p.ring;
+}
+
+cudaError_t launch_pong_raster(const PongDev& p, const FrameSpec* hist, uint8_t* obs0, uint8_t* obs1, FrameSpec* shown,
+                               cudaStream_t s) {
     const long long n_stacks = (long long)p.n * p.n_agents;
     if (n_stacks == 0) return cudaSuccess;
-    const bool aligned = ((uintptr_t)obs0 % 16 == 0) && ((uintptr_t)obs1 % 16 == 0);
-    if (p.fast_tabs == nullptr || !p.fast_ok || !aligned || (p.dim != 84 && p.dim != 42))
-        return launch_pong_raster_generic(p, hist, nullptr, p.ring, obs0, obs1, s);
+    if (shown && !pong_raster_incremental_ok(p, obs0, obs1)) return cudaErrorInvalidValue;
+    if (!fast_path(p, obs0, obs1)) return launch_pong_raster_generic(p, hist, nullptr, p.ring, obs0, obs1, s);
     const long long want = (n_stacks + FAST_WARPS - 1) / FAST_WARPS;
     cudaError_t me = cudaMemsetAsync(p.work_counter, 0, sizeof(unsigned long long), s);
     if (me != cudaSuccess) return me;
     if (p.dim == 84) {
         const unsigned grid = (unsigned)min((long long)p.raster_grid[0], want);
         const FastTabs<84>* tabs = reinterpret_cast<const FastTabs<84>*>(p.fast_tabs);
-        if (p.ring) pong_raster_fast_kernel<84, true><<<grid, FAST_WARPS * 32, fast_smem_bytes<84>(), s>>>(p, hist, obs0, obs1, tabs);
-        else pong_raster_fast_kernel<84, false><<<grid, FAST_WARPS * 32, fast_smem_bytes<84>(), s>>>(p, hist, obs0, obs1, tabs);
+        if (shown) {
+            pong_raster_fast_kernel<84, false, true><<<grid, FAST_WARPS * 32, fast_smem_bytes<84>(), s>>>(p, hist, obs0, obs1, tabs, shown);
+        } else if (p.ring) {
+            pong_raster_fast_kernel<84, true, false><<<grid, FAST_WARPS * 32, fast_smem_bytes<84>(), s>>>(p, hist, obs0, obs1, tabs, nullptr);
+        } else {
+            pong_raster_fast_kernel<84, false, false><<<grid, FAST_WARPS * 32, fast_smem_bytes<84>(), s>>>(p, hist, obs0, obs1, tabs, nullptr);
+        }
     } else if (p.quad_ok && !p.ring && (long long)p.n * p.c * p.n_agents < (1LL << 31)) {
         const long long quads = (((long long)p.n * p.c + 3) / 4) * p.n_agents;
         const unsigned grid = (unsigned)min((long long)p.raster_grid[2], (quads + 4 * QUAD_WARPS - 1) / (4 * QUAD_WARPS));
@@ -968,8 +1113,8 @@ cudaError_t launch_pong_raster(const PongDev& p, const FrameSpec* hist, uint8_t*
     } else {
         const unsigned grid = (unsigned)min((long long)p.raster_grid[1], want);
         const FastTabs<42>* tabs = reinterpret_cast<const FastTabs<42>*>(p.fast_tabs);
-        if (p.ring) pong_raster_fast_kernel<42, true><<<grid, FAST_WARPS * 32, fast_smem_bytes<42>(), s>>>(p, hist, obs0, obs1, tabs);
-        else pong_raster_fast_kernel<42, false><<<grid, FAST_WARPS * 32, fast_smem_bytes<42>(), s>>>(p, hist, obs0, obs1, tabs);
+        if (p.ring) pong_raster_fast_kernel<42, true, false><<<grid, FAST_WARPS * 32, fast_smem_bytes<42>(), s>>>(p, hist, obs0, obs1, tabs, nullptr);
+        else pong_raster_fast_kernel<42, false, false><<<grid, FAST_WARPS * 32, fast_smem_bytes<42>(), s>>>(p, hist, obs0, obs1, tabs, nullptr);
     }
     return cudaGetLastError();
 }

@@ -219,6 +219,12 @@ class CudaPongVecEnv(VecEnv):
     step t + n_buffers.  Keep rollouts alive with a larger `n_buffers`, or pass `copy=True` to get fresh tensors from
     every call (one extra device copy of the observations per step).
 
+    Do not write into the returned observation tensors.  At 84x84 with stack_mode="stack" and uint8 observations the
+    buffer sets are registered with the library (crl_pong_set_obs_buffers), which then stores only the 16-byte chunks of
+    each stack whose frames changed since that buffer was last rendered.  A caller that
+    modifies a returned tensor in place must use `copy=True`, or call `forget_obs()` afterwards so that the next render
+    into each buffer rewrites it whole.
+
     stack_mode="ring" (opt-in): the observations are strided VIEWS `ring[:, k+1 : k+1+C]` of an (N, 2C, D, D) ring per
     agent in which every new frame is stored twice (slots k and k + C), so a step writes 2 frames per agent instead of
     C -- same values, half the HBM traffic (SURVEY.md 8(d): 28 224 B instead of 56 448 B per env-step at 84x84x4).  The
@@ -306,6 +312,10 @@ class CudaPongVecEnv(VecEnv):
                 real=torch.zeros((n, 2), dtype=torch.float32, device=dev),
                 done=torch.zeros((n,), dtype=torch.bool, device=dev),
                 steps=torch.zeros((n,), dtype=torch.int32, device=dev)))
+        self._tracked = not self.ring and not self.f32 and self.dim == 84
+        if self._tracked:
+            self._impl.set_obs_buffers([b["obs"][0] for b in self._sets],
+                                       [b["obs"][1] for b in self._sets] if self.n_agents == 2 else [])
         self._cur = 0
         self._bind(0)
         self._actions = torch.zeros((n, 2) if self.n_agents == 2 else (n,), dtype=torch.int32, device=dev)
@@ -451,6 +461,8 @@ class CudaPongVecEnv(VecEnv):
         if not self.closed and self._impl is not None:
             if torch.cuda.is_available():
                 torch.cuda.synchronize(self.device)
+            if self._tracked:
+                self._impl.set_obs_buffers([], [])
             self._impl.close()
             self._h = None
             # the env's references to its buffers: the observation memory goes back once the caller's are gone too
@@ -476,6 +488,10 @@ class CudaPongVecEnv(VecEnv):
         assert tuple(s.shape) == (self.num_envs, 10)
         self._impl.set_state(s)
         torch.cuda.current_stream(self.device).synchronize()
+
+    def forget_obs(self):
+        """After writing into observation tensors this env returned: the next render into each buffer rewrites it whole."""
+        self._impl.forget_obs()
 
     def check(self):
         """Raise if a device-side error flag is set (serve table overrun, invalid device action).  Synchronises; the flag

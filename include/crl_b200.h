@@ -127,6 +127,20 @@ int crl_pong_ring_phase(crl_pong* h);
 /* same output through the one-thread-per-pixel reference rasteriser (cross-check) */
 int crl_pong_render_obs_generic(crl_pong* h, uint8_t* obs0_dev, uint8_t* obs1_dev, void* stream);
 
+/* Observation buffers whose contents the library may trust (stack_mode 0).  Registers `count` buffer sets: set i is
+ * obs0_devs_host[i] and, for cPongDouble, obs1_devs_host[i] (may be NULL for cPong), each of crl_pong_render_obs's size.
+ * The library remembers which frames a set holds after every render into it; at 84x84 a later crl_pong_render_obs (or
+ * step / reset / step_host) into the same set stores only the 16-byte chunks whose frames changed.
+ * The caller must therefore not write into a registered buffer, or must call crl_pong_forget_obs afterwards; the
+ * library's own other writers (render_obs_generic, render_obs_f32, terminal_obs, load_atlas) do so themselves.
+ * count = 0 unregisters every set.  Synchronises the stream.  Environment: CRL_PONG_FULL_OBS=1 at crl_pong_create makes
+ * every render store whole stacks (A/B runs). */
+#define CRL_PONG_MAX_OBS_SETS 16
+int crl_pong_set_obs_buffers(crl_pong* h, uint8_t* const* obs0_devs_host, uint8_t* const* obs1_devs_host, int32_t count,
+                             void* stream);
+/* the registered sets' contents are unknown (the caller wrote into them): the next render into each stores it whole */
+int crl_pong_forget_obs(crl_pong* h);
+
 /* info["terminal_observation"] of the LAST step: writes, for every env whose
  * done_dev[i] != 0, the stacked observation the episode ended with into
  * term{0,1}_dev[i] (same layout as obs); other envs' slots are left untouched. */
