@@ -26,6 +26,8 @@ EXPORTS = [
     "crl_car_random_actions", "crl_car_get_stats", "crl_car_get_contacts", "crl_car_check",
     "crl_car_seed", "crl_car_step_host", "crl_car_set_elapsed", "crl_car_set_state", "crl_car_ring_phase", "crl_car_render_state", "crl_car_set_obs_rotation",
     "crl_obs_alloc", "crl_obs_free",
+    "crl_pong_opp_create", "crl_pong_opp_destroy", "crl_pong_opp_seed", "crl_pong_opp_load_net", "crl_pong_opp_set_pool",
+    "crl_pong_opp_assign", "crl_pong_opp_restart", "crl_pong_opp_act", "crl_pong_opp_get_ids", "crl_pong_opp_get_stats",
 ]
 
 
@@ -145,6 +147,16 @@ def load():
     L.crl_car_get_stats.argtypes = [vp, vp, vp]
     L.crl_car_get_contacts.argtypes = [vp, vp, vp, vp]
     L.crl_car_check.argtypes = [vp, vp]
+    L.crl_pong_opp_create.argtypes = [i32, i32, u64, ctypes.c_int64, ctypes.POINTER(vp)]
+    L.crl_pong_opp_destroy.argtypes = [vp]
+    L.crl_pong_opp_seed.argtypes = [vp, u64]
+    L.crl_pong_opp_load_net.argtypes = [vp, i32, vp, ctypes.c_size_t, vp]
+    L.crl_pong_opp_set_pool.argtypes = [vp, vp, vp, i32, vp]
+    L.crl_pong_opp_assign.argtypes = [vp, vp, vp]
+    L.crl_pong_opp_restart.argtypes = [vp, i32, vp]
+    L.crl_pong_opp_act.argtypes = [vp, vp, vp, vp, i32, vp, vp, vp]
+    L.crl_pong_opp_get_ids.argtypes = [vp, vp, vp]
+    L.crl_pong_opp_get_stats.argtypes = [vp, vp, vp]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("crl_last_error", "crl_launch_count"):

@@ -15,7 +15,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 OUT = os.path.join(HERE, "libcrl_b200.so")
 SOURCES = ["crl_abi.cu", "pong_step.cu", "pong_raster.cu", "pong_raster_fast.cu", "crl_car_abi.cu",
-           "car_physics.cu", "car_raster.cu"]
+           "car_physics.cu", "car_raster.cu", "pong_opponent.cu"]
 HEADERS = ["pong_common.cuh", "pong_raster_dev.cuh", "car_common.cuh", "car_contact.cuh", "car_spans.cuh", "crl_host.h",
            os.path.join("..", "..", "include", "crl_b200.h")]
 NVCC_FLAGS = [

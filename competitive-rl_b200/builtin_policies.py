@@ -9,6 +9,9 @@ RANDOM a device randint; WEAK / MEDIUM (LightActorCritic, utils/network.py:73-93
 not part of this repository: point COMPETITIVE_RL_RESOURCES (or the resource_dir argument) at the directory that
 holds them; agents whose checkpoint is missing are simply not offered (the reference itself ships only weak and
 medium).  The convolutions / linear layers are plain torch (cuDNN / cuBLAS) library calls.
+
+The per-env opponents of tournament.py (set_opponents) run LightActorCritic networks in the project's own CUDA kernel
+instead; pack_light_actor_critic is the flat parameter image that kernel loads.
 """
 import os
 
@@ -41,6 +44,52 @@ class LightActorCritic(nn.Module):
         x = F.relu(self.conv1(x / 255.0))
         x = F.relu(self.conv2(x)).flatten(1)
         return self.actor_linear(x), self.critic_linear(x)
+
+
+# LightActorCritic's parameters in state-dict order: the flat layout the per-env opponent kernel loads
+# (include/crl_b200.h, CRL_PONG_OPP_NET_FLOATS).  The critic is carried so that the image is the whole state dict.
+LIGHT_ACTOR_CRITIC_LAYOUT = [("conv1.weight", (16, 4, 4, 4)), ("conv1.bias", (16,)), ("conv2.weight", (16, 16, 2, 2)),
+                             ("conv2.bias", (16,)), ("critic_linear.weight", (1, 1600)), ("critic_linear.bias", (1,)),
+                             ("actor_linear.weight", (3, 1600)), ("actor_linear.bias", (3,))]
+LIGHT_ACTOR_CRITIC_FLOATS = 8484
+
+
+def pack_light_actor_critic(state):
+    """float32 CPU tensor of LIGHT_ACTOR_CRITIC_FLOATS: the parameters of a LightActorCritic (a state dict, a checkpoint
+    dict with the state dict under "model", or the module) concatenated row-major in LIGHT_ACTOR_CRITIC_LAYOUT order.
+    ActorCritic (STRONG / ALPHA_PONG) and any other layout are refused with ValueError."""
+    if isinstance(state, nn.Module):
+        state = state.state_dict()
+    if "model" in state and not isinstance(state["model"], torch.Tensor):
+        state = state["model"]
+    names = [n for n, _ in LIGHT_ACTOR_CRITIC_LAYOUT]
+    if any(k.startswith("conv3.") for k in state) or tuple(state.get("conv2.weight", torch.empty(0)).shape) == (32, 16, 4, 4):
+        raise ValueError("an ActorCritic network (STRONG / ALPHA_PONG layout) cannot play in a per-env pool: only the "
+                         "LightActorCritic layout (WEAK / MEDIUM) is supported")
+    if sorted(state) != sorted(names):
+        raise ValueError("not a LightActorCritic state dict: expected parameters %s, got %s" % (names, sorted(state)))
+    parts = []
+    for name, shape in LIGHT_ACTOR_CRITIC_LAYOUT:
+        t = torch.as_tensor(state[name])
+        if tuple(t.shape) != shape:
+            raise ValueError("LightActorCritic parameter %s has shape %s, expected %s" % (name, tuple(t.shape), shape))
+        parts.append(t.detach().to("cpu", torch.float32).reshape(-1))
+    return torch.cat(parts).contiguous()
+
+
+def unpack_light_actor_critic(flat):
+    """Inverse of pack_light_actor_critic: a state dict LightActorCritic.load_state_dict accepts."""
+    flat = torch.as_tensor(flat, dtype=torch.float32).reshape(-1)
+    if flat.numel() != LIGHT_ACTOR_CRITIC_FLOATS:
+        raise ValueError("a LightActorCritic image has %d floats, got %d" % (LIGHT_ACTOR_CRITIC_FLOATS, flat.numel()))
+    out, k = {}, 0
+    for name, shape in LIGHT_ACTOR_CRITIC_LAYOUT:
+        n = 1
+        for d in shape:
+            n *= d
+        out[name] = flat[k:k + n].reshape(shape).clone()
+        k += n
+    return out
 
 
 class ActorCritic(nn.Module):
@@ -124,6 +173,20 @@ def get_builtin_agent_names(resource_dir=None):
             continue
         names.append(n)
     return names
+
+
+def find_checkpoint(agent_name, resource_dir=None):
+    """Path of a built-in network agent's checkpoint file, or None when it cannot be found."""
+    d = find_resource_dir(resource_dir)
+    if agent_name not in _CHECKPOINTS or not d:
+        return None
+    path = os.path.join(d, _CHECKPOINTS[agent_name][0])
+    return path if os.path.isfile(path) else None
+
+
+def is_light_agent(agent_name):
+    """True for the built-in network agents with the LightActorCritic layout (WEAK, MEDIUM)."""
+    return agent_name in _CHECKPOINTS and _CHECKPOINTS[agent_name][1]
 
 
 def get_compute_action_function(agent_name, num_envs=1, device="cuda", resource_dir=None):

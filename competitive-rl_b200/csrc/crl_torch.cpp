@@ -262,6 +262,62 @@ struct Car {
     uint64_t raw_handle() const { return (uint64_t)(uintptr_t)h; }
 };
 
+// ------------------------------------------------------------------------------------------------ per-env opponents
+struct PongOpponents {
+    crl_pong_opp* h = nullptr;
+    int device = 0;
+    int64_t num_envs = 0;
+
+    PongOpponents(int64_t n, int64_t dev, uint64_t seed, int64_t first_env) : device((int)dev), num_envs(n) {
+        check_rc(crl_pong_opp_create((int32_t)n, (int32_t)dev, seed, first_env, &h));
+    }
+    ~PongOpponents() { close(); }
+    void close() {
+        if (h) { crl_pong_opp_destroy(h); h = nullptr; }
+    }
+    crl_pong_opp* handle() const {
+        TORCH_CHECK(h != nullptr, "the opponent handle is closed");
+        return h;
+    }
+    int64_t n() const { return num_envs; }
+
+    void seed(uint64_t s) { check_rc(crl_pong_opp_seed(handle(), s)); }
+    // params: float32 CPU tensor of CRL_PONG_OPP_NET_FLOATS (state-dict order, builtin_policies.pack_light_actor_critic)
+    void load_net(int64_t slot, const at::Tensor& params) {
+        check_rc(crl_pong_opp_load_net(handle(), (int32_t)slot, host_ptr<float>(params, at::kFloat, "params"), (size_t)params.numel(),
+                                       stream_of(device)));
+    }
+    // kinds: int32 CPU tensor (CRL_PONG_OPP_RULE_BASED, CRL_PONG_OPP_RANDOM or a slot); weights: float64 CPU tensor or None
+    void set_pool(const at::Tensor& kinds, const c10::optional<at::Tensor>& weights) {
+        if (weights.has_value()) TORCH_CHECK(weights->numel() == kinds.numel(), "one weight per pool entry");
+        check_rc(crl_pong_opp_set_pool(handle(), host_ptr<int32_t>(kinds, at::kInt, "kinds"),
+                                       weights.has_value() ? host_ptr<double>(*weights, at::kDouble, "weights") : nullptr,
+                                       (int32_t)kinds.numel(), stream_of(device)));
+    }
+    // ids: int32 CPU tensor of num_envs pool indices, or None = draw from the pool
+    void assign(const c10::optional<at::Tensor>& ids) {
+        if (ids.has_value()) TORCH_CHECK(ids->numel() == n(), "ids: expected ", n(), " elements, got ", ids->numel());
+        check_rc(crl_pong_opp_assign(handle(), ids.has_value() ? host_ptr<int32_t>(*ids, at::kInt, "ids") : nullptr, stream_of(device)));
+    }
+    void restart(bool clear_stacks) { check_rc(crl_pong_opp_restart(handle(), clear_stacks ? 1 : 0, stream_of(device))); }
+    void act(const at::Tensor& obs1, const c10::optional<at::Tensor>& rew, const c10::optional<at::Tensor>& done, bool resample,
+             const at::Tensor& actions, const c10::optional<at::Tensor>& logits) {
+        check_rc(crl_pong_opp_act(handle(), dev_ptr<uint8_t>(obs1, at::kByte, device, n() * 42 * 42, "obs1"),
+                                  opt_dev_ptr<float>(rew, at::kFloat, device, 2 * n(), "rew"),
+                                  opt_dev_ptr<uint8_t>(done, at::kBool, device, n(), "done"), resample ? 1 : 0,
+                                  dev_ptr<int32_t>(actions, at::kInt, device, 2 * n(), "actions"),
+                                  opt_dev_ptr<float>(logits, at::kFloat, device, 3 * n(), "logits"), stream_of(device)));
+    }
+    void ids(const at::Tensor& out) {
+        check_rc(crl_pong_opp_get_ids(handle(), dev_ptr<int32_t>(out, at::kInt, device, n(), "ids"), stream_of(device)));
+    }
+    std::vector<uint64_t> stats() {
+        std::vector<uint64_t> s(4 * CRL_PONG_OPP_MAX_POOL);
+        check_rc(crl_pong_opp_get_stats(handle(), s.data(), stream_of(device)));
+        return s;
+    }
+};
+
 // An uninitialised observation buffer: crl_obs_alloc's memory (compressible where the device grants it) viewed as a tensor
 // that gives the memory back through crl_obs_free when its storage is released; with compressible=False, torch.empty.
 // Returns (tensor, whether the memory is compressible).
@@ -329,4 +385,20 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
         .def("contacts", &Car::contacts)
         .def("check", &Car::check)
         .def("raw_handle", &Car::raw_handle);
+    m.attr("OPP_NET_FLOATS") = CRL_PONG_OPP_NET_FLOATS;
+    m.attr("OPP_SLOTS") = CRL_PONG_OPP_SLOTS;
+    m.attr("OPP_MAX_POOL") = CRL_PONG_OPP_MAX_POOL;
+    m.attr("OPP_RULE_BASED") = CRL_PONG_OPP_RULE_BASED;
+    m.attr("OPP_RANDOM") = CRL_PONG_OPP_RANDOM;
+    py::class_<PongOpponents>(m, "PongOpponents")
+        .def(py::init<int64_t, int64_t, uint64_t, int64_t>())
+        .def("close", &PongOpponents::close)
+        .def("seed", &PongOpponents::seed)
+        .def("load_net", &PongOpponents::load_net)
+        .def("set_pool", &PongOpponents::set_pool)
+        .def("assign", &PongOpponents::assign)
+        .def("restart", &PongOpponents::restart)
+        .def("act", &PongOpponents::act)
+        .def("ids", &PongOpponents::ids)
+        .def("stats", &PongOpponents::stats);
 }

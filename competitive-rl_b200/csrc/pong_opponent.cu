@@ -1,0 +1,511 @@
+// pong_opponent.cu -- per-env built-in opponents of cPongTournament-v0 (include/crl_b200.h, crl_pong_opp_*).
+//
+// Replaces, for a batch in which every env plays its own opponent, what TournamentEnvWrapper + policy_serving.Policy
+// (competitive_rl/pong/competitive_pong_env.py:9-53, utils/policy_serving.py:10-66) do for one opponent per batch.
+// One launch of pong_opp_act_kernel per wrapper step, no host synchronisation:
+//   1. episode bookkeeping of the step before: agent 0's clipped reward is summed per env; an env that finished credits
+//      the episode to its opponent (win / draw / loss of agent 0, as pong/evaluate.py:53-88 classifies) and, with
+//      resample, draws its next opponent from the pool;
+//   2. frame stack: agent 1's newest 42x42 frame goes into the env's uint8 4-frame ring (whatever its opponent is);
+//   3. action into column 1 of the int32 (N, 2) step buffer: 999 for RULE_BASED, a Philox draw from {0, 1, 2} for
+//      RANDOM, or the greedy action of a LightActorCritic network (utils/network.py:73-93) over stack / 255 in fp32.
+// The networks run on the SIMT fp32 pipe with explicit __fmaf_rn (the library is compiled with -fmad=false).  Each CTA
+// owns a contiguous range of envs; it sorts them by network slot in shared memory and then runs every slot present
+// with that slot's weights staged once in shared memory, one env at a time over all its threads.
+#include <stdarg.h>
+#include <string.h>
+
+#include <cmath>
+#include <vector>
+
+#include "../../include/crl_b200.h"
+#include "crl_host.h"
+#include "pong_common.cuh"
+
+using namespace crl;
+
+extern "C" const char* crl_last_error(void);
+extern int crl_set_error(int code, const char* fmt, ...);
+extern void crl_count_launch(int n);
+
+#define CUDA_TRY(expr)                                                                                   \
+    do {                                                                                                 \
+        cudaError_t _e = (expr);                                                                         \
+        if (_e != cudaSuccess) return crl_set_error(CRL_E_CUDA, "%s: %s", #expr, cudaGetErrorString(_e)); \
+    } while (0)
+#define LAUNCH(expr)         \
+    do {                     \
+        CUDA_TRY(expr);      \
+        crl_count_launch(1); \
+    } while (0)
+
+namespace crl {
+namespace opp {
+
+constexpr int DIM = 42;
+constexpr int FRAME = DIM * DIM;             // 1764 bytes, 441 words
+constexpr int FRAME_WORDS = FRAME / 4;
+constexpr int STACK = 4;
+constexpr int H1 = 20;                       // conv1 4x4 / 2: 42 -> 20
+constexpr int H2 = 10;                       // conv2 2x2 / 2: 20 -> 10
+constexpr int C1 = 16, C2 = 16;
+constexpr int FEATS = C2 * H2 * H2;          // 1600
+constexpr int THREADS = 224;                 // 7 warps: conv1 = 200 items of 2 positions x 16 channels
+constexpr int SUB = 64;                      // envs a CTA sorts by slot at a time
+
+// A slot's weights in shared memory (floats), transposed at load time so that a thread's 16 output channels of one
+// tap are 16 consecutive floats (four broadcast 128-bit loads):
+//   W1[64][16]  tap (ci*16 + kh*4 + kw), channel    conv1
+//   B1[16]
+//   W2[64][16]  tap (ci*4 + kh*2 + kw), channel     conv2
+//   B2[16]
+//   WA[3][1600] feature (c*100 + y*10 + x)           actor_linear (the flatten order of (16, 10, 10))
+//   BA[4]       3 used
+constexpr int OFF_W1 = 0, OFF_B1 = OFF_W1 + 64 * C1, OFF_W2 = OFF_B1 + C1, OFF_B2 = OFF_W2 + 64 * C2,
+              OFF_WA = OFF_B2 + C2, OFF_BA = OFF_WA + 3 * FEATS, NET_DEV = OFF_BA + 4;
+static_assert(NET_DEV % 4 == 0, "slot image is copied as float4");
+// the state-dict order of CRL_PONG_OPP_NET_FLOATS (LightActorCritic: conv1.weight, conv1.bias, conv2.weight, conv2.bias,
+// critic_linear.weight, critic_linear.bias, actor_linear.weight, actor_linear.bias)
+constexpr int SD_W1 = 0, SD_B1 = SD_W1 + C1 * STACK * 16, SD_W2 = SD_B1 + C1, SD_B2 = SD_W2 + C2 * C1 * 4,
+              SD_WC = SD_B2 + C2, SD_BC = SD_WC + FEATS, SD_WA = SD_BC + 1, SD_BA = SD_WA + 3 * FEATS, SD_END = SD_BA + 3;
+static_assert(SD_END == CRL_PONG_OPP_NET_FLOATS, "flat layout of the header");
+
+// shared memory of the act kernel (floats unless noted); h2 reuses the input stack, which conv1 is done with
+constexpr int SM_W = 0, SM_X = SM_W + NET_DEV, SM_H1 = SM_X + STACK * FRAME, SM_LUT = SM_H1 + C1 * H1 * H1,
+              SM_RED = SM_LUT + 256, SM_FLOATS = SM_RED + 8 * 3;
+constexpr size_t SMEM_BYTES = SM_FLOATS * sizeof(float) + CRL_PONG_OPP_SLOTS * SUB + 16 * sizeof(int);
+
+constexpr int KIND_RULE = CRL_PONG_OPP_RULE_BASED;   // CRL_PONG_OPP_RANDOM is the other negative kind
+
+struct OppArgs {
+    int n;
+    int pool_size;
+    int phase;                // ring slot the newest frame goes to this step; the stack is slots phase+1 .. phase (oldest -> newest)
+    int resample;
+    int64_t first_env;
+    uint64_t seed;
+    uint64_t step;            // RANDOM's counter: act calls since the handle was created
+    int8_t kind[CRL_PONG_OPP_MAX_POOL];      // CRL_PONG_OPP_RULE_BASED, CRL_PONG_OPP_RANDOM or a network slot
+    uint64_t cum[CRL_PONG_OPP_MAX_POOL];     // draw: entry k is the first with r32 < cum[k]
+    const uint8_t* obs1;      // [n][1764] agent 1's observation of the previous step
+    const float* rew;         // [n][2] or nullptr (no bookkeeping this step)
+    const uint8_t* done;      // [n]
+    int32_t* actions;         // [n][2], column 1 written
+    float* logits;            // [n][3] or nullptr
+    int32_t* ids;             // [n]
+    uint8_t* stack;           // [n][4][1764]
+    float* ret;               // [n] agent 0's summed clipped reward of the episode in progress
+    uint32_t* episodes;       // [n] episodes finished since the handle was created (the draw counter)
+    unsigned long long* stats;   // [16][4] episodes, wins, draws, losses of agent 0
+    const float* nets;        // [8][NET_DEV]
+};
+
+// Philox streams: (global env, tag) x counter, keyed by the seed.  tag 1 = RANDOM's actions, tag 2 = opponent draws.
+__device__ __forceinline__ uint32_t opp_rand(uint64_t seed, int64_t g, uint32_t tag, uint64_t ctr) {
+    uint32_t r[4];
+    philox4x32_10((uint32_t)g, (uint32_t)((uint64_t)g >> 32) ^ (tag << 24), (uint32_t)ctr, (uint32_t)(ctr >> 32),
+                  (uint32_t)seed, (uint32_t)(seed >> 32), r);
+    return r[0];
+}
+
+__device__ __forceinline__ int opp_draw(const OppArgs& a, int64_t g, uint32_t episode) {
+    const uint64_t r = opp_rand(a.seed, g, 2u, episode);
+    int k = 0;
+    while (k < a.pool_size - 1 && r >= a.cum[k]) ++k;
+    return k;
+}
+
+__global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs a) {
+    extern __shared__ __align__(16) float sm[];
+    float* const w = sm + SM_W;
+    float* const xs = sm + SM_X;
+    float* const h1 = sm + SM_H1;
+    float* const h2 = xs;
+    float* const lut = sm + SM_LUT;
+    float* const red = sm + SM_RED;
+    uint8_t* const list = (uint8_t*)(sm + SM_FLOATS);             // [slot][SUB]
+    int* const cnt = (int*)(list + CRL_PONG_OPP_SLOTS * SUB);   // [slot]
+    const int tid = threadIdx.x;
+
+    for (int b = tid; b < 256; b += THREADS) lut[b] = (float)b / 255.0f;
+    const int r0 = (int)((int64_t)a.n * blockIdx.x / gridDim.x), r1 = (int)((int64_t)a.n * (blockIdx.x + 1) / gridDim.x);
+    for (int e0 = r0; e0 < r1; e0 += SUB) {
+        const int ne = min(SUB, r1 - e0);
+        if (tid < CRL_PONG_OPP_SLOTS) cnt[tid] = 0;
+        __syncthreads();
+        // ---- per env: bookkeeping of the step before, redraw, actions of the non-network kinds, sort by slot
+        if (tid < ne) {
+            const int i = e0 + tid;
+            const int64_t g = a.first_env + i;
+            int id = a.ids[i];
+            if (a.rew) {
+                float r = a.ret[i] + a.rew[2 * i];
+                if (a.done[i]) {
+                    unsigned long long* st = a.stats + 4 * id;
+                    atomicAdd(st, 1ull);
+                    atomicAdd(st + (r > 0.f ? 1 : r == 0.f ? 2 : 3), 1ull);
+                    r = 0.f;
+                    const uint32_t ep = a.episodes[i] + 1u;
+                    a.episodes[i] = ep;
+                    if (a.resample) {
+                        id = opp_draw(a, g, ep);
+                        a.ids[i] = id;
+                    }
+                }
+                a.ret[i] = r;
+            }
+            const int kind = a.kind[id];
+            if (kind >= 0) {
+                list[kind * SUB + atomicAdd(&cnt[kind], 1)] = (uint8_t)tid;
+            } else {
+                a.actions[2 * i + 1] = kind == KIND_RULE ? CHEAT_CODES
+                                                         : (int32_t)(((uint64_t)opp_rand(a.seed, g, 1u, a.step) * 3u) >> 32);
+                if (a.logits) a.logits[3 * i] = a.logits[3 * i + 1] = a.logits[3 * i + 2] = 0.f;
+            }
+        }
+        // ---- the newest frame into ring slot `phase` of every env of the range
+        {
+            const uint32_t* src = (const uint32_t*)(a.obs1 + (size_t)e0 * FRAME);
+            uint32_t* dst = (uint32_t*)(a.stack + (size_t)e0 * STACK * FRAME + (size_t)a.phase * FRAME);
+            for (int k = tid; k < ne * FRAME_WORDS; k += THREADS) {
+                const int e = k / FRAME_WORDS, j = k - e * FRAME_WORDS;
+                dst[(size_t)e * STACK * FRAME_WORDS + j] = src[k];
+            }
+        }
+        __syncthreads();
+        // ---- networks, slot by slot
+        for (int s = 0; s < CRL_PONG_OPP_SLOTS; ++s) {
+            const int m = cnt[s];
+            if (m == 0) continue;
+            {
+                const float4* src = (const float4*)(a.nets + (size_t)s * NET_DEV);
+                for (int k = tid; k < NET_DEV / 4; k += THREADS) ((float4*)w)[k] = src[k];
+            }
+            for (int q = 0; q < m; ++q) {
+                const int i = e0 + list[s * SUB + q];
+                {   // stack / 255 -> xs[ci][42][42], ci 0 = oldest
+                    const uint32_t* src = (const uint32_t*)(a.stack + (size_t)i * STACK * FRAME);
+                    for (int k = tid; k < STACK * FRAME_WORDS; k += THREADS) {
+                        const int ci = k / FRAME_WORDS, j = k - ci * FRAME_WORDS;
+                        const uint32_t v = src[((a.phase + 1 + ci) & 3) * FRAME_WORDS + j];
+                        float4 f;
+                        f.x = lut[v & 255]; f.y = lut[(v >> 8) & 255]; f.z = lut[(v >> 16) & 255]; f.w = lut[v >> 24];
+                        *(float4*)&xs[ci * FRAME + 4 * j] = f;
+                    }
+                }
+                __syncthreads();
+                if (tid < H1 * H1 / 2) {   // conv1 + relu: positions (oy, ox) and (oy, ox + 10), all 16 channels
+                    const int oy = tid / 10, ox = tid - oy * 10;
+                    float acc0[C1], acc1[C1];
+#pragma unroll
+                    for (int c = 0; c < C1; ++c) acc0[c] = acc1[c] = w[OFF_B1 + c];
+#pragma unroll 1
+                    for (int ci = 0; ci < STACK; ++ci)
+#pragma unroll
+                        for (int kh = 0; kh < 4; ++kh)
+#pragma unroll
+                            for (int kw = 0; kw < 4; ++kw) {
+                                const float* xp = xs + ci * FRAME + (2 * oy + kh) * DIM + 2 * ox + kw;
+                                const float x0 = xp[0], x1 = xp[20];
+                                const float4* wp = (const float4*)(w + OFF_W1 + (ci * 16 + kh * 4 + kw) * C1);
+#pragma unroll
+                                for (int c4 = 0; c4 < C1 / 4; ++c4) {
+                                    const float4 wv = wp[c4];
+                                    acc0[4 * c4 + 0] = __fmaf_rn(wv.x, x0, acc0[4 * c4 + 0]);
+                                    acc0[4 * c4 + 1] = __fmaf_rn(wv.y, x0, acc0[4 * c4 + 1]);
+                                    acc0[4 * c4 + 2] = __fmaf_rn(wv.z, x0, acc0[4 * c4 + 2]);
+                                    acc0[4 * c4 + 3] = __fmaf_rn(wv.w, x0, acc0[4 * c4 + 3]);
+                                    acc1[4 * c4 + 0] = __fmaf_rn(wv.x, x1, acc1[4 * c4 + 0]);
+                                    acc1[4 * c4 + 1] = __fmaf_rn(wv.y, x1, acc1[4 * c4 + 1]);
+                                    acc1[4 * c4 + 2] = __fmaf_rn(wv.z, x1, acc1[4 * c4 + 2]);
+                                    acc1[4 * c4 + 3] = __fmaf_rn(wv.w, x1, acc1[4 * c4 + 3]);
+                                }
+                            }
+#pragma unroll
+                    for (int c = 0; c < C1; ++c) {
+                        h1[c * H1 * H1 + oy * H1 + ox] = fmaxf(acc0[c], 0.f);
+                        h1[c * H1 * H1 + oy * H1 + ox + 10] = fmaxf(acc1[c], 0.f);
+                    }
+                }
+                __syncthreads();
+                if (tid < 2 * H2 * H2) {   // conv2 + relu: one position, 8 channels
+                    const int half = tid / (H2 * H2), p = tid - half * H2 * H2, oy = p / H2, ox = p - oy * H2;
+                    float acc[8];
+#pragma unroll
+                    for (int c = 0; c < 8; ++c) acc[c] = w[OFF_B2 + half * 8 + c];
+#pragma unroll 4
+                    for (int ci = 0; ci < C1; ++ci)
+#pragma unroll
+                        for (int kh = 0; kh < 2; ++kh)
+#pragma unroll
+                            for (int kw = 0; kw < 2; ++kw) {
+                                const float x = h1[ci * H1 * H1 + (2 * oy + kh) * H1 + 2 * ox + kw];
+                                const float4* wp = (const float4*)(w + OFF_W2 + (ci * 4 + kh * 2 + kw) * C2 + half * 8);
+                                const float4 u = wp[0], v = wp[1];
+                                acc[0] = __fmaf_rn(u.x, x, acc[0]); acc[1] = __fmaf_rn(u.y, x, acc[1]);
+                                acc[2] = __fmaf_rn(u.z, x, acc[2]); acc[3] = __fmaf_rn(u.w, x, acc[3]);
+                                acc[4] = __fmaf_rn(v.x, x, acc[4]); acc[5] = __fmaf_rn(v.y, x, acc[5]);
+                                acc[6] = __fmaf_rn(v.z, x, acc[6]); acc[7] = __fmaf_rn(v.w, x, acc[7]);
+                            }
+#pragma unroll
+                    for (int c = 0; c < 8; ++c) h2[(half * 8 + c) * H2 * H2 + p] = fmaxf(acc[c], 0.f);
+                }
+                __syncthreads();
+                {   // actor_linear: strided partial sums, warp tree, then 7 warp sums in order
+                    float s0 = 0.f, s1 = 0.f, s2 = 0.f;
+                    for (int f = tid; f < FEATS; f += THREADS) {
+                        const float x = h2[f];
+                        s0 = __fmaf_rn(w[OFF_WA + f], x, s0);
+                        s1 = __fmaf_rn(w[OFF_WA + FEATS + f], x, s1);
+                        s2 = __fmaf_rn(w[OFF_WA + 2 * FEATS + f], x, s2);
+                    }
+#pragma unroll
+                    for (int o = 16; o > 0; o >>= 1) {
+                        s0 += __shfl_xor_sync(0xffffffffu, s0, o);
+                        s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+                        s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+                    }
+                    if ((tid & 31) == 0) {
+                        red[3 * (tid >> 5)] = s0; red[3 * (tid >> 5) + 1] = s1; red[3 * (tid >> 5) + 2] = s2;
+                    }
+                }
+                __syncthreads();
+                if (tid == 0) {
+                    float l[3];
+#pragma unroll
+                    for (int k = 0; k < 3; ++k) {
+                        float v = 0.f;
+                        for (int wi = 0; wi < THREADS / 32; ++wi) v += red[3 * wi + k];
+                        l[k] = v + w[OFF_BA + k];
+                    }
+                    int act = 0;                       // argmax, ties to the lowest index
+                    float best = l[0];
+                    if (l[1] > best) { act = 1; best = l[1]; }
+                    if (l[2] > best) act = 2;
+                    a.actions[2 * i + 1] = act;
+                    if (a.logits) { a.logits[3 * i] = l[0]; a.logits[3 * i + 1] = l[1]; a.logits[3 * i + 2] = l[2]; }
+                }
+            }
+            __syncthreads();   // thread 0 is done with this slot's bias before the next slot's weights arrive
+        }
+    }
+}
+
+// explicit assignment (ids already validated on the host) or a draw from the pool for every env
+__global__ void pong_opp_draw_kernel(const OppArgs a) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < a.n) a.ids[i] = opp_draw(a, a.first_env + i, a.episodes[i]);
+}
+
+}  // namespace opp
+}  // namespace crl
+
+using namespace crl::opp;
+
+struct crl_pong_opp {
+    int n = 0, device = 0, grid = 0;
+    uint64_t seed = 0;
+    int64_t first_env = 0;
+    uint64_t steps = 0;
+    int phase = 0;
+    int pool_size = 0;
+    bool assigned = false;
+    bool loaded[CRL_PONG_OPP_SLOTS] = {};
+    int8_t kind[CRL_PONG_OPP_MAX_POOL] = {};
+    uint64_t cum[CRL_PONG_OPP_MAX_POOL] = {};
+    float* nets = nullptr;
+    int32_t* ids = nullptr;
+    uint8_t* stack = nullptr;
+    float* ret = nullptr;
+    uint32_t* episodes = nullptr;
+    unsigned long long* stats = nullptr;
+};
+
+static OppArgs opp_args(const crl_pong_opp* h) {
+    OppArgs a;
+    memset(&a, 0, sizeof a);
+    a.n = h->n; a.pool_size = h->pool_size; a.phase = h->phase; a.first_env = h->first_env; a.seed = h->seed; a.step = h->steps;
+    memcpy(a.kind, h->kind, sizeof a.kind);
+    memcpy(a.cum, h->cum, sizeof a.cum);
+    a.ids = h->ids; a.stack = h->stack; a.ret = h->ret; a.episodes = h->episodes; a.stats = h->stats; a.nets = h->nets;
+    return a;
+}
+
+#define CHECK_OPP(h)                                                      \
+    if (!(h)) return crl_set_error(CRL_E_INVALID, "null handle");         \
+    CrlDeviceGuard guard((h)->device);                                    \
+    CUDA_TRY(guard.err)
+
+extern "C" {
+
+int crl_pong_opp_destroy(crl_pong_opp* h) {
+    if (!h) return CRL_OK;
+    CrlDeviceGuard guard(h->device);
+    for (void* p : {(void*)h->nets, (void*)h->ids, (void*)h->stack, (void*)h->ret, (void*)h->episodes, (void*)h->stats})
+        if (p) cudaFree(p);
+    delete h;
+    return CRL_OK;
+}
+
+int crl_pong_opp_create(int32_t num_envs, int32_t device, uint64_t seed, int64_t first_env, crl_pong_opp** out) {
+    if (!out) return crl_set_error(CRL_E_INVALID, "null argument");
+    *out = nullptr;
+    if (num_envs <= 0) return crl_set_error(CRL_E_INVALID, "num_envs must be positive");
+    int ndev = 0;
+    cudaError_t e = cudaGetDeviceCount(&ndev);
+    if (e != cudaSuccess || ndev == 0)
+        return crl_set_error(CRL_E_CUDA, "no CUDA device available (%s); this library has no CPU path", cudaGetErrorString(e));
+    if (device < 0 || device >= ndev) return crl_set_error(CRL_E_INVALID, "device %d out of range", device);
+    CrlDeviceGuard guard(device);
+    CUDA_TRY(guard.err);
+    crl_pong_opp* h = new crl_pong_opp();
+    h->n = num_envs; h->device = device; h->seed = seed; h->first_env = first_env;
+    const size_t n = (size_t)num_envs;
+    int sms = 0, per_sm = 0;
+    cudaError_t err = cudaMalloc(&h->nets, sizeof(float) * NET_DEV * CRL_PONG_OPP_SLOTS);
+    if (err == cudaSuccess) err = cudaMalloc(&h->ids, sizeof(int32_t) * n);
+    if (err == cudaSuccess) err = cudaMalloc(&h->stack, (size_t)STACK * FRAME * n);
+    if (err == cudaSuccess) err = cudaMalloc(&h->ret, sizeof(float) * n);
+    if (err == cudaSuccess) err = cudaMalloc(&h->episodes, sizeof(uint32_t) * n);
+    if (err == cudaSuccess) err = cudaMalloc(&h->stats, sizeof(unsigned long long) * 4 * CRL_PONG_OPP_MAX_POOL);
+    if (err == cudaSuccess) err = cudaMemset(h->nets, 0, sizeof(float) * NET_DEV * CRL_PONG_OPP_SLOTS);
+    if (err == cudaSuccess) err = cudaMemset(h->ids, 0, sizeof(int32_t) * n);
+    if (err == cudaSuccess) err = cudaMemset(h->stack, 0, (size_t)STACK * FRAME * n);
+    if (err == cudaSuccess) err = cudaMemset(h->ret, 0, sizeof(float) * n);
+    if (err == cudaSuccess) err = cudaMemset(h->episodes, 0, sizeof(uint32_t) * n);
+    if (err == cudaSuccess) err = cudaMemset(h->stats, 0, sizeof(unsigned long long) * 4 * CRL_PONG_OPP_MAX_POOL);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(pong_opp_act_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
+    if (err == cudaSuccess) err = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    if (err == cudaSuccess) err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pong_opp_act_kernel, THREADS, SMEM_BYTES);
+    if (err == cudaSuccess) err = cudaDeviceSynchronize();
+    if (err != cudaSuccess) {
+        crl_pong_opp_destroy(h);
+        return crl_set_error(CRL_E_CUDA, "crl_pong_opp_create: %s", cudaGetErrorString(err));
+    }
+    // one resident wave: every CTA owns an equal contiguous range of envs
+    h->grid = (int)std::min<int64_t>((int64_t)std::max(per_sm, 1) * sms, num_envs);
+    *out = h;
+    return CRL_OK;
+}
+
+int crl_pong_opp_seed(crl_pong_opp* h, uint64_t seed) {
+    if (!h) return crl_set_error(CRL_E_INVALID, "null handle");
+    h->seed = seed;
+    return CRL_OK;
+}
+
+int crl_pong_opp_load_net(crl_pong_opp* h, int32_t slot, const float* params_host, size_t count, void* stream) {
+    CHECK_OPP(h);
+    if (slot < 0 || slot >= CRL_PONG_OPP_SLOTS) return crl_set_error(CRL_E_INVALID, "network slot must be in [0, %d)", CRL_PONG_OPP_SLOTS);
+    if (!params_host || count != (size_t)CRL_PONG_OPP_NET_FLOATS)
+        return crl_set_error(CRL_E_INVALID, "a LightActorCritic parameter image has %d floats (got %zu)", CRL_PONG_OPP_NET_FLOATS, count);
+    for (size_t k = 0; k < count; ++k)
+        if (!std::isfinite(params_host[k])) return crl_set_error(CRL_E_INVALID, "network parameter %zu is not finite", k);
+    std::vector<float> img(NET_DEV, 0.f);
+    const float* p = params_host;
+    for (int co = 0; co < C1; ++co)
+        for (int t = 0; t < 64; ++t) img[OFF_W1 + t * C1 + co] = p[SD_W1 + co * 64 + t];     // [co][ci][kh][kw] -> [tap][co]
+    for (int co = 0; co < C1; ++co) img[OFF_B1 + co] = p[SD_B1 + co];
+    for (int co = 0; co < C2; ++co)
+        for (int t = 0; t < 64; ++t) img[OFF_W2 + t * C2 + co] = p[SD_W2 + co * 64 + t];     // [co][ci][kh][kw], 16 x 4 taps
+    for (int co = 0; co < C2; ++co) img[OFF_B2 + co] = p[SD_B2 + co];
+    for (int k = 0; k < 3 * FEATS; ++k) img[OFF_WA + k] = p[SD_WA + k];
+    for (int k = 0; k < 3; ++k) img[OFF_BA + k] = p[SD_BA + k];
+    CUDA_TRY(cudaMemcpyAsync(h->nets + (size_t)slot * NET_DEV, img.data(), sizeof(float) * NET_DEV, cudaMemcpyHostToDevice,
+                             (cudaStream_t)stream));
+    CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
+    h->loaded[slot] = true;
+    return CRL_OK;
+}
+
+int crl_pong_opp_set_pool(crl_pong_opp* h, const int32_t* kinds_host, const double* weights_host, int32_t pool_size, void* stream) {
+    CHECK_OPP(h);
+    if (!kinds_host || pool_size < 1 || pool_size > CRL_PONG_OPP_MAX_POOL)
+        return crl_set_error(CRL_E_INVALID, "a pool has 1 to %d entries", CRL_PONG_OPP_MAX_POOL);
+    double total = 0.0;
+    for (int k = 0; k < pool_size; ++k) {
+        const int kd = kinds_host[k];
+        if (kd != CRL_PONG_OPP_RULE_BASED && kd != CRL_PONG_OPP_RANDOM && (kd < 0 || kd >= CRL_PONG_OPP_SLOTS))
+            return crl_set_error(CRL_E_INVALID, "pool entry %d: kind %d is neither RULE_BASED, RANDOM nor a network slot", k, kd);
+        if (kd >= 0 && !h->loaded[kd]) return crl_set_error(CRL_E_STATE, "pool entry %d: network slot %d was never loaded", k, kd);
+        const double wk = weights_host ? weights_host[k] : 1.0;
+        if (!(wk >= 0.0) || !std::isfinite(wk)) return crl_set_error(CRL_E_INVALID, "pool entry %d: weight must be finite and >= 0", k);
+        total += wk;
+    }
+    if (!(total > 0.0)) return crl_set_error(CRL_E_INVALID, "the pool's weights sum to 0");
+    double run = 0.0;
+    int last = 0;
+    for (int k = 0; k < pool_size; ++k)
+        if ((weights_host ? weights_host[k] : 1.0) > 0.0) last = k;
+    for (int k = 0; k < CRL_PONG_OPP_MAX_POOL; ++k) {
+        h->kind[k] = k < pool_size ? (int8_t)kinds_host[k] : (int8_t)CRL_PONG_OPP_RULE_BASED;
+        if (k < pool_size) run += weights_host ? weights_host[k] : 1.0;
+        // r32 < cum[k] picks entry k first: a zero weight repeats the previous bound and is never drawn
+        h->cum[k] = k >= last ? (1ull << 32) : (uint64_t)std::floor(run / total * 4294967296.0);
+    }
+    h->pool_size = pool_size;
+    h->assigned = false;
+    CUDA_TRY(cudaMemsetAsync(h->stats, 0, sizeof(unsigned long long) * 4 * CRL_PONG_OPP_MAX_POOL, (cudaStream_t)stream));
+    return CRL_OK;
+}
+
+int crl_pong_opp_assign(crl_pong_opp* h, const int32_t* ids_host, void* stream) {
+    CHECK_OPP(h);
+    if (h->pool_size == 0) return crl_set_error(CRL_E_STATE, "crl_pong_opp_set_pool first");
+    if (ids_host) {
+        for (int i = 0; i < h->n; ++i)
+            if (ids_host[i] < 0 || ids_host[i] >= h->pool_size)
+                return crl_set_error(CRL_E_INVALID, "env %d: opponent id %d is not in [0, %d)", i, ids_host[i], h->pool_size);
+        CUDA_TRY(cudaMemcpyAsync(h->ids, ids_host, sizeof(int32_t) * h->n, cudaMemcpyHostToDevice, (cudaStream_t)stream));
+        CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
+    } else {
+        LAUNCH((pong_opp_draw_kernel<<<(h->n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(opp_args(h)), cudaGetLastError()));
+    }
+    h->assigned = true;
+    return CRL_OK;
+}
+
+int crl_pong_opp_restart(crl_pong_opp* h, int32_t clear_stacks, void* stream) {
+    CHECK_OPP(h);
+    CUDA_TRY(cudaMemsetAsync(h->ret, 0, sizeof(float) * h->n, (cudaStream_t)stream));
+    if (clear_stacks) {
+        CUDA_TRY(cudaMemsetAsync(h->stack, 0, (size_t)STACK * FRAME * h->n, (cudaStream_t)stream));
+        h->phase = 0;
+    }
+    return CRL_OK;
+}
+
+int crl_pong_opp_act(crl_pong_opp* h, const uint8_t* obs1_dev, const float* rew_dev, const uint8_t* done_dev, int32_t resample,
+                     int32_t* actions_dev, float* logits_dev, void* stream) {
+    CHECK_OPP(h);
+    if (!h->assigned) return crl_set_error(CRL_E_STATE, "crl_pong_opp_assign after every crl_pong_opp_set_pool");
+    if (!obs1_dev || !actions_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
+    if ((rew_dev == nullptr) != (done_dev == nullptr)) return crl_set_error(CRL_E_INVALID, "rew_dev and done_dev go together");
+    if (((uintptr_t)obs1_dev & 3) != 0) return crl_set_error(CRL_E_INVALID, "obs1_dev must be 4-byte aligned");
+    OppArgs a = opp_args(h);
+    a.resample = resample ? 1 : 0;
+    a.obs1 = obs1_dev; a.rew = rew_dev; a.done = done_dev; a.actions = actions_dev; a.logits = logits_dev;
+    LAUNCH((pong_opp_act_kernel<<<h->grid, THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(a), cudaGetLastError()));
+    h->phase = (h->phase + 1) & 3;
+    h->steps += 1;
+    return CRL_OK;
+}
+
+int crl_pong_opp_get_ids(crl_pong_opp* h, int32_t* ids_dev, void* stream) {
+    CHECK_OPP(h);
+    if (!ids_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
+    CUDA_TRY(cudaMemcpyAsync(ids_dev, h->ids, sizeof(int32_t) * h->n, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    return CRL_OK;
+}
+
+int crl_pong_opp_get_stats(crl_pong_opp* h, uint64_t* stats_host, void* stream) {
+    CHECK_OPP(h);
+    if (!stats_host) return crl_set_error(CRL_E_INVALID, "null buffer");
+    unsigned long long raw[4 * CRL_PONG_OPP_MAX_POOL];
+    CUDA_TRY(cudaMemcpyAsync(raw, h->stats, sizeof raw, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+    CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
+    for (int k = 0; k < 4 * CRL_PONG_OPP_MAX_POOL; ++k) stats_host[k] = raw[k];
+    return CRL_OK;
+}
+
+}  // extern "C"

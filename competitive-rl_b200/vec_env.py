@@ -263,6 +263,7 @@ class CudaPongVecEnv(VecEnv):
         self.copy = bool(copy)
         self.stack_mode = stack_mode
         self.ring = stack_mode == "ring"
+        self.first_env = int(first_env)
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())

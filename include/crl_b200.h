@@ -197,6 +197,69 @@ int crl_obs_alloc(int32_t device, size_t bytes, void** ptr, int32_t* compressed)
 int crl_obs_free(void* ptr);
 
 /* ======================================================================================
+ * cPongTournament-v0 per-env opponents
+ * The reference's TournamentEnvWrapper (pong/competitive_pong_env.py:9-53) lets ONE built-in opponent play every env of
+ * the batch.  A crl_pong_opp handle lets every env of a 42x42 cPongDouble shard play its own opponent, drawn from a
+ * pool, in one kernel launch per step (crl_pong_opp_act), with no host synchronisation.
+ *
+ *   Pool        1..16 entries; an entry is CRL_PONG_OPP_RULE_BASED, CRL_PONG_OPP_RANDOM, or one of 8 network slots
+ *               holding a LightActorCritic (utils/network.py:73-93: 4x42x42 -> conv 4x4/2 (16) -> conv 2x2/2 (16) ->
+ *               1600 -> 3 logits).  ActorCritic networks are not supported.
+ *   Assignment  int32 opponent id per env (an index into the pool): given explicitly, or drawn with the pool's weights
+ *               from Philox keyed by (seed, global env index first_env + i, the env's count of finished episodes), so
+ *               draws do not depend on the sharding.
+ *   Stack       uint8 [num_envs][4][42][42] per handle, oldest -> newest, zero at creation.  Every act pushes agent 1's
+ *               observation of the previous step, whatever the env's opponent is; done does not clear it (the
+ *               reference's policy_serving.Policy stack is never cleared either).
+ *   Action      written into column 1 of the caller's int32 [num_envs][2] step buffer (column 0 is the learner's):
+ *               RULE_BASED 999; RANDOM a Philox-uniform draw from {0, 1, 2} keyed by (seed, global env index, act
+ *               count); a network the argmax (ties: lowest index) of its actor logits over stack / 255 in fp32.
+ *   Episodes    act receives the previous step's reward and done.  Agent 0's clipped rewards are summed per env; an env
+ *               that finished credits the episode to the pool entry it played (agent 0 wins when the sum is > 0,
+ *               draws at 0, loses below: pong/evaluate.py:53-88) and, with resample != 0, draws a new id.
+ * ====================================================================================== */
+#define CRL_PONG_OPP_MAX_POOL 16
+#define CRL_PONG_OPP_SLOTS 8
+#define CRL_PONG_OPP_RULE_BASED (-1)   /* pool entry kinds; 0 .. CRL_PONG_OPP_SLOTS-1 = network slot */
+#define CRL_PONG_OPP_RANDOM (-2)
+/* LightActorCritic parameters in state-dict order, each row-major: conv1.weight [16][4][4][4], conv1.bias [16],
+ * conv2.weight [16][16][2][2], conv2.bias [16], critic_linear.weight [1][1600], critic_linear.bias [1],
+ * actor_linear.weight [3][1600], actor_linear.bias [3] (the critic is carried but not evaluated) */
+#define CRL_PONG_OPP_NET_FLOATS 8484
+
+typedef struct crl_pong_opp crl_pong_opp; /* opaque handle: the opponents of one shard of envs on one GPU */
+
+/* seed keys the draws and RANDOM's actions; first_env is the global index of env 0 of the shard */
+int crl_pong_opp_create(int32_t num_envs, int32_t device, uint64_t seed, int64_t first_env, crl_pong_opp** out);
+int crl_pong_opp_destroy(crl_pong_opp* h);
+/* re-keys future draws and RANDOM actions; no device work */
+int crl_pong_opp_seed(crl_pong_opp* h, uint64_t seed);
+/* network slot <- params_host[CRL_PONG_OPP_NET_FLOATS] (finite).  Synchronises the stream. */
+int crl_pong_opp_load_net(crl_pong_opp* h, int32_t slot, const float* params_host, size_t count, void* stream);
+/* pool <- kinds_host[pool_size] (RULE_BASED, RANDOM or a loaded slot) with draw weights weights_host[pool_size] (>= 0,
+ * not all 0; NULL = uniform).  Zeroes the per-entry statistics; crl_pong_opp_assign must follow before the next act. */
+int crl_pong_opp_set_pool(crl_pong_opp* h, const int32_t* kinds_host, const double* weights_host, int32_t pool_size,
+                          void* stream);
+/* every env's opponent id <- ids_host[num_envs] (validated; synchronises), or drawn from the pool (ids_host NULL) */
+int crl_pong_opp_assign(crl_pong_opp* h, const int32_t* ids_host, void* stream);
+/* restarts the per-env reward sums (VecEnv.reset); clear_stacks != 0 also zeroes every frame stack */
+int crl_pong_opp_restart(crl_pong_opp* h, int32_t clear_stacks, void* stream);
+/* One step's opponents, before crl_pong_step:
+ *   obs1_dev     uint8 [num_envs][42][42] agent 1's observation of the previous step (frame_stack None), 4-byte aligned
+ *   rew_dev      float32 [num_envs][2] and done_dev uint8 [num_envs] of the previous step, or both NULL for the first
+ *                act after a reset (no episode bookkeeping)
+ *   resample     != 0: envs whose previous step ended an episode draw a new opponent id before acting
+ *   actions_dev  int32 [num_envs][2]: column 1 receives the opponents' actions, column 0 is not touched
+ *   logits_dev   float32 [num_envs][3] or NULL: the network envs' actor logits (0 for the other kinds) */
+int crl_pong_opp_act(crl_pong_opp* h, const uint8_t* obs1_dev, const float* rew_dev, const uint8_t* done_dev, int32_t resample,
+                     int32_t* actions_dev, float* logits_dev, void* stream);
+/* ids_dev int32 [num_envs] <- every env's current opponent id */
+int crl_pong_opp_get_ids(crl_pong_opp* h, int32_t* ids_dev, void* stream);
+/* stats_host uint64 [16][4]: per pool entry, episodes finished against it, agent 0's wins, draws, losses (since the
+ * last crl_pong_opp_set_pool).  Synchronises the stream. */
+int crl_pong_opp_get_stats(crl_pong_opp* h, uint64_t* stats_host, void* stream);
+
+/* ======================================================================================
  * cCarRacing-v0 / cCarRacingDouble-v0
  * Replaces the env stack built by make_car_racing / make_car_racing_double
  * (car_racing/register.py:29-53): gym.make(id) [TimeLimit(1000)] -> FrameStack |
