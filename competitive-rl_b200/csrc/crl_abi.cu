@@ -23,14 +23,6 @@ using namespace crl;
 static thread_local char g_err[512] = "";
 static std::atomic<uint64_t> g_launches{0};
 
-static int fail(int code, const char* fmt, ...) {
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_err, sizeof g_err, fmt, ap);
-    va_end(ap);
-    return code;
-}
-
 int crl_set_error(int code, const char* fmt, ...) {
     va_list ap;
     va_start(ap, fmt);
@@ -40,23 +32,10 @@ int crl_set_error(int code, const char* fmt, ...) {
 }
 void crl_count_launch(int n) { g_launches += (uint64_t)n; }
 
-#define CUDA_TRY(expr)                                                                                \
-    do {                                                                                              \
-        cudaError_t _e = (expr);                                                                      \
-        if (_e != cudaSuccess) return fail(CRL_E_CUDA, "%s: %s", #expr, cudaGetErrorString(_e));      \
-    } while (0)
-
-#define LAUNCH(expr)     \
-    do {                 \
-        CUDA_TRY(expr);  \
-        g_launches += 1; \
-    } while (0)
-
 struct crl_pong {
     crl_pong_config cfg;
     PongDev dev;
-    std::vector<void*> allocs;
-    double* serves_dev = nullptr;
+    DeviceAllocs allocs;
     uint8_t* atlas_dev = nullptr;
     uint8_t* text_tab_dev = nullptr;
     uint8_t* tmpl_dev = nullptr;
@@ -71,8 +50,7 @@ struct crl_pong {
     bool atlas_loaded = false;
     bool was_reset = false;
     // crl_pong_step_host: the small results go back to the host on a side stream while the rasteriser runs
-    cudaStream_t copy_stream = nullptr;
-    cudaEvent_t ev_state = nullptr, ev_copied = nullptr;
+    SideStream copy;
     // crl_pong_set_obs_buffers: observation buffers whose contents the library tracks.  shown ([agent][c][n] FrameSpecs per
     // set) describes what the set's buffers hold while `valid`; renders into a valid set store only what changed.
     struct ObsSet {
@@ -146,16 +124,6 @@ static bool build_tabs(int dim, AreaTabs* t) {
     return true;
 }
 
-template <typename T>
-static cudaError_t dev_alloc(crl_pong* h, T** p, size_t count) {
-    void* q = nullptr;
-    cudaError_t e = cudaMalloc(&q, count * sizeof(T) + 16);
-    if (e != cudaSuccess) return e;
-    h->allocs.push_back(q);
-    *p = (T*)q;
-    return cudaMemset(q, 0, count * sizeof(T) + 16);
-}
-
 extern "C" {
 
 int crl_abi_version(void) { return CRL_ABI_VERSION; }
@@ -165,39 +133,32 @@ uint64_t crl_launch_count(void) { return g_launches.load(); }
 int crl_pong_destroy(crl_pong* h) {
     if (!h) return CRL_OK;
     CrlDeviceGuard guard(h->cfg.device);
-    for (void* p : h->allocs) cudaFree(p);
-    if (h->shown_dev) cudaFree(h->shown_dev);
-    if (h->ev_state) cudaEventDestroy(h->ev_state);
-    if (h->ev_copied) cudaEventDestroy(h->ev_copied);
-    if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
+    h->copy.sync();
+    h->allocs.free_all();
+    h->copy.destroy();
     delete h;
     return CRL_OK;
 }
 
 int crl_pong_create(const crl_pong_config* cfg, crl_pong** out) {
-    if (!cfg || !out) return fail(CRL_E_INVALID, "null argument");
+    if (!cfg || !out) return crl_set_error(CRL_E_INVALID, "null argument");
     *out = nullptr;
-    if (cfg->num_envs <= 0) return fail(CRL_E_INVALID, "num_envs must be positive");
-    if (cfg->n_agents != 1 && cfg->n_agents != 2) return fail(CRL_E_INVALID, "n_agents must be 1 or 2");
+    if (cfg->num_envs <= 0) return crl_set_error(CRL_E_INVALID, "num_envs must be positive");
+    if (cfg->n_agents != 1 && cfg->n_agents != 2) return crl_set_error(CRL_E_INVALID, "n_agents must be 1 or 2");
     if (cfg->resized_dim < 8 || cfg->resized_dim > MAX_DIM || cfg->resized_dim % 2)
-        return fail(CRL_E_INVALID, "resized_dim must be even and in [8, %d]", MAX_DIM);
+        return crl_set_error(CRL_E_INVALID, "resized_dim must be even and in [8, %d]", MAX_DIM);
     if (cfg->frame_stack < 0 || cfg->frame_stack > MAX_STACK)
-        return fail(CRL_E_INVALID, "frame_stack must be in [0, %d]", MAX_STACK);
-    if (cfg->stack_mode != 0 && cfg->stack_mode != 1) return fail(CRL_E_INVALID, "stack_mode must be 0 (stack) or 1 (ring)");
-    if (cfg->stack_mode == 1 && cfg->frame_stack < 2) return fail(CRL_E_INVALID, "stack_mode ring needs frame_stack >= 2");
+        return crl_set_error(CRL_E_INVALID, "frame_stack must be in [0, %d]", MAX_STACK);
+    if (cfg->stack_mode != 0 && cfg->stack_mode != 1) return crl_set_error(CRL_E_INVALID, "stack_mode must be 0 (stack) or 1 (ring)");
+    if (cfg->stack_mode == 1 && cfg->frame_stack < 2) return crl_set_error(CRL_E_INVALID, "stack_mode ring needs frame_stack >= 2");
     if (cfg->max_num_rounds < 1 || cfg->max_num_rounds > ATLAS_SCORES - 1)
-        return fail(CRL_E_INVALID, "max_num_rounds must be in [1, %d] (scoreboard atlas range)", ATLAS_SCORES - 1);
-    int ndev = 0;
-    cudaError_t e = cudaGetDeviceCount(&ndev);
-    if (e != cudaSuccess || ndev == 0)
-        return fail(CRL_E_CUDA, "no CUDA device available (%s); this library has no CPU path",
-                    cudaGetErrorString(e));
-    if (cfg->device < 0 || cfg->device >= ndev) return fail(CRL_E_INVALID, "device %d out of range", cfg->device);
+        return crl_set_error(CRL_E_INVALID, "max_num_rounds must be in [1, %d] (scoreboard atlas range)", ATLAS_SCORES - 1);
+    if (int r = crl_check_device(cfg->device)) return r;
     CrlDeviceGuard guard(cfg->device);
     CUDA_TRY(guard.err);
     AreaTabs tabs;
     if (!build_tabs(cfg->resized_dim, &tabs))
-        return fail(CRL_E_INVALID, "resized_dim %d needs more than %d taps per pixel", cfg->resized_dim, MAX_TAPS);
+        return crl_set_error(CRL_E_INVALID, "resized_dim %d needs more than %d taps per pixel", cfg->resized_dim, MAX_TAPS);
 
     crl_pong* h = new crl_pong();
     h->cfg = *cfg;
@@ -217,73 +178,62 @@ int crl_pong_create(const crl_pong_config* cfg, crl_pong** out) {
     d.text_stride = ((tabs.text_rows * d.dim + 15) / 16) * 16;
     if (d.text_stride > ((dd + 15) / 16) * 16) d.text_stride = ((dd + 15) / 16) * 16;
     d.text_w0 = 0; d.text_w1 = d.text_stride / 4;
-#define ALLOC(ptr, count)                                                        \
-    do {                                                                         \
-        cudaError_t _e = dev_alloc(h, &(ptr), (count));                          \
-        if (_e != cudaSuccess) {                                                 \
-            crl_pong_destroy(h);                                                 \
-            return fail(CRL_E_CUDA, "cudaMalloc: %s", cudaGetErrorString(_e));   \
-        }                                                                        \
-    } while (0)
-    ALLOC(d.ball, n); ALLOC(d.vx, n); ALLOC(d.vy, n); ALLOC(d.bats, n); ALLOC(d.score, n);
-    ALLOC(d.num_steps, n); ALLOC(d.clip_steps, n); ALLOC(d.serve_count, n); ALLOC(d.last_done, n);
-    ALLOC(d.skipbuf, 2 * n); ALLOC(d.hist, d.c * n); ALLOC(d.term_hist, d.c * n);
-    ALLOC(d.serve_overrun, 1);
-    ALLOC(d.stats, 8);
-    ALLOC(d.work_counter, 2);
-    ALLOC(h->tabs_dev, 1);
-    ALLOC(h->atlas_dev, (size_t)CRL_PONG_ATLAS_BYTES);
-    ALLOC(h->text_tab_dev, (size_t)ATLAS_SCORES * ATLAS_SCORES * 3 * 2 * d.text_stride);
-    ALLOC(h->tmpl_dev, (size_t)((dd + 15) / 16) * 16);
-    ALLOC(h->actions_stage, 2 * n); ALLOC(h->rew_stage, 2 * n); ALLOC(h->done_stage, n);
-    ALLOC(h->steps_stage, n); ALLOC(h->real_stage, 2 * n);
-    h->tabs_host = tabs;
+    cudaError_t e = cudaSuccess;
+    auto alloc = [&](auto** p, size_t count) { if (e == cudaSuccess) e = h->allocs.alloc(p, count); };
+    alloc(&d.ball, n); alloc(&d.vx, n); alloc(&d.vy, n); alloc(&d.bats, n); alloc(&d.score, n);
+    alloc(&d.num_steps, n); alloc(&d.clip_steps, n); alloc(&d.serve_count, n); alloc(&d.last_done, n);
+    alloc(&d.skipbuf, 2 * n); alloc(&d.hist, d.c * n); alloc(&d.term_hist, d.c * n);
+    alloc(&d.serve_overrun, 1);
+    alloc(&d.stats, 8);
+    alloc(&d.work_counter, 2);
+    alloc(&h->tabs_dev, 1);
+    alloc(&h->atlas_dev, (size_t)CRL_PONG_ATLAS_BYTES);
+    alloc(&h->text_tab_dev, (size_t)ATLAS_SCORES * ATLAS_SCORES * 3 * 2 * d.text_stride);
+    alloc(&h->tmpl_dev, (size_t)((dd + 15) / 16) * 16);
+    alloc(&h->actions_stage, 2 * n); alloc(&h->rew_stage, 2 * n); alloc(&h->done_stage, n);
+    alloc(&h->steps_stage, n); alloc(&h->real_stage, 2 * n);
     const size_t ftb = pong_fast_tabs_bytes(d.dim);
-    if (ftb) {
-        std::vector<uint8_t> img(ftb);
-        if (pong_fast_tabs_fill(tabs, d.text_stride, img.data())) {
-            ALLOC(h->fast_tabs_dev, ftb);
-            cudaError_t _e = cudaMemcpy(h->fast_tabs_dev, img.data(), ftb, cudaMemcpyHostToDevice);
-            if (_e == cudaSuccess) _e = launch_pong_build_bat_lut(d.dim, h->fast_tabs_dev, 0);
-            if (_e != cudaSuccess) {
-                crl_pong_destroy(h);
-                return fail(CRL_E_CUDA, "fast tabs upload: %s", cudaGetErrorString(_e));
-            }
-            g_launches += 1;
-            d.fast_tabs = h->fast_tabs_dev;
-            d.quad_ok = (pong_quad_ok(tabs) && getenv("CRL_PONG_NO_QUAD") == nullptr) ? 1 : 0;
-            h->full_obs = getenv("CRL_PONG_FULL_OBS") != nullptr;   // A/B switch: no incremental stacks
+    std::vector<uint8_t> img(ftb);
+    const bool fast = ftb && pong_fast_tabs_fill(tabs, d.text_stride, img.data());
+    if (fast) alloc(&h->fast_tabs_dev, ftb);
+    if (e != cudaSuccess) {
+        crl_pong_destroy(h);
+        return crl_set_error(CRL_E_CUDA, "cudaMalloc: %s", cudaGetErrorString(e));
+    }
+    h->tabs_host = tabs;
+    if (fast) {
+        e = cudaMemcpy(h->fast_tabs_dev, img.data(), ftb, cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) e = launch_pong_build_bat_lut(d.dim, h->fast_tabs_dev, 0);
+        if (e != cudaSuccess) {
+            crl_pong_destroy(h);
+            return crl_set_error(CRL_E_CUDA, "fast tabs upload: %s", cudaGetErrorString(e));
         }
+        crl_count_launch(1);
+        d.fast_tabs = h->fast_tabs_dev;
+        d.quad_ok = (pong_quad_ok(tabs) && getenv("CRL_PONG_NO_QUAD") == nullptr) ? 1 : 0;
+        h->full_obs = getenv("CRL_PONG_FULL_OBS") != nullptr;   // A/B switch: no incremental stacks
     }
     d.tabs = h->tabs_dev;
     d.atlas = h->atlas_dev;
     d.text_tab = h->text_tab_dev;
     d.tmpl = h->tmpl_dev;
-#undef ALLOC
     e = cudaMemcpy(h->tabs_dev, &tabs, sizeof tabs, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = pong_raster_init(d.raster_grid);
     if (e == cudaSuccess) e = launch_pong_construct(d, 0);
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
         crl_pong_destroy(h);
-        return fail(CRL_E_CUDA, "construct: %s", cudaGetErrorString(e));
+        return crl_set_error(CRL_E_CUDA, "construct: %s", cudaGetErrorString(e));
     }
-    g_launches += 1;
+    crl_count_launch(1);
     *out = h;
     return CRL_OK;
 }
 
-#define CHECK_HANDLE(h)                                        \
-    do {                                                       \
-        if (!(h)) return fail(CRL_E_INVALID, "null handle");   \
-    } while (0);                                               \
-    CrlDeviceGuard crl_guard_((h)->cfg.device);                \
-    CUDA_TRY(crl_guard_.err)
-
 int crl_pong_load_atlas(crl_pong* h, const uint8_t* strips_host, size_t bytes, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!strips_host || bytes != (size_t)CRL_PONG_ATLAS_BYTES)
-        return fail(CRL_E_INVALID, "atlas must be %d bytes ([22][22][34][160][3] uint8)", CRL_PONG_ATLAS_BYTES);
+        return crl_set_error(CRL_E_INVALID, "atlas must be %d bytes ([22][22][34][160][3] uint8)", CRL_PONG_ATLAS_BYTES);
     cudaStream_t s = (cudaStream_t)stream;
     // The hot kernel treats source rows above the arena that share a destination row with arena
     // rows as pure white (true for any scoreboard that stays clear of the arena edge); otherwise
@@ -301,7 +251,7 @@ int crl_pong_load_atlas(crl_pong* h, const uint8_t* strips_host, size_t bytes, v
         h->dev.fast_ok = white ? 1 : 0;
     }
     CUDA_TRY(cudaMemcpyAsync(h->atlas_dev, strips_host, bytes, cudaMemcpyHostToDevice, s));
-    LAUNCH(launch_pong_build_tables(h->dev, h->text_tab_dev, h->tmpl_dev, s));
+    LAUNCH(launch_pong_build_tables(h->dev, h->text_tab_dev, h->tmpl_dev, s), 1);
     CUDA_TRY(cudaStreamSynchronize(s));
     {   // The words of a scoreboard entry that differ between entries (any score pair, kind, agent) or from the template: the
         // score digits cover a few of the rows above the arena only, and the rest of an entry never needs copying.
@@ -326,37 +276,38 @@ int crl_pong_load_atlas(crl_pong* h, const uint8_t* strips_host, size_t bytes, v
 }
 
 int crl_pong_inject_serves(crl_pong* h, const double* serves_host, int32_t k, void* stream) {
-    CHECK_HANDLE(h);
-    if (!serves_host || k < 3) return fail(CRL_E_INVALID, "serve table needs k >= 3 entries per env");
+    CHECK_HANDLE(h, h->cfg.device);
+    if (!serves_host || k < 3) return crl_set_error(CRL_E_INVALID, "serve table needs k >= 3 entries per env");
     cudaStream_t s = (cudaStream_t)stream;
     double* buf = nullptr;
-    CUDA_TRY(dev_alloc(h, &buf, (size_t)h->dev.n * k * 2));
+    CUDA_TRY(h->allocs.alloc(&buf, (size_t)h->dev.n * k * 2));
     CUDA_TRY(cudaMemcpyAsync(buf, serves_host, (size_t)h->dev.n * k * 2 * sizeof(double), cudaMemcpyHostToDevice, s));
-    h->serves_dev = buf;
+    const double* old = h->dev.serves;
     h->dev.serves = buf;
     h->dev.serves_k = k;
-    LAUNCH(launch_pong_construct(h->dev, s));   // constructors re-run: serves 0 and 1 from the table
+    LAUNCH(launch_pong_construct(h->dev, s), 1);   // constructors re-run: serves 0 and 1 from the table
     CUDA_TRY(cudaStreamSynchronize(s));
     h->was_reset = false;
+    CUDA_TRY(h->allocs.free(old));
     return CRL_OK;
 }
 
 int crl_pong_seed(crl_pong* h, uint64_t seed) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     h->dev.seed = seed;
     return CRL_OK;
 }
 
 static int need_ready(crl_pong* h, bool need_reset) {
-    if (!h->atlas_loaded) return fail(CRL_E_STATE, "crl_pong_load_atlas must be called before reset/step");
-    if (need_reset && !h->was_reset) return fail(CRL_E_STATE, "reset must be called before step");
+    if (!h->atlas_loaded) return crl_set_error(CRL_E_STATE, "crl_pong_load_atlas must be called before reset/step");
+    if (need_reset && !h->was_reset) return crl_set_error(CRL_E_STATE, "reset must be called before step");
     return CRL_OK;
 }
 
 int crl_pong_render_obs(crl_pong* h, uint8_t* obs0_dev, uint8_t* obs1_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (int r = need_ready(h, true)) return r;
-    if (!obs0_dev || (h->dev.n_agents == 2 && !obs1_dev)) return fail(CRL_E_INVALID, "null observation buffer");
+    if (!obs0_dev || (h->dev.n_agents == 2 && !obs1_dev)) return crl_set_error(CRL_E_INVALID, "null observation buffer");
     if (h->dev.n_agents == 1) obs1_dev = obs0_dev;
     cudaStream_t s = (cudaStream_t)stream;
     crl_pong::ObsSet* set = nullptr;
@@ -364,10 +315,10 @@ int crl_pong_render_obs(crl_pong* h, uint8_t* obs0_dev, uint8_t* obs1_dev, void*
         if (st.obs[0] == obs0_dev && (h->dev.n_agents == 1 || st.obs[1] == obs1_dev)) set = &st;
     const bool incremental = !h->full_obs && pong_raster_incremental_ok(h->dev, obs0_dev, obs1_dev);
     if (set && set->valid && incremental) {
-        LAUNCH(launch_pong_raster(h->dev, h->dev.hist, obs0_dev, obs1_dev, set->shown, s));
+        LAUNCH(launch_pong_raster(h->dev, h->dev.hist, obs0_dev, obs1_dev, set->shown, s), 1);
         return CRL_OK;
     }
-    LAUNCH(launch_pong_raster(h->dev, h->dev.hist, obs0_dev, obs1_dev, nullptr, s));
+    LAUNCH(launch_pong_raster(h->dev, h->dev.hist, obs0_dev, obs1_dev, nullptr, s), 1);
     if (!set) {
         obs_written(h, obs0_dev, obs_bytes(h));
         obs_written(h, obs1_dev, obs_bytes(h));
@@ -385,94 +336,87 @@ int crl_pong_render_obs(crl_pong* h, uint8_t* obs0_dev, uint8_t* obs1_dev, void*
 
 int crl_pong_set_obs_buffers(crl_pong* h, uint8_t* const* obs0_devs_host, uint8_t* const* obs1_devs_host, int32_t count,
                              void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     const int na = h->dev.n_agents;
     if (count != 0) {
-        if (h->dev.ring) return fail(CRL_E_STATE, "stack_mode ring keeps its own frames: there are no buffer sets to register");
+        if (h->dev.ring) return crl_set_error(CRL_E_STATE, "stack_mode ring keeps its own frames: there are no buffer sets to register");
         if (count < 0 || count > CRL_PONG_MAX_OBS_SETS || !obs0_devs_host || (na == 2 && !obs1_devs_host))
-            return fail(CRL_E_INVALID, "need 1 .. %d buffer sets (and obs1 buffers for cPongDouble), got %d",
-                        CRL_PONG_MAX_OBS_SETS, count);
+            return crl_set_error(CRL_E_INVALID, "need 1 .. %d buffer sets (and obs1 buffers for cPongDouble), got %d",
+                                 CRL_PONG_MAX_OBS_SETS, count);
         std::vector<uint8_t*> all;
         for (int i = 0; i < count; ++i)
             for (int k = 0; k < na; ++k) {
                 uint8_t* b = k ? obs1_devs_host[i] : obs0_devs_host[i];
-                if (!b) return fail(CRL_E_INVALID, "null buffer in set %d", i);
+                if (!b) return crl_set_error(CRL_E_INVALID, "null buffer in set %d", i);
                 for (uint8_t* o : all)
-                    if (o == b) return fail(CRL_E_INVALID, "a buffer appears twice in the sets");
+                    if (o == b) return crl_set_error(CRL_E_INVALID, "a buffer appears twice in the sets");
                 all.push_back(b);
             }
     }
     CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));   // no render in flight reads the old specs
     h->sets.clear();
-    if (h->shown_dev) {
-        CUDA_TRY(cudaFree(h->shown_dev));
-        h->shown_dev = nullptr;
-    }
+    CUDA_TRY(h->allocs.free(h->shown_dev));
+    h->shown_dev = nullptr;
     if (count == 0) return CRL_OK;
     const size_t per_set = (size_t)na * h->dev.c * h->dev.n;
-    CUDA_TRY(cudaMalloc(&h->shown_dev, (size_t)count * per_set * sizeof(FrameSpec)));
+    CUDA_TRY(h->allocs.alloc(&h->shown_dev, (size_t)count * per_set));
     for (int i = 0; i < count; ++i)
         h->sets.push_back({{obs0_devs_host[i], na == 2 ? obs1_devs_host[i] : obs0_devs_host[i]}, h->shown_dev + i * per_set, false});
     return CRL_OK;
 }
 
 int crl_pong_forget_obs(crl_pong* h) {
-    if (!h) return fail(CRL_E_INVALID, "null handle");
+    if (!h) return crl_set_error(CRL_E_INVALID, "null handle");
     for (auto& st : h->sets) st.valid = false;
     return CRL_OK;
 }
 
 int crl_pong_render_obs_generic(crl_pong* h, uint8_t* obs0_dev, uint8_t* obs1_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (int r = need_ready(h, true)) return r;
-    if (!obs0_dev || (h->dev.n_agents == 2 && !obs1_dev)) return fail(CRL_E_INVALID, "null observation buffer");
-    LAUNCH(launch_pong_raster_generic(h->dev, h->dev.hist, nullptr, h->dev.ring, obs0_dev, obs1_dev, (cudaStream_t)stream));
+    if (!obs0_dev || (h->dev.n_agents == 2 && !obs1_dev)) return crl_set_error(CRL_E_INVALID, "null observation buffer");
+    LAUNCH(launch_pong_raster_generic(h->dev, h->dev.hist, nullptr, h->dev.ring, obs0_dev, obs1_dev, (cudaStream_t)stream), 1);
     obs_written(h, obs0_dev, obs_bytes(h));
     obs_written(h, obs1_dev, obs_bytes(h));
     return CRL_OK;
 }
 
 int crl_pong_render_obs_f32(crl_pong* h, int32_t terminal, const uint8_t* only_done_dev, float* obs0_dev, float* obs1_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (int r = need_ready(h, true)) return r;
-    if (h->dev.ring) return fail(CRL_E_STATE, "float32 observations are plain stacks: create the handle with stack_mode 0");
-    if (!obs0_dev || (h->dev.n_agents == 2 && !obs1_dev)) return fail(CRL_E_INVALID, "null observation buffer");
-    LAUNCH(launch_pong_raster_f32(h->dev, terminal ? h->dev.term_hist : h->dev.hist, only_done_dev, obs0_dev, obs1_dev, (cudaStream_t)stream));
+    if (h->dev.ring) return crl_set_error(CRL_E_STATE, "float32 observations are plain stacks: create the handle with stack_mode 0");
+    if (!obs0_dev || (h->dev.n_agents == 2 && !obs1_dev)) return crl_set_error(CRL_E_INVALID, "null observation buffer");
+    LAUNCH(launch_pong_raster_f32(h->dev, terminal ? h->dev.term_hist : h->dev.hist, only_done_dev, obs0_dev, obs1_dev, (cudaStream_t)stream), 1);
     obs_written(h, obs0_dev, 4 * obs_bytes(h));
     obs_written(h, obs1_dev, 4 * obs_bytes(h));
     return CRL_OK;
 }
 
 int crl_pong_reset_state(crl_pong* h, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (int r = need_ready(h, false)) return r;
-    LAUNCH(launch_pong_reset(h->dev, (cudaStream_t)stream));
+    LAUNCH(launch_pong_reset(h->dev, (cudaStream_t)stream), 1);
     h->was_reset = true;
     h->dev.ring_phase = 0;
-    h->dev.fill_all = 1;
+    h->dev.fill_all = 1;      // until the next step: every ring is (re)written completely
     return CRL_OK;
 }
 
 int crl_pong_reset(crl_pong* h, uint8_t* obs0_dev, uint8_t* obs1_dev, void* stream) {
-    CHECK_HANDLE(h);
-    if (int r = need_ready(h, false)) return r;
-    LAUNCH(launch_pong_reset(h->dev, (cudaStream_t)stream));
-    h->was_reset = true;
-    h->dev.ring_phase = 0;
-    h->dev.fill_all = 1;      // until the next step: every ring is (re)written completely
+    if (int r = crl_pong_reset_state(h, stream)) return r;
     return crl_pong_render_obs(h, obs0_dev, obs1_dev, stream);
 }
 
 int crl_pong_step_state(crl_pong* h, const int32_t* actions_dev, float* rew_dev, uint8_t* done_dev,
                         int32_t* num_steps_dev, float* real_reward_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (int r = need_ready(h, true)) return r;
     if (!actions_dev || !rew_dev || !done_dev || !num_steps_dev || !real_reward_dev)
-        return fail(CRL_E_INVALID, "null step buffer");
+        return crl_set_error(CRL_E_INVALID, "null step buffer");
     h->dev.fill_all = 0;
     if (h->dev.ring) h->dev.ring_phase = (h->dev.ring_phase + 1) % h->dev.c;
     LAUNCH(launch_pong_step(h->dev, actions_dev, rew_dev, done_dev, num_steps_dev, real_reward_dev,
-                            (cudaStream_t)stream));
+                            (cudaStream_t)stream), 1);
     return CRL_OK;
 }
 
@@ -484,10 +428,10 @@ int crl_pong_step(crl_pong* h, const int32_t* actions_dev, uint8_t* obs0_dev, ui
 }
 
 int crl_pong_terminal_obs(crl_pong* h, const uint8_t* done_dev, uint8_t* term0_dev, uint8_t* term1_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (int r = need_ready(h, true)) return r;
-    if (!done_dev || !term0_dev || (h->dev.n_agents == 2 && !term1_dev)) return fail(CRL_E_INVALID, "null buffer");
-    LAUNCH(launch_pong_raster_generic(h->dev, h->dev.term_hist, done_dev, 0, term0_dev, term1_dev, (cudaStream_t)stream));
+    if (!done_dev || !term0_dev || (h->dev.n_agents == 2 && !term1_dev)) return crl_set_error(CRL_E_INVALID, "null buffer");
+    LAUNCH(launch_pong_raster_generic(h->dev, h->dev.term_hist, done_dev, 0, term0_dev, term1_dev, (cudaStream_t)stream), 1);
     obs_written(h, term0_dev, obs_bytes(h));
     obs_written(h, term1_dev, obs_bytes(h));
     return CRL_OK;
@@ -496,34 +440,28 @@ int crl_pong_terminal_obs(crl_pong* h, const uint8_t* done_dev, uint8_t* term0_d
 int crl_pong_step_host(crl_pong* h, const int32_t* actions_host, uint8_t* obs0_dev, uint8_t* obs1_dev,
                        uint8_t* obs0_host, uint8_t* obs1_host, float* rew_host, uint8_t* done_host,
                        int32_t* num_steps_host, float* real_reward_host, void* stream) {
-    CHECK_HANDLE(h);
-    if (!actions_host || !rew_host || !done_host) return fail(CRL_E_INVALID, "null host buffer");
+    CHECK_HANDLE(h, h->cfg.device);
+    if (!actions_host || !rew_host || !done_host) return crl_set_error(CRL_E_INVALID, "null host buffer");
     cudaStream_t s = (cudaStream_t)stream;
     const size_t n = (size_t)h->dev.n;
     const size_t aw = h->dev.n_agents == 2 ? 2 : 1;
-    if (!h->copy_stream) {
-        CUDA_TRY(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-        CUDA_TRY(cudaEventCreateWithFlags(&h->ev_state, cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&h->ev_copied, cudaEventDisableTiming));
-    }
+    CUDA_TRY(h->copy.ensure(false));
     CUDA_TRY(cudaMemcpyAsync(h->actions_stage, actions_host, n * aw * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     if (int r = crl_pong_step_state(h, h->actions_stage, h->rew_stage, h->done_stage, h->steps_stage, h->real_stage, stream))
         return r;
     // rewards / dones / counters are final once the game-core kernel has run: copy them out on the side stream,
     // behind the rasteriser (which is the whole cost of the step)
-    CUDA_TRY(cudaEventRecord(h->ev_state, s));
-    CUDA_TRY(cudaStreamWaitEvent(h->copy_stream, h->ev_state, 0));
-    cudaStream_t cs = h->copy_stream;
+    CUDA_TRY(h->copy.fork(s));
+    cudaStream_t cs = h->copy.stream;
     CUDA_TRY(cudaMemcpyAsync(rew_host, h->rew_stage, n * 2 * sizeof(float), cudaMemcpyDeviceToHost, cs));
     CUDA_TRY(cudaMemcpyAsync(done_host, h->done_stage, n, cudaMemcpyDeviceToHost, cs));
     if (num_steps_host)
         CUDA_TRY(cudaMemcpyAsync(num_steps_host, h->steps_stage, n * sizeof(int32_t), cudaMemcpyDeviceToHost, cs));
     if (real_reward_host)
         CUDA_TRY(cudaMemcpyAsync(real_reward_host, h->real_stage, n * 2 * sizeof(float), cudaMemcpyDeviceToHost, cs));
-    CUDA_TRY(cudaEventRecord(h->ev_copied, cs));
     if (int r = crl_pong_render_obs(h, obs0_dev, obs1_dev, stream)) return r;
-    CUDA_TRY(cudaStreamWaitEvent(s, h->ev_copied, 0));
-    const size_t ob = n * (h->dev.ring ? 2 * h->dev.c : h->dev.c) * h->dev.dim * h->dev.dim;
+    CUDA_TRY(h->copy.join(s));
+    const size_t ob = obs_bytes(h);
     if (obs0_host) CUDA_TRY(cudaMemcpyAsync(obs0_host, obs0_dev, ob, cudaMemcpyDeviceToHost, s));
     if (obs1_host && h->dev.n_agents == 2) CUDA_TRY(cudaMemcpyAsync(obs1_host, obs1_dev, ob, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
@@ -531,51 +469,47 @@ int crl_pong_step_host(crl_pong* h, const int32_t* actions_host, uint8_t* obs0_d
 }
 
 int crl_pong_ring_phase(crl_pong* h) {
-    if (!h) return fail(CRL_E_INVALID, "null handle");
-    if (!h->dev.ring) return fail(CRL_E_STATE, "the handle was not created with stack_mode ring");
+    if (!h) return crl_set_error(CRL_E_INVALID, "null handle");
+    if (!h->dev.ring) return crl_set_error(CRL_E_STATE, "the handle was not created with stack_mode ring");
     return h->dev.ring_phase;
 }
 
 int crl_pong_get_state(crl_pong* h, double* state_dev, void* stream) {
-    CHECK_HANDLE(h);
-    if (!state_dev) return fail(CRL_E_INVALID, "null buffer");
-    LAUNCH(launch_pong_get_state(h->dev, state_dev, (cudaStream_t)stream));
+    CHECK_HANDLE(h, h->cfg.device);
+    if (!state_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
+    LAUNCH(launch_pong_get_state(h->dev, state_dev, (cudaStream_t)stream), 1);
     return CRL_OK;
 }
 
 int crl_pong_set_state(crl_pong* h, const double* state_dev, void* stream) {
-    CHECK_HANDLE(h);
-    if (!state_dev) return fail(CRL_E_INVALID, "null buffer");
-    LAUNCH(launch_pong_set_state(h->dev, state_dev, (cudaStream_t)stream));
+    CHECK_HANDLE(h, h->cfg.device);
+    if (!state_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
+    LAUNCH(launch_pong_set_state(h->dev, state_dev, (cudaStream_t)stream), 1);
     return CRL_OK;
 }
 
 int crl_pong_render_raw(crl_pong* h, int32_t env, uint8_t* rgb0_dev, uint8_t* rgb1_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (int r = need_ready(h, false)) return r;
-    if (env < 0 || env >= h->dev.n || !rgb0_dev) return fail(CRL_E_INVALID, "bad env index or null buffer");
-    LAUNCH(launch_pong_raw_frame(h->dev, env, rgb0_dev, rgb1_dev, (cudaStream_t)stream));
+    if (env < 0 || env >= h->dev.n || !rgb0_dev) return crl_set_error(CRL_E_INVALID, "bad env index or null buffer");
+    LAUNCH(launch_pong_raw_frame(h->dev, env, rgb0_dev, rgb1_dev, (cudaStream_t)stream), 1);
     return CRL_OK;
 }
 
 int crl_pong_random_actions(int32_t* actions_dev, int32_t n_values, uint64_t seed, uint64_t step, void* stream) {
-    if (!actions_dev || n_values <= 0) return fail(CRL_E_INVALID, "bad arguments");
-    LAUNCH(launch_pong_random_actions(actions_dev, n_values, seed, step, (cudaStream_t)stream));
+    if (!actions_dev || n_values <= 0) return crl_set_error(CRL_E_INVALID, "bad arguments");
+    LAUNCH(launch_pong_random_actions(actions_dev, n_values, seed, step, (cudaStream_t)stream), 1);
     return CRL_OK;
 }
 
 int crl_pong_get_stats(crl_pong* h, uint64_t* stats_host, void* stream) {
-    CHECK_HANDLE(h);
-    if (!stats_host) return fail(CRL_E_INVALID, "null buffer");
-    unsigned long long raw[8];
-    CUDA_TRY(cudaMemcpyAsync(raw, h->dev.stats, sizeof raw, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
-    CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
-    for (int i = 0; i < 8; ++i) stats_host[i] = raw[i];
-    return CRL_OK;
+    CHECK_HANDLE(h, h->cfg.device);
+    if (!stats_host) return crl_set_error(CRL_E_INVALID, "null buffer");
+    return crl_read_counters(h->dev.stats, stats_host, 8, (cudaStream_t)stream);
 }
 
 int crl_pong_check(crl_pong* h, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     int32_t flag = 0;
     CUDA_TRY(cudaMemcpyAsync(&flag, h->dev.serve_overrun, sizeof flag, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
     CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
@@ -583,8 +517,8 @@ int crl_pong_check(crl_pong* h, void* stream) {
         CUDA_TRY(cudaMemsetAsync(h->dev.serve_overrun, 0, sizeof flag, (cudaStream_t)stream));
         CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
     }
-    if (flag & 2) return fail(CRL_E_INVALID, "an action outside {0, 1, 2} (cPongDouble: or 999) was passed to step; it was played as 1 (stay)");
-    if (flag & 1) return fail(CRL_E_SERVES, "injected serve table exhausted");
+    if (flag & 2) return crl_set_error(CRL_E_INVALID, "an action outside {0, 1, 2} (cPongDouble: or 999) was passed to step; it was played as 1 (stay)");
+    if (flag & 1) return crl_set_error(CRL_E_SERVES, "injected serve table exhausted");
     return CRL_OK;
 }
 
@@ -676,7 +610,7 @@ static void* obs_map_compressible(int device, size_t bytes, size_t* mapped, int3
 }
 
 int crl_obs_alloc(int32_t device, size_t bytes, void** ptr, int32_t* compressed) {
-    if (!ptr || !compressed || bytes == 0) return fail(CRL_E_INVALID, "crl_obs_alloc: null output pointer or zero bytes");
+    if (!ptr || !compressed || bytes == 0) return crl_set_error(CRL_E_INVALID, "crl_obs_alloc: null output pointer or zero bytes");
     *ptr = nullptr;
     *compressed = 0;
     CrlDeviceGuard guard(device);
@@ -704,7 +638,7 @@ int crl_obs_free(void* ptr) {
     {
         std::lock_guard<std::mutex> lk(g_obs_mu);
         auto it = g_obs.find(ptr);
-        if (it == g_obs.end()) return fail(CRL_E_INVALID, "crl_obs_free: %p was not returned by crl_obs_alloc", ptr);
+        if (it == g_obs.end()) return crl_set_error(CRL_E_INVALID, "crl_obs_free: %p was not returned by crl_obs_alloc", ptr);
         a = it->second;
         g_obs.erase(it);
     }
@@ -718,7 +652,7 @@ int crl_obs_free(void* ptr) {
     const ObsDriver& d = obs_driver();
     CUresult r = d.unmap(reinterpret_cast<CUdeviceptr>(ptr), a.bytes);
     if (r == CUDA_SUCCESS) r = d.address_free(reinterpret_cast<CUdeviceptr>(ptr), a.bytes);
-    if (r != CUDA_SUCCESS) return fail(CRL_E_CUDA, "crl_obs_free: cuMemUnmap / cuMemAddressFree failed (CUresult %d)", (int)r);
+    if (r != CUDA_SUCCESS) return crl_set_error(CRL_E_CUDA, "crl_obs_free: cuMemUnmap / cuMemAddressFree failed (CUresult %d)", (int)r);
     return CRL_OK;
 }
 

@@ -1,7 +1,5 @@
 // crl_car_abi.cu -- C ABI (include/crl_b200.h, crl_car_*) over the car-racing kernels. Host side only.
 #include <math.h>
-#include <stdarg.h>
-#include <stdio.h>
 #include <string.h>
 
 #include <vector>
@@ -12,39 +10,20 @@
 
 using namespace crl;
 
-extern "C" const char* crl_last_error(void);
-extern int crl_set_error(int code, const char* fmt, ...);
-extern void crl_count_launch(int n);
-
-#define CUDA_TRY(expr)                                                                                   \
-    do {                                                                                                 \
-        cudaError_t _e = (expr);                                                                         \
-        if (_e != cudaSuccess) return crl_set_error(CRL_E_CUDA, "%s: %s", #expr, cudaGetErrorString(_e)); \
-    } while (0)
-#define LAUNCH(expr, n)      \
-    do {                     \
-        CUDA_TRY(expr);      \
-        crl_count_launch(n); \
-    } while (0)
-
 struct crl_car {
     crl_car_config cfg;
     CarDev dev;
-    std::vector<void*> allocs;
+    DeviceAllocs allocs;
     // crl_car_step of two-car envs: envs whose cars touch are stepped on a side stream while the others render
-    cudaStream_t side_stream = nullptr;
-    cudaEvent_t ev_fast = nullptr, ev_slow = nullptr;
+    SideStream side;
     // plain stack mode without a registered buffer rotation ("stack-shift"): the C - 1 frames that stay in the observation
     // are moved ring -> obs on this stream beside the render passes
-    cudaStream_t copy_stream = nullptr;
-    cudaEvent_t ev_copy_go = nullptr, ev_copy_done = nullptr;
+    SideStream copy;
     // the sensor kernel of the NEXT step, started on its own stream as soon as this step's auto-resets are done
-    cudaStream_t sens_stream = nullptr;
-    cudaEvent_t ev_sens_go = nullptr, ev_sens_done = nullptr;
+    SideStream sens;
     bool sensors_ahead = false;      // sensor_now (and, two-car envs, slow list / deferred) of the current poses are in flight or ready
     // next tracks are generated ahead of time on this stream (car_pregen_kernel); at most one launch in flight
-    cudaStream_t pregen_stream = nullptr;
-    cudaEvent_t ev_pregen_go = nullptr;
+    SideStream pregen;
     uint64_t pregen_launches = 0;
     bool was_reset = false;
     // crl_car_step_host staging
@@ -200,16 +179,6 @@ void car_constants(CarHullConst* K) {
     g[G_GREEN] = gray_of(0, 255, 0); g[G_RED] = gray_of(255, 0, 0); g[G_TEXT] = gray_of(255, 255, 255);
 }
 
-template <typename T>
-cudaError_t car_alloc(crl_car* h, T** p, size_t count) {
-    void* q = nullptr;
-    cudaError_t e = cudaMalloc(&q, count * sizeof(T) + 16);
-    if (e != cudaSuccess) return e;
-    h->allocs.push_back(q);
-    *p = (T*)q;
-    return cudaMemset(q, 0, count * sizeof(T) + 16);
-}
-
 // Generate the next track of every env that has none, behind everything queued on `s` so far, on the handle's side
 // stream.  Launched after every step: the host runs many steps ahead of the GPU, so "launch when the previous one has
 // finished" would batch ~80 steps' worth of resets into one burst of curve walks; a launch per step keeps it at the
@@ -218,9 +187,8 @@ cudaError_t car_alloc(crl_car* h, T** p, size_t count) {
 // its next track is ready generates it inside car_reset_kernel.  High stream priority: the few warps that have work
 // live ~1.5 ms each (the walk is a serial fp64 chain) and should start at once.
 int kick_pregen(crl_car* h, cudaStream_t s) {
-    CUDA_TRY(cudaEventRecord(h->ev_pregen_go, s));
-    CUDA_TRY(cudaStreamWaitEvent(h->pregen_stream, h->ev_pregen_go, 0));
-    LAUNCH(launch_car_pregen(h->dev, h->pregen_stream), 1);
+    CUDA_TRY(h->pregen.fork(s));
+    LAUNCH(launch_car_pregen(h->dev, h->pregen.stream), 1);
     h->pregen_launches += 1;
     return CRL_OK;
 }
@@ -228,7 +196,7 @@ int kick_pregen(crl_car* h, cudaStream_t s) {
 // The inputs of track generation changed (seed, injected tables, fixed tracks): tracks generated ahead are dropped
 // and their attempts given back, so that what follows does not depend on how far the side stream had got.
 int discard_pregen(crl_car* h, cudaStream_t s) {
-    CUDA_TRY(cudaStreamSynchronize(h->pregen_stream));
+    CUDA_TRY(h->pregen.sync());
     LAUNCH(launch_car_discard_next(h->dev, s), 1);
     return CRL_OK;
 }
@@ -251,18 +219,12 @@ int rotate_obs(crl_car* h, uint8_t* obs_dev, bool at_reset) {
 bool moves_frames(const crl_car* h) { return !h->dev.ring_mode && h->dev.rot_n == 0 && h->dev.c >= 2; }   // internal ring + stack shift
 
 // Stack mode: start moving the frames that stay in the observation (ring -> channels 0 .. C-2 of obs) on the copy stream,
-// behind everything queued on `s` so far; join_stack_shift makes `s` wait for it (before the auto-reset pass).
+// behind everything queued on `s` so far; finish_step makes `s` wait for it (before the auto-reset pass).
 int fork_stack_shift(crl_car* h, uint8_t* obs_dev, cudaStream_t s) {
     if (!moves_frames(h)) return CRL_OK;
-    if (!h->copy_stream) {
-        CUDA_TRY(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-        CUDA_TRY(cudaEventCreateWithFlags(&h->ev_copy_go, cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&h->ev_copy_done, cudaEventDisableTiming));
-    }
-    CUDA_TRY(cudaEventRecord(h->ev_copy_go, s));
-    CUDA_TRY(cudaStreamWaitEvent(h->copy_stream, h->ev_copy_go, 0));
-    LAUNCH(launch_car_stack_shift(h->dev, obs_dev, h->copy_stream), 1);
-    CUDA_TRY(cudaEventRecord(h->ev_copy_done, h->copy_stream));
+    CUDA_TRY(h->copy.ensure(false));
+    CUDA_TRY(h->copy.fork(s));
+    LAUNCH(launch_car_stack_shift(h->dev, obs_dev, h->copy.stream), 1);
     return CRL_OK;
 }
 
@@ -270,19 +232,11 @@ int fork_stack_shift(crl_car* h, uint8_t* obs_dev, cudaStream_t s) {
 // behind: started on their own stream behind everything queued on `s` so far (the auto-reset spawns included), they run
 // under the auto-reset render passes instead of at the head of the next step.
 int sensors_ahead_of_next_step(crl_car* h, cudaStream_t s) {
-    if (!h->sens_stream) {
-        int lo = 0, hi = 0;
-        CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-        CUDA_TRY(cudaStreamCreateWithPriority(&h->sens_stream, cudaStreamNonBlocking, hi));
-        CUDA_TRY(cudaEventCreateWithFlags(&h->ev_sens_go, cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&h->ev_sens_done, cudaEventDisableTiming));
-    }
-    CUDA_TRY(cudaEventRecord(h->ev_sens_go, s));
-    CUDA_TRY(cudaStreamWaitEvent(h->sens_stream, h->ev_sens_go, 0));
-    if (h->dev.players == 2) CUDA_TRY(cudaMemsetAsync(h->dev.slow_count, 0, 2 * sizeof(int32_t), h->sens_stream));   // slow + near counts
-    LAUNCH(launch_car_sensors(h->dev, h->dev.players == 2 ? 1 : 0, h->sens_stream), 1);
-    if (h->dev.players == 2) LAUNCH(launch_car_collide(h->dev, h->sens_stream), 1);     // manifolds of the near envs -> slow list
-    CUDA_TRY(cudaEventRecord(h->ev_sens_done, h->sens_stream));
+    CUDA_TRY(h->sens.ensure(true));
+    CUDA_TRY(h->sens.fork(s));
+    if (h->dev.players == 2) CUDA_TRY(cudaMemsetAsync(h->dev.slow_count, 0, 2 * sizeof(int32_t), h->sens.stream));   // slow + near counts
+    LAUNCH(launch_car_sensors(h->dev, h->dev.players == 2 ? 1 : 0, h->sens.stream), 1);
+    if (h->dev.players == 2) LAUNCH(launch_car_collide(h->dev, h->sens.stream), 1);     // manifolds of the near envs -> slow list
     h->sensors_ahead = true;
     return CRL_OK;
 }
@@ -291,7 +245,7 @@ int sensors_ahead_of_next_step(crl_car* h, cudaStream_t s) {
 // them now (first step, after set_state / reset).
 int sensors_for_this_step(crl_car* h, cudaStream_t s) {
     if (h->sensors_ahead) {
-        CUDA_TRY(cudaStreamWaitEvent(s, h->ev_sens_done, 0));
+        CUDA_TRY(h->sens.join(s));
         h->sensors_ahead = false;
         return CRL_OK;
     }
@@ -306,15 +260,22 @@ int sensors_for_this_step(crl_car* h, cudaStream_t s) {
 // kernel computing it must not be reading the bodies while they are rewritten.
 int drop_sensors_ahead(crl_car* h, cudaStream_t s) {
     if (!h->sensors_ahead) return CRL_OK;
-    CUDA_TRY(cudaStreamWaitEvent(s, h->ev_sens_done, 0));
+    CUDA_TRY(h->sens.join(s));
     h->sensors_ahead = false;
     return CRL_OK;
 }
 
-int join_stack_shift(crl_car* h, cudaStream_t s) {
-    if (!moves_frames(h)) return CRL_OK;
-    CUDA_TRY(cudaStreamWaitEvent(s, h->ev_copy_done, 0));
-    return CRL_OK;
+// The tail of every step: the auto-reset of finished envs and their reset observation, with the next step's sensors and
+// tracks started ahead.
+int finish_step(crl_car* h, uint8_t* obs_dev, cudaStream_t s) {
+    if (moves_frames(h)) {
+        CUDA_TRY(h->copy.join(s));                                             // it reads ring_pos; the auto-reset pass rewrites whole stacks
+        LAUNCH(launch_car_ring_advance(h->dev, s), 1);
+    }
+    LAUNCH(launch_car_reset(h->dev, 1, s), 1);                                 // auto-reset of finished envs
+    if (int r = sensors_ahead_of_next_step(h, s)) return r;
+    LAUNCH(launch_car_render(h->dev, 1, 0, 1, obs_dev, nullptr, s), 3);        // their reset observation
+    return kick_pregen(h, s);
 }
 }  // namespace
 
@@ -323,21 +284,10 @@ extern "C" {
 int crl_car_destroy(crl_car* h) {
     if (!h) return CRL_OK;
     CrlDeviceGuard guard(h->cfg.device);
-    if (h->pregen_stream) cudaStreamSynchronize(h->pregen_stream);
-    for (void* p : h->allocs) cudaFree(p);
-    if (h->ev_pregen_go) cudaEventDestroy(h->ev_pregen_go);
-    if (h->pregen_stream) cudaStreamDestroy(h->pregen_stream);
-    if (h->ev_fast) cudaEventDestroy(h->ev_fast);
-    if (h->ev_slow) cudaEventDestroy(h->ev_slow);
-    if (h->side_stream) cudaStreamDestroy(h->side_stream);
-    if (h->copy_stream) cudaStreamSynchronize(h->copy_stream);
-    if (h->sens_stream) cudaStreamSynchronize(h->sens_stream);
-    if (h->ev_sens_go) cudaEventDestroy(h->ev_sens_go);
-    if (h->ev_sens_done) cudaEventDestroy(h->ev_sens_done);
-    if (h->sens_stream) cudaStreamDestroy(h->sens_stream);
-    if (h->ev_copy_go) cudaEventDestroy(h->ev_copy_go);
-    if (h->ev_copy_done) cudaEventDestroy(h->ev_copy_done);
-    if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
+    SideStream* streams[] = {&h->side, &h->copy, &h->sens, &h->pregen};
+    for (SideStream* st : streams) st->sync();      // kernels on them read the buffers freed below
+    h->allocs.free_all();
+    for (SideStream* st : streams) st->destroy();
     delete h;
     return CRL_OK;
 }
@@ -352,11 +302,7 @@ int crl_car_create(const crl_car_config* cfg, crl_car** out) {
     if (cfg->stack_mode != 0 && cfg->stack_mode != 1) return crl_set_error(CRL_E_INVALID, "stack_mode must be 0 (stack) or 1 (ring)");
     if (cfg->stack_mode == 1 && cfg->frame_stack < 2) return crl_set_error(CRL_E_INVALID, "stack_mode ring needs frame_stack >= 2");
     if (cfg->done_mode != 0 && cfg->done_mode != 1) return crl_set_error(CRL_E_INVALID, "done_mode must be 0 (any car) or 1 (car 0)");
-    int ndev = 0;
-    cudaError_t e = cudaGetDeviceCount(&ndev);
-    if (e != cudaSuccess || ndev == 0)
-        return crl_set_error(CRL_E_CUDA, "no CUDA device available (%s); this library has no CPU path", cudaGetErrorString(e));
-    if (cfg->device < 0 || cfg->device >= ndev) return crl_set_error(CRL_E_INVALID, "device %d out of range", cfg->device);
+    if (int r = crl_check_device(cfg->device)) return r;
     CrlDeviceGuard guard(cfg->device);
     CUDA_TRY(guard.err);
     crl_car* h = new crl_car();
@@ -370,38 +316,35 @@ int crl_car_create(const crl_car_config* cfg, crl_car** out) {
     d.done_mode = cfg->done_mode;
     d.ring_mode = cfg->stack_mode == 1 ? 1 : 0;
     d.first_env = cfg->first_env; d.seed = cfg->seed;
-#define ALLOC(ptr, count)                                                                   \
-    do {                                                                                    \
-        cudaError_t _e = car_alloc(h, &(ptr), (count));                                     \
-        if (_e != cudaSuccess) {                                                            \
-            crl_car_destroy(h);                                                             \
-            return crl_set_error(CRL_E_CUDA, "cudaMalloc: %s", cudaGetErrorString(_e));      \
-        }                                                                                   \
-    } while (0)
-    ALLOC(d.n_track, 2 * n); ALLOC(d.tiles, 2 * n * CAR_MAX_TRACK); ALLOC(d.samples, 2 * n * CAR_MAX_SAMPLES);
-    ALLOC(d.start_pose, 2 * n * 3); ALLOC(d.track_pts, 2 * n * CAR_MAX_TRACK * 3);
-    ALLOC(d.sel, n); ALLOC(d.next_state, n); ALLOC(d.next_att0, n); ALLOC(d.raw_ring, n * CAR_RAW_RING * 3);
-    ALLOC(d.step_count, n); ALLOC(d.elapsed, n); ALLOC(d.reset_count, n);
-    ALLOC(d.attempt_count, n); ALLOC(d.inv_dt0, n); ALLOC(d.env_done, n); ALLOC(d.ring_pos, n);
-    ALLOC(d.body, nc * 40); ALLOC(d.joint, nc * 24); ALLOC(d.wheel, nc * 8); ALLOC(d.reward, nc * 2);
-    ALLOC(d.counters, nc * 4); ALLOC(d.touching, nc * 64); ALLOC(d.visited, nc * 16); ALLOC(d.sensor_now, nc * 64);
-    ALLOC(d.overrun, 4); ALLOC(d.stats, 8);
-    ALLOC(d.contact_overflow, 1);
+    cudaError_t e = cudaSuccess;
+    auto alloc = [&](auto** p, size_t count) { if (e == cudaSuccess) e = h->allocs.alloc(p, count); };
+    alloc(&d.n_track, 2 * n); alloc(&d.tiles, 2 * n * CAR_MAX_TRACK); alloc(&d.samples, 2 * n * CAR_MAX_SAMPLES);
+    alloc(&d.start_pose, 2 * n * 3); alloc(&d.track_pts, 2 * n * CAR_MAX_TRACK * 3);
+    alloc(&d.sel, n); alloc(&d.next_state, n); alloc(&d.next_att0, n); alloc(&d.raw_ring, n * CAR_RAW_RING * 3);
+    alloc(&d.step_count, n); alloc(&d.elapsed, n); alloc(&d.reset_count, n);
+    alloc(&d.attempt_count, n); alloc(&d.inv_dt0, n); alloc(&d.env_done, n); alloc(&d.ring_pos, n);
+    alloc(&d.body, nc * 40); alloc(&d.joint, nc * 24); alloc(&d.wheel, nc * 8); alloc(&d.reward, nc * 2);
+    alloc(&d.counters, nc * 4); alloc(&d.touching, nc * 64); alloc(&d.visited, nc * 16); alloc(&d.sensor_now, nc * 64);
+    alloc(&d.overrun, 4); alloc(&d.stats, 8);
+    alloc(&d.contact_overflow, 1);
     {
         uint8_t* fmraw = nullptr;
-        ALLOC(fmraw, nc * car_frame_map_bytes());
+        alloc(&fmraw, nc * car_frame_map_bytes());
         d.frame_map = reinterpret_cast<FrameMap*>(fmraw);
-        ALLOC(d.frame_aux, nc * car_frame_aux_bytes());
+        alloc(&d.frame_aux, nc * car_frame_aux_bytes());
     }
-    ALLOC(d.map_index, 2 * n * CAR_MAP_GRID * CAR_MAP_GRID); ALLOC(d.map_blocks, 2 * n * CAR_MAP_MAX_BLOCKS * 256);
-    ALLOC(d.tile_centres, 2 * n * CAR_MAX_TRACK);
-    ALLOC(h->actions_stage, nc * 2); ALLOC(h->rew_stage, nc); ALLOC(h->done_stage, n); ALLOC(h->steps_stage, n); ALLOC(h->trunc_stage, n);
-    if (P == 2) { ALLOC(d.contacts, n * CAR_MAX_CONTACTS); ALLOC(d.n_contacts, n); ALLOC(d.n_contacts_step, n); ALLOC(d.slow_list, n); ALLOC(d.slow_count, 2); d.near_count = d.slow_count + 1; ALLOC(d.near_list, n); }
-    ALLOC(d.deferred, n);
-    ALLOC(d.done_list, n); ALLOC(d.done_count, 1);
+    alloc(&d.map_index, 2 * n * CAR_MAP_GRID * CAR_MAP_GRID); alloc(&d.map_blocks, 2 * n * CAR_MAP_MAX_BLOCKS * 256);
+    alloc(&d.tile_centres, 2 * n * CAR_MAX_TRACK);
+    alloc(&h->actions_stage, nc * 2); alloc(&h->rew_stage, nc); alloc(&h->done_stage, n); alloc(&h->steps_stage, n); alloc(&h->trunc_stage, n);
+    if (P == 2) { alloc(&d.contacts, n * CAR_MAX_CONTACTS); alloc(&d.n_contacts, n); alloc(&d.n_contacts_step, n); alloc(&d.slow_list, n); alloc(&d.slow_count, 2); d.near_count = d.slow_count + 1; alloc(&d.near_list, n); }
+    alloc(&d.deferred, n);
+    alloc(&d.done_list, n); alloc(&d.done_count, 1);
     CarHullConst* kdev = nullptr;
-    ALLOC(kdev, 1);
-#undef ALLOC
+    alloc(&kdev, 1);
+    if (e != cudaSuccess) {
+        crl_car_destroy(h);
+        return crl_set_error(CRL_E_CUDA, "cudaMalloc: %s", cudaGetErrorString(e));
+    }
     CarHullConst K;
     memset(&K, 0, sizeof K);
     car_constants(&K);
@@ -414,7 +357,7 @@ int crl_car_create(const crl_car_config* cfg, crl_car** out) {
                 for (int v = K.checker[(axis * 20 + i) * 2]; v <= K.checker[(axis * 20 + i) * 2 + 1]; ++v)
                     if (v >= CAR_MAP_ORIGIN && v < CAR_MAP_ORIGIN + 2048) chk[axis * 2048 + v - CAR_MAP_ORIGIN] = 0xFF;
         uint8_t* cdev = nullptr;
-        if (e == cudaSuccess) e = car_alloc(h, &cdev, chk.size());
+        if (e == cudaSuccess) e = h->allocs.alloc(&cdev, chk.size());
         if (e == cudaSuccess) e = cudaMemcpy(cdev, chk.data(), chk.size(), cudaMemcpyHostToDevice);
         d.chk = cdev;
     }
@@ -425,69 +368,64 @@ int crl_car_create(const crl_car_config* cfg, crl_car** out) {
         return crl_set_error(CRL_E_CUDA, "init: %s", cudaGetErrorString(e));
     }
     d.consts = kdev;
-    {
-        int lo = 0, hi = 0;
-        e = cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&h->pregen_stream, cudaStreamNonBlocking, hi);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_pregen_go, cudaEventDisableTiming);
-        if (e != cudaSuccess) {
-            crl_car_destroy(h);
-            return crl_set_error(CRL_E_CUDA, "pregen stream: %s", cudaGetErrorString(e));
-        }
+    e = h->pregen.ensure(true);
+    if (e != cudaSuccess) {
+        crl_car_destroy(h);
+        return crl_set_error(CRL_E_CUDA, "pregen stream: %s", cudaGetErrorString(e));
     }
     *out = h;
     return CRL_OK;
 }
 
-#define CHECK_HANDLE(h)                                               \
-    do {                                                              \
-        if (!(h)) return crl_set_error(CRL_E_INVALID, "null handle"); \
-    } while (0);                                                      \
-    CrlDeviceGuard crl_guard_((h)->cfg.device);                       \
-    CUDA_TRY(crl_guard_.err)
-
 int crl_car_load_glyphs(crl_car* h, const uint8_t* glyphs_host, size_t bytes, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!glyphs_host || bytes != (size_t)CRL_CAR_GLYPH_BYTES) return crl_set_error(CRL_E_INVALID, "glyph atlas must be %d bytes", CRL_CAR_GLYPH_BYTES);
     uint8_t* g = nullptr;
-    CUDA_TRY(car_alloc(h, &g, bytes));
+    CUDA_TRY(h->allocs.alloc(&g, bytes));
     CUDA_TRY(cudaMemcpyAsync(g, glyphs_host, bytes, cudaMemcpyHostToDevice, (cudaStream_t)stream));
     CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
+    const uint8_t* old = h->dev.glyphs;
     h->dev.glyphs = g;
+    CUDA_TRY(h->allocs.free(old));
     return CRL_OK;
 }
 
 int crl_car_inject_tracks(crl_car* h, const double* draws_host, int32_t k_draws, const int32_t* birth_host,
                           int32_t k_birth, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!draws_host || k_draws < 1) return crl_set_error(CRL_E_INVALID, "need at least one attempt of draws per env");
     cudaStream_t s = (cudaStream_t)stream;
     double* dd = nullptr;
     const size_t cnt = (size_t)h->dev.n * k_draws * CAR_DRAWS;
-    CUDA_TRY(car_alloc(h, &dd, cnt));
+    CUDA_TRY(h->allocs.alloc(&dd, cnt));
     CUDA_TRY(cudaMemcpyAsync(dd, draws_host, cnt * sizeof(double), cudaMemcpyHostToDevice, s));
     if (int r = discard_pregen(h, s)) return r;
+    const void* old[2] = {h->dev.track_draws, nullptr};
     h->dev.track_draws = dd; h->dev.k_draws = k_draws;
-    if (birth_host && k_birth > 0) {
+    if (birth_host && k_birth > 0) {                // without one, the previous birth table stays
         int32_t* bb = nullptr;
         const size_t bc = (size_t)h->dev.n * k_birth * h->dev.players;
-        CUDA_TRY(car_alloc(h, &bb, bc));
+        CUDA_TRY(h->allocs.alloc(&bb, bc));
         CUDA_TRY(cudaMemcpyAsync(bb, birth_host, bc * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        old[1] = h->dev.birth;
         h->dev.birth = bb; h->dev.k_birth = k_birth;
     }
     CUDA_TRY(cudaMemsetAsync(h->dev.attempt_count, 0, (size_t)h->dev.n * sizeof(int32_t), s));
     CUDA_TRY(cudaMemsetAsync(h->dev.reset_count, 0, (size_t)h->dev.n * sizeof(int32_t), s));
     CUDA_TRY(cudaStreamSynchronize(s));
+    for (const void* p : old) CUDA_TRY(h->allocs.free(p));
     return CRL_OK;
 }
 
 int crl_car_load_tracks(crl_car* h, const double* pts_host, const int32_t* counts_host, int32_t n_tracks, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     cudaStream_t s = (cudaStream_t)stream;
     if (int r = discard_pregen(h, s)) return r;
     CUDA_TRY(cudaStreamSynchronize(s));
+    const void* old[2] = {h->dev.fixed_tracks, h->dev.fixed_counts};
     if (n_tracks <= 0) {                       // back to generated tracks
         h->dev.fixed_tracks = nullptr; h->dev.fixed_counts = nullptr; h->dev.n_fixed = 0;
+        for (const void* p : old) CUDA_TRY(h->allocs.free(p));
         return CRL_OK;
     }
     if (!pts_host || !counts_host) return crl_set_error(CRL_E_INVALID, "null track buffer");
@@ -496,23 +434,24 @@ int crl_car_load_tracks(crl_car* h, const double* pts_host, const int32_t* count
             return crl_set_error(CRL_E_INVALID, "track %d has %d points; need 9..%d", k, counts_host[k], CAR_MAX_TRACK);
     double* dp = nullptr;
     int32_t* dc = nullptr;
-    CUDA_TRY(car_alloc(h, &dp, (size_t)n_tracks * CAR_MAX_TRACK * 3));
-    CUDA_TRY(car_alloc(h, &dc, (size_t)n_tracks));
+    CUDA_TRY(h->allocs.alloc(&dp, (size_t)n_tracks * CAR_MAX_TRACK * 3));
+    CUDA_TRY(h->allocs.alloc(&dc, (size_t)n_tracks));
     CUDA_TRY(cudaMemcpyAsync(dp, pts_host, (size_t)n_tracks * CAR_MAX_TRACK * 3 * sizeof(double), cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaMemcpyAsync(dc, counts_host, (size_t)n_tracks * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaStreamSynchronize(s));
     h->dev.fixed_tracks = dp; h->dev.fixed_counts = dc; h->dev.n_fixed = n_tracks;
+    for (const void* p : old) CUDA_TRY(h->allocs.free(p));
     return CRL_OK;
 }
 
 int crl_car_reset(crl_car* h, uint8_t* obs_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!obs_dev) return crl_set_error(CRL_E_INVALID, "null observation buffer");
     cudaStream_t s = (cudaStream_t)stream;
     if (int r = rotate_obs(h, obs_dev, true)) return r;
     if (int r = drop_sensors_ahead(h, s)) return r;
     if (!h->dev.ring_mode && h->dev.rot_n == 0 && h->dev.ring == nullptr)   // the internal frame ring of the plain stack mode, on first use (1.2 GB at config 5)
-        CUDA_TRY(car_alloc(h, &h->dev.ring, (size_t)h->dev.n * h->dev.players * h->dev.c * CAR_PIX));
+        CUDA_TRY(h->allocs.alloc(&h->dev.ring, (size_t)h->dev.n * h->dev.players * h->dev.c * CAR_PIX));
     CUDA_TRY(cudaMemsetAsync(h->dev.ring_pos, 0xFF, (size_t)h->dev.n * sizeof(int32_t), s));
     CUDA_TRY(cudaMemsetAsync(h->dev.env_done, 0, (size_t)h->dev.n, s));
     h->dev.ring_phase = 0;
@@ -525,7 +464,7 @@ int crl_car_reset(crl_car* h, uint8_t* obs_dev, void* stream) {
 
 int crl_car_step_state(crl_car* h, const float* actions_dev, float* rew_dev, uint8_t* done_dev,
                        int32_t* num_steps_dev, uint8_t* truncated_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!h->was_reset) return crl_set_error(CRL_E_STATE, "reset must be called before step");
     if (!actions_dev || !rew_dev || !done_dev || !num_steps_dev || !truncated_dev) return crl_set_error(CRL_E_INVALID, "null step buffer");
     h->dev.fill_all = 0;
@@ -536,7 +475,7 @@ int crl_car_step_state(crl_car* h, const float* actions_dev, float* rew_dev, uin
 }
 
 int crl_car_render_obs(crl_car* h, uint8_t* obs_dev, uint8_t* term_obs_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!h->was_reset) return crl_set_error(CRL_E_STATE, "reset must be called before step");
     if (!obs_dev) return crl_set_error(CRL_E_INVALID, "null observation buffer");
     cudaStream_t s = (cudaStream_t)stream;
@@ -553,24 +492,19 @@ int crl_car_render_obs(crl_car* h, uint8_t* obs_dev, uint8_t* term_obs_dev, void
 
 int crl_car_step(crl_car* h, const float* actions_dev, uint8_t* obs_dev, float* rew_dev, uint8_t* done_dev,
                  int32_t* num_steps_dev, uint8_t* truncated_dev, uint8_t* term_obs_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
+    if (!h->was_reset) return crl_set_error(CRL_E_STATE, "reset must be called before step");
+    if (!actions_dev || !obs_dev || !rew_dev || !done_dev || !num_steps_dev || !truncated_dev) return crl_set_error(CRL_E_INVALID, "null step buffer");
+    cudaStream_t s = (cudaStream_t)stream;
     if (h->dev.players == 1) {
-        if (!h->was_reset) return crl_set_error(CRL_E_STATE, "reset must be called before step");
-        if (!actions_dev || !obs_dev || !rew_dev || !done_dev || !num_steps_dev || !truncated_dev) return crl_set_error(CRL_E_INVALID, "null step buffer");
-        cudaStream_t s1 = (cudaStream_t)stream;
         if (int r = rotate_obs(h, obs_dev, false)) return r;      // after the argument checks: a refused call leaves the rotation where it was
         if (int r = crl_car_step_state(h, actions_dev, rew_dev, done_dev, num_steps_dev, truncated_dev, stream)) return r;
-        if (int r = fork_stack_shift(h, obs_dev, s1)) return r;                    // next to the render pass
-        CUDA_TRY(cudaMemsetAsync(h->dev.done_count, 0, sizeof(int32_t), s1));
+        if (int r = fork_stack_shift(h, obs_dev, s)) return r;                     // next to the render pass
+        CUDA_TRY(cudaMemsetAsync(h->dev.done_count, 0, sizeof(int32_t), s));
         h->dev.collect_done = 1;
-        LAUNCH(launch_car_render(h->dev, 0, 0, 0, obs_dev, term_obs_dev, s1), 3);   // post-step frame (terminal obs of finished envs)
+        LAUNCH(launch_car_render(h->dev, 0, 0, 0, obs_dev, term_obs_dev, s), 3);   // post-step frame (terminal obs of finished envs)
         h->dev.collect_done = 0;
-        if (int r = join_stack_shift(h, s1)) return r;                             // it reads ring_pos; the auto-reset pass rewrites whole stacks
-        if (moves_frames(h)) LAUNCH(launch_car_ring_advance(h->dev, s1), 1);
-        LAUNCH(launch_car_reset(h->dev, 1, s1), 1);                                 // auto-reset of finished envs
-        if (int r = sensors_ahead_of_next_step(h, s1)) return r;
-        LAUNCH(launch_car_render(h->dev, 1, 0, 1, obs_dev, nullptr, s1), 3);        // their reset observation
-        return kick_pregen(h, s1);
+        return finish_step(h, obs_dev, s);
     }
     // Two-car envs.  The step kernel is one wave of latency-bound threads; lane pairs whose cars touch run the sequential
     // contact solver and take several times longer than the rest.  So the sensor kernel lists the envs whose cars are near
@@ -578,44 +512,28 @@ int crl_car_step(crl_car* h, const float* actions_dev, uint8_t* obs_dev, float* 
     // pass) and renders their frames; the frames of the listed envs follow.  Per env nothing changes; only the launch
     // schedule does.  (Without a registered buffer rotation the frames that stay in the observation stack move ring -> obs
     // on a third stream meanwhile.)
-    if (!h->was_reset) return crl_set_error(CRL_E_STATE, "reset must be called before step");
-    if (!actions_dev || !obs_dev || !rew_dev || !done_dev || !num_steps_dev || !truncated_dev) return crl_set_error(CRL_E_INVALID, "null step buffer");
-    cudaStream_t s = (cudaStream_t)stream;
-    if (!h->side_stream) {
-        int lo = 0, hi = 0;
-        CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-        CUDA_TRY(cudaStreamCreateWithPriority(&h->side_stream, cudaStreamNonBlocking, hi));
-        CUDA_TRY(cudaEventCreateWithFlags(&h->ev_fast, cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&h->ev_slow, cudaEventDisableTiming));
-    }
+    CUDA_TRY(h->side.ensure(true));
     if (int r = rotate_obs(h, obs_dev, false)) return r;
     h->dev.fill_all = 0;
     if (h->dev.ring_mode) h->dev.ring_phase = (h->dev.ring_phase + 1) % h->dev.c;
     CUDA_TRY(cudaMemsetAsync(h->dev.done_count, 0, sizeof(int32_t), s));
     if (int r = sensors_for_this_step(h, s)) return r;                         // wheel-tile overlaps, manifolds, the slow list
-    CUDA_TRY(cudaEventRecord(h->ev_fast, s));
-    CUDA_TRY(cudaStreamWaitEvent(h->side_stream, h->ev_fast, 0));
-    LAUNCH(launch_car_step(h->dev, 2, actions_dev, rew_dev, done_dev, num_steps_dev, truncated_dev, h->side_stream), 1);
-    CUDA_TRY(cudaEventRecord(h->ev_slow, h->side_stream));
+    CUDA_TRY(h->side.fork(s));
+    LAUNCH(launch_car_step(h->dev, 2, actions_dev, rew_dev, done_dev, num_steps_dev, truncated_dev, h->side.stream), 1);
     LAUNCH(launch_car_step(h->dev, 1, actions_dev, rew_dev, done_dev, num_steps_dev, truncated_dev, s), 1);
     // "stack-shift" only: the frames that stay in the stack, ring -> obs, next to the render passes (DRAM-bound beside
     // issue-bound; the step kernels before it fill the register files, so it is not started under them)
     if (int r = fork_stack_shift(h, obs_dev, s)) return r;
     h->dev.collect_done = 1;
     LAUNCH(launch_car_render(h->dev, 0, 1, 0, obs_dev, term_obs_dev, s), 3);   // frames of the envs stepped by the fast pass
-    CUDA_TRY(cudaStreamWaitEvent(s, h->ev_slow, 0));
+    CUDA_TRY(h->side.join(s));
     LAUNCH(launch_car_render(h->dev, 0, 2, 0, obs_dev, term_obs_dev, s), 3);   // frames of the listed envs
     h->dev.collect_done = 0;
-    if (int r = join_stack_shift(h, s)) return r;                             // it reads ring_pos; the auto-reset pass rewrites whole stacks
-    if (moves_frames(h)) LAUNCH(launch_car_ring_advance(h->dev, s), 1);
-    LAUNCH(launch_car_reset(h->dev, 1, s), 1);                                 // auto-reset of finished envs
-    if (int r = sensors_ahead_of_next_step(h, s)) return r;
-    LAUNCH(launch_car_render(h->dev, 1, 0, 1, obs_dev, nullptr, s), 3);        // their reset observation
-    return kick_pregen(h, s);
+    return finish_step(h, obs_dev, s);
 }
 
 int crl_car_seed(crl_car* h, uint64_t seed, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (int r = discard_pregen(h, (cudaStream_t)stream)) return r;
     CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
     h->dev.seed = seed;
@@ -623,7 +541,7 @@ int crl_car_seed(crl_car* h, uint64_t seed, void* stream) {
 }
 
 int crl_car_set_elapsed(crl_car* h, const int32_t* elapsed_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!elapsed_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
     CUDA_TRY(cudaMemcpyAsync(h->dev.elapsed, elapsed_dev, (size_t)h->dev.n * sizeof(int32_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return CRL_OK;
@@ -631,7 +549,7 @@ int crl_car_set_elapsed(crl_car* h, const int32_t* elapsed_dev, void* stream) {
 
 int crl_car_step_host(crl_car* h, const float* actions_host, uint8_t* obs_dev, uint8_t* obs_host, float* rew_host,
                       uint8_t* done_host, int32_t* num_steps_host, uint8_t* truncated_host, uint8_t* term_obs_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!actions_host || !obs_dev || !rew_host || !done_host) return crl_set_error(CRL_E_INVALID, "null host buffer");
     cudaStream_t s = (cudaStream_t)stream;
     const size_t n = (size_t)h->dev.n, nc = n * h->dev.players;
@@ -648,14 +566,14 @@ int crl_car_step_host(crl_car* h, const float* actions_host, uint8_t* obs_dev, u
 }
 
 int crl_car_get_state(crl_car* h, double* state_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!state_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
     LAUNCH(launch_car_get_state(h->dev, state_dev, (cudaStream_t)stream), 1);
     return CRL_OK;
 }
 
 int crl_car_set_state(crl_car* h, const double* state_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!state_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
     if (!h->was_reset) return crl_set_error(CRL_E_STATE, "reset must be called before set_state");
     if (int r = drop_sensors_ahead(h, (cudaStream_t)stream)) return r;
@@ -664,7 +582,7 @@ int crl_car_set_state(crl_car* h, const double* state_dev, void* stream) {
 }
 
 int crl_car_render_state(crl_car* h, uint8_t* obs_dev, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!h->was_reset) return crl_set_error(CRL_E_STATE, "reset must be called before rendering");
     if (!obs_dev) return crl_set_error(CRL_E_INVALID, "null observation buffer");
     if (int r = rotate_obs(h, obs_dev, false)) return r;
@@ -676,7 +594,7 @@ int crl_car_render_state(crl_car* h, uint8_t* obs_dev, void* stream) {
 }
 
 int crl_car_set_obs_rotation(crl_car* h, uint8_t* const* obs_devs_host, int32_t count, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     CarDev& d = h->dev;
     if (count == 0) { d.rot_n = 0; d.rot_pos = 0; h->was_reset = false; return CRL_OK; }   // plain mode again, from the next reset on
     if (d.ring_mode) return crl_set_error(CRL_E_STATE, "stack_mode ring has no use for a buffer rotation");
@@ -702,7 +620,7 @@ int crl_car_ring_phase(crl_car* h) {
 }
 
 int crl_car_get_track(crl_car* h, int32_t env, int32_t* n_out, double* pts_host, int32_t max_points, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (env < 0 || env >= h->dev.n || !n_out) return crl_set_error(CRL_E_INVALID, "bad arguments");
     cudaStream_t s = (cudaStream_t)stream;
     int32_t n = 0, sel = 0;
@@ -727,12 +645,9 @@ int crl_car_random_actions(float* actions_dev, int32_t n_values, uint64_t seed, 
 }
 
 int crl_car_get_stats(crl_car* h, uint64_t* stats_host, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     if (!stats_host) return crl_set_error(CRL_E_INVALID, "null buffer");
-    unsigned long long raw[8];
-    CUDA_TRY(cudaMemcpyAsync(raw, h->dev.stats, sizeof raw, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
-    CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
-    for (int i = 0; i < 8; ++i) stats_host[i] = raw[i];
+    if (int r = crl_read_counters(h->dev.stats, stats_host, 8, (cudaStream_t)stream)) return r;
     int32_t flags[4] = {0, 0, 0, 0};
     CUDA_TRY(cudaMemcpyAsync(flags, h->dev.overrun, sizeof flags, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
     CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
@@ -743,7 +658,7 @@ int crl_car_get_stats(crl_car* h, uint64_t* stats_host, void* stream) {
 }
 
 int crl_car_get_contacts(crl_car* h, int32_t* counts_host, int32_t* overflow_host, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     cudaStream_t s = (cudaStream_t)stream;
     if (counts_host) {
         if (h->dev.n_contacts_step) CUDA_TRY(cudaMemcpyAsync(counts_host, h->dev.n_contacts_step, (size_t)h->dev.n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
@@ -755,7 +670,7 @@ int crl_car_get_contacts(crl_car* h, int32_t* counts_host, int32_t* overflow_hos
 }
 
 int crl_car_check(crl_car* h, void* stream) {
-    CHECK_HANDLE(h);
+    CHECK_HANDLE(h, h->cfg.device);
     int32_t flags[4] = {0, 0, 0, 0};
     CUDA_TRY(cudaMemcpyAsync(flags, h->dev.overrun, sizeof flags, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
     CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));

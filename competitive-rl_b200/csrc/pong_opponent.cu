@@ -12,7 +12,6 @@
 // The networks run on the SIMT fp32 pipe with explicit __fmaf_rn (the library is compiled with -fmad=false).  Each CTA
 // owns a contiguous range of envs; it sorts them by network slot in shared memory and then runs every slot present
 // with that slot's weights staged once in shared memory, one env at a time over all its threads.
-#include <stdarg.h>
 #include <string.h>
 
 #include <cmath>
@@ -23,21 +22,6 @@
 #include "pong_common.cuh"
 
 using namespace crl;
-
-extern "C" const char* crl_last_error(void);
-extern int crl_set_error(int code, const char* fmt, ...);
-extern void crl_count_launch(int n);
-
-#define CUDA_TRY(expr)                                                                                   \
-    do {                                                                                                 \
-        cudaError_t _e = (expr);                                                                         \
-        if (_e != cudaSuccess) return crl_set_error(CRL_E_CUDA, "%s: %s", #expr, cudaGetErrorString(_e)); \
-    } while (0)
-#define LAUNCH(expr)         \
-    do {                     \
-        CUDA_TRY(expr);      \
-        crl_count_launch(1); \
-    } while (0)
 
 namespace crl {
 namespace opp {
@@ -313,6 +297,7 @@ struct crl_pong_opp {
     bool loaded[CRL_PONG_OPP_SLOTS] = {};
     int8_t kind[CRL_PONG_OPP_MAX_POOL] = {};
     uint64_t cum[CRL_PONG_OPP_MAX_POOL] = {};
+    DeviceAllocs allocs;
     float* nets = nullptr;
     int32_t* ids = nullptr;
     uint8_t* stack = nullptr;
@@ -331,18 +316,12 @@ static OppArgs opp_args(const crl_pong_opp* h) {
     return a;
 }
 
-#define CHECK_OPP(h)                                                      \
-    if (!(h)) return crl_set_error(CRL_E_INVALID, "null handle");         \
-    CrlDeviceGuard guard((h)->device);                                    \
-    CUDA_TRY(guard.err)
-
 extern "C" {
 
 int crl_pong_opp_destroy(crl_pong_opp* h) {
     if (!h) return CRL_OK;
     CrlDeviceGuard guard(h->device);
-    for (void* p : {(void*)h->nets, (void*)h->ids, (void*)h->stack, (void*)h->ret, (void*)h->episodes, (void*)h->stats})
-        if (p) cudaFree(p);
+    h->allocs.free_all();
     delete h;
     return CRL_OK;
 }
@@ -351,29 +330,18 @@ int crl_pong_opp_create(int32_t num_envs, int32_t device, uint64_t seed, int64_t
     if (!out) return crl_set_error(CRL_E_INVALID, "null argument");
     *out = nullptr;
     if (num_envs <= 0) return crl_set_error(CRL_E_INVALID, "num_envs must be positive");
-    int ndev = 0;
-    cudaError_t e = cudaGetDeviceCount(&ndev);
-    if (e != cudaSuccess || ndev == 0)
-        return crl_set_error(CRL_E_CUDA, "no CUDA device available (%s); this library has no CPU path", cudaGetErrorString(e));
-    if (device < 0 || device >= ndev) return crl_set_error(CRL_E_INVALID, "device %d out of range", device);
+    if (int r = crl_check_device(device)) return r;
     CrlDeviceGuard guard(device);
     CUDA_TRY(guard.err);
     crl_pong_opp* h = new crl_pong_opp();
     h->n = num_envs; h->device = device; h->seed = seed; h->first_env = first_env;
     const size_t n = (size_t)num_envs;
     int sms = 0, per_sm = 0;
-    cudaError_t err = cudaMalloc(&h->nets, sizeof(float) * NET_DEV * CRL_PONG_OPP_SLOTS);
-    if (err == cudaSuccess) err = cudaMalloc(&h->ids, sizeof(int32_t) * n);
-    if (err == cudaSuccess) err = cudaMalloc(&h->stack, (size_t)STACK * FRAME * n);
-    if (err == cudaSuccess) err = cudaMalloc(&h->ret, sizeof(float) * n);
-    if (err == cudaSuccess) err = cudaMalloc(&h->episodes, sizeof(uint32_t) * n);
-    if (err == cudaSuccess) err = cudaMalloc(&h->stats, sizeof(unsigned long long) * 4 * CRL_PONG_OPP_MAX_POOL);
-    if (err == cudaSuccess) err = cudaMemset(h->nets, 0, sizeof(float) * NET_DEV * CRL_PONG_OPP_SLOTS);
-    if (err == cudaSuccess) err = cudaMemset(h->ids, 0, sizeof(int32_t) * n);
-    if (err == cudaSuccess) err = cudaMemset(h->stack, 0, (size_t)STACK * FRAME * n);
-    if (err == cudaSuccess) err = cudaMemset(h->ret, 0, sizeof(float) * n);
-    if (err == cudaSuccess) err = cudaMemset(h->episodes, 0, sizeof(uint32_t) * n);
-    if (err == cudaSuccess) err = cudaMemset(h->stats, 0, sizeof(unsigned long long) * 4 * CRL_PONG_OPP_MAX_POOL);
+    cudaError_t err = cudaSuccess;
+    auto alloc = [&](auto** p, size_t count) { if (err == cudaSuccess) err = h->allocs.alloc(p, count); };
+    alloc(&h->nets, (size_t)NET_DEV * CRL_PONG_OPP_SLOTS);
+    alloc(&h->ids, n); alloc(&h->stack, (size_t)STACK * FRAME * n); alloc(&h->ret, n); alloc(&h->episodes, n);
+    alloc(&h->stats, 4 * CRL_PONG_OPP_MAX_POOL);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(pong_opp_act_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
     if (err == cudaSuccess) err = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
     if (err == cudaSuccess) err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pong_opp_act_kernel, THREADS, SMEM_BYTES);
@@ -395,7 +363,7 @@ int crl_pong_opp_seed(crl_pong_opp* h, uint64_t seed) {
 }
 
 int crl_pong_opp_load_net(crl_pong_opp* h, int32_t slot, const float* params_host, size_t count, void* stream) {
-    CHECK_OPP(h);
+    CHECK_HANDLE(h, h->device);
     if (slot < 0 || slot >= CRL_PONG_OPP_SLOTS) return crl_set_error(CRL_E_INVALID, "network slot must be in [0, %d)", CRL_PONG_OPP_SLOTS);
     if (!params_host || count != (size_t)CRL_PONG_OPP_NET_FLOATS)
         return crl_set_error(CRL_E_INVALID, "a LightActorCritic parameter image has %d floats (got %zu)", CRL_PONG_OPP_NET_FLOATS, count);
@@ -419,7 +387,7 @@ int crl_pong_opp_load_net(crl_pong_opp* h, int32_t slot, const float* params_hos
 }
 
 int crl_pong_opp_set_pool(crl_pong_opp* h, const int32_t* kinds_host, const double* weights_host, int32_t pool_size, void* stream) {
-    CHECK_OPP(h);
+    CHECK_HANDLE(h, h->device);
     if (!kinds_host || pool_size < 1 || pool_size > CRL_PONG_OPP_MAX_POOL)
         return crl_set_error(CRL_E_INVALID, "a pool has 1 to %d entries", CRL_PONG_OPP_MAX_POOL);
     double total = 0.0;
@@ -450,7 +418,7 @@ int crl_pong_opp_set_pool(crl_pong_opp* h, const int32_t* kinds_host, const doub
 }
 
 int crl_pong_opp_assign(crl_pong_opp* h, const int32_t* ids_host, void* stream) {
-    CHECK_OPP(h);
+    CHECK_HANDLE(h, h->device);
     if (h->pool_size == 0) return crl_set_error(CRL_E_STATE, "crl_pong_opp_set_pool first");
     if (ids_host) {
         for (int i = 0; i < h->n; ++i)
@@ -459,14 +427,14 @@ int crl_pong_opp_assign(crl_pong_opp* h, const int32_t* ids_host, void* stream) 
         CUDA_TRY(cudaMemcpyAsync(h->ids, ids_host, sizeof(int32_t) * h->n, cudaMemcpyHostToDevice, (cudaStream_t)stream));
         CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
     } else {
-        LAUNCH((pong_opp_draw_kernel<<<(h->n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(opp_args(h)), cudaGetLastError()));
+        LAUNCH((pong_opp_draw_kernel<<<(h->n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(opp_args(h)), cudaGetLastError()), 1);
     }
     h->assigned = true;
     return CRL_OK;
 }
 
 int crl_pong_opp_restart(crl_pong_opp* h, int32_t clear_stacks, void* stream) {
-    CHECK_OPP(h);
+    CHECK_HANDLE(h, h->device);
     CUDA_TRY(cudaMemsetAsync(h->ret, 0, sizeof(float) * h->n, (cudaStream_t)stream));
     if (clear_stacks) {
         CUDA_TRY(cudaMemsetAsync(h->stack, 0, (size_t)STACK * FRAME * h->n, (cudaStream_t)stream));
@@ -477,7 +445,7 @@ int crl_pong_opp_restart(crl_pong_opp* h, int32_t clear_stacks, void* stream) {
 
 int crl_pong_opp_act(crl_pong_opp* h, const uint8_t* obs1_dev, const float* rew_dev, const uint8_t* done_dev, int32_t resample,
                      int32_t* actions_dev, float* logits_dev, void* stream) {
-    CHECK_OPP(h);
+    CHECK_HANDLE(h, h->device);
     if (!h->assigned) return crl_set_error(CRL_E_STATE, "crl_pong_opp_assign after every crl_pong_opp_set_pool");
     if (!obs1_dev || !actions_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
     if ((rew_dev == nullptr) != (done_dev == nullptr)) return crl_set_error(CRL_E_INVALID, "rew_dev and done_dev go together");
@@ -485,27 +453,23 @@ int crl_pong_opp_act(crl_pong_opp* h, const uint8_t* obs1_dev, const float* rew_
     OppArgs a = opp_args(h);
     a.resample = resample ? 1 : 0;
     a.obs1 = obs1_dev; a.rew = rew_dev; a.done = done_dev; a.actions = actions_dev; a.logits = logits_dev;
-    LAUNCH((pong_opp_act_kernel<<<h->grid, THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(a), cudaGetLastError()));
+    LAUNCH((pong_opp_act_kernel<<<h->grid, THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(a), cudaGetLastError()), 1);
     h->phase = (h->phase + 1) & 3;
     h->steps += 1;
     return CRL_OK;
 }
 
 int crl_pong_opp_get_ids(crl_pong_opp* h, int32_t* ids_dev, void* stream) {
-    CHECK_OPP(h);
+    CHECK_HANDLE(h, h->device);
     if (!ids_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
     CUDA_TRY(cudaMemcpyAsync(ids_dev, h->ids, sizeof(int32_t) * h->n, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return CRL_OK;
 }
 
 int crl_pong_opp_get_stats(crl_pong_opp* h, uint64_t* stats_host, void* stream) {
-    CHECK_OPP(h);
+    CHECK_HANDLE(h, h->device);
     if (!stats_host) return crl_set_error(CRL_E_INVALID, "null buffer");
-    unsigned long long raw[4 * CRL_PONG_OPP_MAX_POOL];
-    CUDA_TRY(cudaMemcpyAsync(raw, h->stats, sizeof raw, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
-    CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
-    for (int k = 0; k < 4 * CRL_PONG_OPP_MAX_POOL; ++k) stats_host[k] = raw[k];
-    return CRL_OK;
+    return crl_read_counters(h->stats, stats_host, 4 * CRL_PONG_OPP_MAX_POOL, (cudaStream_t)stream);
 }
 
 }  // extern "C"
