@@ -11,6 +11,7 @@
 
 #include <atomic>
 #include <mutex>
+#include <string>
 #include <unordered_map>
 #include <vector>
 
@@ -517,9 +518,20 @@ int crl_pong_check(crl_pong* h, void* stream) {
         CUDA_TRY(cudaMemsetAsync(h->dev.serve_overrun, 0, sizeof flag, (cudaStream_t)stream));
         CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
     }
-    if (flag & 2) return crl_set_error(CRL_E_INVALID, "an action outside {0, 1, 2} (cPongDouble: or 999) was passed to step; it was played as 1 (stay)");
-    if (flag & 1) return crl_set_error(CRL_E_SERVES, "injected serve table exhausted");
-    return CRL_OK;
+    if (flag == 0) return CRL_OK;
+    // every flag that is set goes into the one message (they are cleared together); the code is the first one's
+    static const struct { int32_t bit; int code; const char* what; } flags[] = {
+        {4, CRL_E_INVALID, "state outside the set_state domain: crl_pong_set_state left those envs unchanged"},
+        {2, CRL_E_INVALID, "an action outside {0, 1, 2} (cPongDouble: or 999) was passed to step; it was played as 1 (stay)"},
+        {1, CRL_E_SERVES, "injected serve table exhausted"}};
+    std::string msg;
+    int code = CRL_OK;
+    for (const auto& f : flags)
+        if (flag & f.bit) {
+            if (code == CRL_OK) code = f.code;
+            msg += (msg.empty() ? "" : "; ") + std::string(f.what);
+        }
+    return crl_set_error(code, "%s", msg.c_str());
 }
 
 // ---- observation buffers in compressible memory (crl_obs_alloc / crl_obs_free) ----

@@ -55,6 +55,17 @@ __host__ __device__ inline RenderState make_render_state(int bx, int by, int ly,
     return r;
 }
 
+// Both score pairs of two render-state y words lie inside the scoreboard atlas (scores 0..21).  A later point can take a
+// score from 21 to 22 (crl_pong_set_state accepts score 21 with rounds still to play); such a frame shows no text: rows
+// 0..33 are plain white, as the reference's renderer leaves them when the atlas has no strip (oracle/pong_oracle.c).
+// The four score bytes are tested at once: b + 0x6A sets bit 7 exactly when b >= 22, and no byte carries into the next
+// (scores stay below 21 + max_num_rounds <= 42).
+__device__ __forceinline__ bool scores_in_atlas(uint32_t ya, uint32_t yb) {
+    static_assert(ATLAS_SCORES == 0x80 - 0x6A, "the byte test's offset");
+    const uint32_t s = (ya & 0xffffu) | (yb << 16);
+    return ((s + 0x6A6A6A6Au) & 0x80808080u) == 0u;
+}
+
 // cv2 INTER_AREA tap tables (OpenCV computeResizeAreaTab; SURVEY.md A.2). Taps of one
 // destination index are contiguous source indices src0 .. src0+n-1.
 struct AreaTabs {
@@ -102,7 +113,7 @@ struct PongDev {
     // --- validation mode: injected serves ---
     const double* serves;   // [n][K][2] (vx, vy) or nullptr
     int serves_k;
-    int32_t* serve_overrun; // device flag
+    int32_t* serve_overrun; // device flags for crl_pong_check: 1 serve table exhausted, 2 invalid action, 4 set_state row outside the domain
     // episode statistics, accumulated on done: [0] episodes, [1] sum of episode lengths (env-steps),
     // [2] left wins, [3] right wins, [4] draws, [5] sum of (score_left - score_right) + 64*episodes
     unsigned long long* stats;

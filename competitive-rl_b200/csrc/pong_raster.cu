@@ -39,6 +39,7 @@ __global__ void pong_build_tables_kernel(PongDev p, uint8_t* text_tab, uint8_t* 
 #pragma unroll
         for (int k = 0; k < 6; ++k) c.rect[k] = 0u;
         c.any_valid = true;
+        c.blank = false;
         int pix;
         uint8_t* dst;
         if (i < (long long)entries * p.text_stride) {
@@ -127,7 +128,9 @@ __global__ void pong_raw_frame_kernel(PongDev p, int env, uint8_t* rgb0, uint8_t
     const int bx = (int16_t)(b & 0xffff), by = (int16_t)(b >> 16), ly = t & 0xffff, ry = (t >> 16) & 0xffff;
     const int pair = (s & 0xff) * ATLAS_SCORES + ((s >> 8) & 0xff);
     uint8_t r, g, bl;
-    if (y < ATLAS_ROWS) {
+    if (y < ATLAS_ROWS && !scores_in_atlas((uint32_t)s, (uint32_t)s)) {
+        r = g = bl = 255;   // a score past 21: no text
+    } else if (y < ATLAS_ROWS) {
         const uint8_t* a = p.atlas + ((size_t)(pair * ATLAS_ROWS + y) * SCREEN_W + x) * 3;
         r = a[0]; g = a[1]; bl = a[2];
     } else if (y >= ARENA_BOTTOM) {

@@ -11,6 +11,7 @@ namespace crl {
 struct FrameCtx {
     uint32_t rect[6];   // x0 | x1<<8 | y0<<16 | y1<<24 (arena-clipped; 0 = empty)
     int pairA, pairB;   // atlas score-pair index l*22+r of the two frames
+    bool blank;         // a frame's score pair is outside the atlas: the rows above the arena are white (no text)
     bool mirror;
     bool any_valid;
 };
@@ -31,8 +32,9 @@ __device__ __forceinline__ FrameCtx make_ctx(const FrameSpec f, const int agent)
     c.mirror = agent != 0;
     if (!va) { ax = bx; ay = by; }      // max(0-frame, X) = X
     if (!vb) { bx = ax; by = ay; }
-    c.pairA = (int)(ay & 255u) * ATLAS_SCORES + (int)((ay >> 8) & 255u);
-    c.pairB = (int)(by & 255u) * ATLAS_SCORES + (int)((by >> 8) & 255u);
+    c.blank = !scores_in_atlas(ay, by);
+    c.pairA = c.blank ? 0 : (int)(ay & 255u) * ATLAS_SCORES + (int)((ay >> 8) & 255u);
+    c.pairB = c.blank ? 0 : (int)(by & 255u) * ATLAS_SCORES + (int)((by >> 8) & 255u);
     {
         const int x = ax & 255u, y = (ax >> 8) & 255u, l = (ax >> 16) & 255u, r = (ax >> 24) & 255u;
         c.rect[0] = pack_rect(x, x + BALL_SIZE, y, y + BALL_SIZE, c.mirror);
@@ -58,6 +60,7 @@ __device__ __forceinline__ uint32_t span_bits(int lo, int hi, int s0, int n) {
 
 // gray value of the max-pooled source pixel in the rows above the arena
 __device__ __forceinline__ int text_gray(const FrameCtx& c, const uint8_t* __restrict__ atlas, int sy, int sx) {
+    if (c.blank) return 255;   // max(white, X) = white; gray(255, 255, 255) = 255
     const int ax = (c.mirror && sy >= MIRROR_ROW) ? (SCREEN_W - 1 - sx) : sx;
     const uint8_t* pa = atlas + ((size_t)(c.pairA * ATLAS_ROWS + sy) * SCREEN_W + ax) * 3;
     const uint8_t* pb = atlas + ((size_t)(c.pairB * ATLAS_ROWS + sy) * SCREEN_W + ax) * 3;
@@ -69,6 +72,7 @@ __device__ __forceinline__ int text_gray(const FrameCtx& c, const uint8_t* __res
 // fma(B, 0.114f, fma(R, 0.299f, G * 0.587f)) in fp32 -- pinned against cv2 4.13 on random and Pong-like images
 // (tests/test_oracle_cv2.py); pure white gives exactly 255.0f, so only the antialiased text pixels differ from text_gray
 __device__ __forceinline__ float text_gray_f32(const FrameCtx& c, const uint8_t* __restrict__ atlas, int sy, int sx) {
+    if (c.blank) return 255.f;
     const int ax = (c.mirror && sy >= MIRROR_ROW) ? (SCREEN_W - 1 - sx) : sx;
     const uint8_t* pa = atlas + ((size_t)(c.pairA * ATLAS_ROWS + sy) * SCREEN_W + ax) * 3;
     const uint8_t* pb = atlas + ((size_t)(c.pairB * ATLAS_ROWS + sy) * SCREEN_W + ax) * 3;

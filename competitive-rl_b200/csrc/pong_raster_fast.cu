@@ -160,11 +160,13 @@ __global__ void pong_build_bat_lut_kernel(FastTabs<DIM>* T) {
 }
 
 // Scoreboard rows for a score combination that is not in text_tab (the two pooled frames differ by
-// more than one point: only reachable through crl_pong_set_state): exact evaluation straight from
-// the atlas.  Arena taps count as black here; pixels that also see a rectangle are overwritten by
-// the bat/ball patches, which (fast_ok) treat the atlas rows they share a destination row with as white.
+// more than one point, or a score is past 21 (blank: white rows, no text); only reachable through
+// crl_pong_set_state): exact evaluation straight from the atlas.  Arena taps count as black here; pixels that
+// also see a rectangle are overwritten by the bat/ball patches, which (fast_ok) treat the atlas rows they share
+// a destination row with as white.  Reached from game states only with blank: two different in-atlas pairs need a
+// history frame pooling buffers more than one point apart, which exists only in terminal observations (generic kernel).
 __device__ __forceinline__ uint8_t eval_text_pixel(const AreaTabs* __restrict__ T, const uint8_t* __restrict__ atlas,
-                                                   int pairA, int pairB, bool mirror, int dy, int dx) {
+                                                   int pairA, int pairB, bool blank, bool mirror, int dy, int dx) {
     const int sx0 = T->x_src0[dx], nx = T->x_n[dx], sy0 = T->y_src0[dy], ny = T->y_n[dy];
     float sum = 0.f;
     for (int ty = 0; ty < ny; ++ty) {
@@ -172,7 +174,9 @@ __device__ __forceinline__ uint8_t eval_text_pixel(const AreaTabs* __restrict__ 
         float buf = 0.f;
         for (int tx = 0; tx < nx; ++tx) {
             int g = 0;
-            if (sy < ARENA_TOP) {
+            if (sy < ARENA_TOP && blank) {
+                g = 255;
+            } else if (sy < ARENA_TOP) {
                 const int sx = sx0 + tx;
                 const int ax = (mirror && sy >= MIRROR_ROW) ? (SCREEN_W - 1 - sx) : sx;
                 const uint8_t* pa = atlas + ((size_t)(pairA * ATLAS_ROWS + sy) * SCREEN_W + ax) * 3;
@@ -200,13 +204,14 @@ __device__ __forceinline__ uint32_t spec_diff(const FrameSpec& a, const FrameSpe
     return (a.x ^ b.x) | ((a.y ^ b.y) & nr) | (a.z ^ b.z) | ((a.w ^ b.w) & nr);
 }
 
-// scoreboard entry of a frame (the kernel's text_id), -2 when its score combination is outside text_tab; any_valid = 0: the
-// all-zero frame
+// scoreboard entry of a frame (the kernel's text_id), -2 when its score combination is outside text_tab (also: a score
+// past the atlas); any_valid = 0: the all-zero frame
 __device__ __forceinline__ int frame_text_id(FrameSpec f, int agent, bool& any_valid) {
     const bool va = (f.y >> 16) & 1u, vb = (f.w >> 16) & 1u;
     any_valid = va || vb;
     if (!va) f.y = f.w;
     if (!vb) f.w = f.y;
+    if (!scores_in_atlas(f.y, f.w)) return -2;
     const int pairA = (int)(f.y & 255u) * ATLAS_SCORES + (int)((f.y >> 8) & 255u);
     const int pairB = (int)(f.w & 255u) * ATLAS_SCORES + (int)((f.w >> 8) & 255u);
     int base = pairA, kind = 0;
@@ -377,11 +382,14 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
             const int pairA = (int)(f.y & 255u) * ATLAS_SCORES + (int)((f.y >> 8) & 255u);
             const int pairB = (int)(f.w & 255u) * ATLAS_SCORES + (int)((f.w >> 8) & 255u);
             int base = pairA, kind = 0;
-            bool text_ok = true;
-            if (pairA != pairB) {   // one point scored between the two pooled frames
+            const bool blank = !scores_in_atlas(f.y, f.w);   // a score past 21: no text, never a table index
+            bool text_ok = !blank;
+            if (text_ok && pairA != pairB) {   // one point scored between the two pooled frames
                 const int d = pairB - pairA;
                 if (d == ATLAS_SCORES) kind = 1;
                 else if (d == 1 && (pairA % ATLAS_SCORES) != ATLAS_SCORES - 1) kind = 2;
+                // d < 0 and |d| not in {1, 22} are not reached from game states: a history frame pools sub-steps 2 and 3 of
+                // one step (a done replaces the whole history), so frame B never shows fewer points, nor two more, than A
                 else if (d == -ATLAS_SCORES) { base = pairB; kind = 1; }
                 else if (d == -1 && (pairB % ATLAS_SCORES) != ATLAS_SCORES - 1) { base = pairB; kind = 2; }
                 else text_ok = false;
@@ -530,7 +538,7 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
                 } else {   // score combination outside the table: exact rows straight from the atlas
                     const int n_text = p.tabs->text_rows * DIM;
                     for (int i = lane; i < n_text; i += 32)
-                        sm8[i] = eval_text_pixel(p.tabs, p.atlas, pairA, pairB, agent != 0, i / DIM, i % DIM);
+                        sm8[i] = eval_text_pixel(p.tabs, p.atlas, pairA, pairB, blank, agent != 0, i / DIM, i % DIM);
                 }
                 cur_text = text_id;
                 __syncwarp();
@@ -615,7 +623,7 @@ pong_raster_fast_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
 // (a bat touches <= 4 destination rows and exactly two destination columns -> one 16-bit store), per pooled ball the
 // <= 3 x 2 destination pixels.  The quad is then drained as one flat run of 16-byte st.global.cs (1 764 is not a multiple
 // of 16, 7 056 is), instead of 4-byte stores.  Arithmetic is the kernel's above, so the results are bit-identical.
-// Quads containing an unusual frame (both pool buffers zero, score combination outside text_tab) are evaluated exactly,
+// Quads containing an unusual frame (both pool buffers zero, score combination outside text_tab or past the atlas) are evaluated exactly,
 // pixel by pixel, like pong_raster_generic_kernel does.
 // the tables of FastTabs the quad kernel keeps in shared memory (the bat LUT narrowed to the two columns a bat touches)
 template <int DIM> struct alignas(16) QuadTabs {
@@ -736,12 +744,12 @@ pong_raster_quad_kernel(PongDev p, const FrameSpec* __restrict__ hist, uint8_t* 
         const int pairA = (int)(f.y & 255u) * ATLAS_SCORES + (int)((f.y >> 8) & 255u);
         const int pairB = (int)(f.w & 255u) * ATLAS_SCORES + (int)((f.w >> 8) & 255u);
         int base = pairA, kind = 0;
-        bool text_ok = true;
-        if (pairA != pairB) {   // one point scored between the two pooled frames
+        bool text_ok = scores_in_atlas(f.y, f.w);            // a score past 21: the exact path draws no text
+        if (text_ok && pairA != pairB) {   // one point scored between the two pooled frames
             const int d = pairB - pairA;
             if (d == ATLAS_SCORES) kind = 1;
             else if (d == 1 && (pairA % ATLAS_SCORES) != ATLAS_SCORES - 1) kind = 2;
-            else if (d == -ATLAS_SCORES) { base = pairB; kind = 1; }
+            else if (d == -ATLAS_SCORES) { base = pairB; kind = 1; }   // d < 0: not reached from game states (see above)
             else if (d == -1 && (pairB % ATLAS_SCORES) != ATLAS_SCORES - 1) { base = pairB; kind = 2; }
             else text_ok = false;
         }

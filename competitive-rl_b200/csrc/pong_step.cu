@@ -314,11 +314,27 @@ __global__ void pong_get_state_kernel(PongDev p, double* state) {
     s[6] = g.score_left; s[7] = g.score_right; s[8] = g.num_rounds; s[9] = g.num_steps;
 }
 
+// v is an integer in [lo, hi] (false for NaN)
+__device__ __forceinline__ bool int_in(double v, double lo, double hi) { return v >= lo && v <= hi && v == trunc(v); }
+
+// The set_state domain (include/crl_b200.h): every field fits the packed state and the 8-bit render-state coordinates,
+// and every score has an atlas strip.  A row outside it is not applied; crl_pong_check reports it (flag bit 4).
+__device__ __forceinline__ bool state_in_domain(const double* s, int max_rounds) {
+    return int_in(s[0], 0.0, (double)(SCREEN_W - BALL_SIZE)) && int_in(s[1], 0.0, (double)(ARENA_BOTTOM - BALL_SIZE)) &&
+           fabs(s[2]) <= 64.0 && fabs(s[3]) <= 64.0 && int_in(s[4], 0.0, 255.0) && int_in(s[5], 0.0, 255.0) &&
+           int_in(s[6], 0.0, (double)(ATLAS_SCORES - 1)) && int_in(s[7], 0.0, (double)(ATLAS_SCORES - 1)) &&
+           int_in(s[8], 0.0, (double)(max_rounds - 1)) && int_in(s[9], 0.0, (double)MAX_STEP_PER_ROUND);
+}
+
 __global__ void pong_set_state_kernel(PongDev p, const double* state) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= p.n) return;
-    Game g = load_game(p, e);
     const double* s = state + (size_t)e * 10;
+    if (!state_in_domain(s, p.max_rounds)) {
+        atomicOr(p.serve_overrun, 4);
+        return;
+    }
+    Game g = load_game(p, e);
     g.ball_x = (int)s[0]; g.ball_y = (int)s[1]; g.vx = s[2]; g.vy = s[3]; g.left_y = (int)s[4]; g.right_y = (int)s[5];
     g.score_left = (int)s[6]; g.score_right = (int)s[7]; g.num_rounds = (int)s[8]; g.num_steps = (int)s[9];
     store_game(p, e, g);

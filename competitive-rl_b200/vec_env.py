@@ -485,10 +485,14 @@ class CudaPongVecEnv(VecEnv):
         return s
 
     def set_state(self, state):
+        """Write (N, 10) game states laid out as get_state() returns them.  Rows outside the set_state domain
+        (include/crl_b200.h: positions on the board, |v| <= 64, scores 0..21, num_rounds < max_num_rounds, integral
+        integer fields) are not applied and raise CrlError here, as does any other pending device error (see check())."""
         s = torch.as_tensor(state, dtype=torch.float64).to(self.device).contiguous()
         assert tuple(s.shape) == (self.num_envs, 10)
         self._impl.set_state(s)
         torch.cuda.current_stream(self.device).synchronize()
+        self.check()
 
     def forget_obs(self):
         """After writing into observation tensors this env returned: the next render into each buffer rewrites it whole."""

@@ -158,7 +158,20 @@ int crl_pong_step_host(crl_pong* h, const int32_t* actions_host, uint8_t* obs0_d
                        int32_t* num_steps_host, float* real_reward_host, void* stream);
 
 /* Game state, float64 [num_envs][10]: ball_x, ball_y, vx, vy, left_y, right_y,
- * score_left, score_right, num_rounds, num_steps (PongGame fields). */
+ * score_left, score_right, num_rounds, num_steps (PongGame fields).
+ *
+ * crl_pong_set_state writes the game state only: Bat._current_move, the serve counter, the
+ * MaxAndSkip buffers and the FrameStack history keep what they held.  Integer fields take the
+ * C (int) truncation, vx / vy are stored as given.  The set_state domain, per row:
+ *   ball_x in [0, 156], ball_y in [0, 190], left_y and right_y in [0, 255],
+ *   vx and vy finite with |v| <= 64, score_left and score_right in [0, 21],
+ *   num_rounds in [0, max_num_rounds - 1], num_steps in [0, 10000],
+ *   every integer field integral.
+ * The check runs on the device: a row outside the domain is not applied (that env keeps its
+ * state) and the next crl_pong_check returns CRL_E_INVALID ("state outside the set_state domain").
+ * A point scored after set_state can still take a score from 21 to 22 (when rounds remain):
+ * the scoreboard atlas has no strip for such a score, and, as the reference's renderer leaves
+ * them without a strip, frames showing it have plain white rows 0..33, no text. */
 int crl_pong_get_state(crl_pong* h, double* state_dev, void* stream);
 int crl_pong_set_state(crl_pong* h, const double* state_dev, void* stream);
 
@@ -181,7 +194,10 @@ int crl_pong_get_stats(crl_pong* h, uint64_t* stats_host, void* stream);
  * gpu_launches), and the deferred error check (synchronises): CRL_E_SERVES after a
  * serve-table overrun, CRL_E_INVALID after a step saw an action outside {0, 1, 2}
  * (cPongDouble: or 999) -- the reference asserts / raises IndexError there
- * (pong/base_pong_env.py:42, :124, :134); the device step plays it as 1 (stay). */
+ * (pong/base_pong_env.py:42, :124, :134); the device step plays it as 1 (stay) -- and
+ * CRL_E_INVALID after crl_pong_set_state refused a row outside the set_state domain.  The flags
+ * are cleared once reported; when several are set, the message names each of them and the code is
+ * the first one's in this order: set_state domain, action, serve table. */
 uint64_t crl_launch_count(void);
 int crl_pong_check(crl_pong* h, void* stream);
 

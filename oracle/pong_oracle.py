@@ -40,8 +40,35 @@ def lib():
         L.pong_oracle_set_threads.argtypes = [ctypes.c_int]
         L.pong_oracle_serve_overrun.argtypes = [ctypes.c_void_p]
         L.pong_oracle_serve_overrun.restype = ctypes.c_int
+        L.pong_oracle_game_ptr.restype = ctypes.POINTER(Game)
+        L.pong_oracle_game_ptr.argtypes = [ctypes.c_void_p, ctypes.c_int]
         _lib = L
     return _lib
+
+
+class Game(ctypes.Structure):
+    """pong_oracle.c's Game: one env's PongGame fields (pong_oracle_game_ptr)."""
+    _fields_ = [("ball_x", ctypes.c_int), ("ball_y", ctypes.c_int), ("vx", ctypes.c_double),
+                ("vy", ctypes.c_double), ("left_y", ctypes.c_int), ("right_y", ctypes.c_int),
+                ("left_move", ctypes.c_int), ("right_move", ctypes.c_int), ("score_left", ctypes.c_int),
+                ("score_right", ctypes.c_int), ("num_rounds", ctypes.c_int), ("num_steps", ctypes.c_int)]
+
+
+# get_state() column -> Game field; vx / vy (columns 2, 3) are the float fields
+STATE_FIELDS = ("ball_x", "ball_y", "vx", "vy", "left_y", "right_y", "score_left", "score_right", "num_rounds", "num_steps")
+
+
+def state_in_domain(state, max_rounds=21):
+    """(N,) bool: the rows of an (N, 10) get_state()-layout array inside the set_state domain of include/crl_b200.h
+    (ball_x 0..156, ball_y 0..190, bats 0..255, finite |vx|, |vy| <= 64, scores 0..21, num_rounds 0..max_rounds-1,
+    num_steps 0..10000, integer fields integral)."""
+    s = np.asarray(state, np.float64).reshape(-1, 10)
+    with np.errstate(invalid="ignore"):
+        ok = (np.abs(s[:, 2]) <= 64) & (np.abs(s[:, 3]) <= 64)
+        for col, hi in ((0, 156), (1, 190), (4, 255), (5, 255), (6, 21), (7, 21), (8, max_rounds - 1), (9, 10000)):
+            v = s[:, col]
+            ok &= (v >= 0) & (v <= hi) & (v == np.trunc(v))
+    return ok
 
 
 def _p(a):
@@ -139,6 +166,17 @@ class PongOracleVec(object):
         s = np.zeros((self.n, 10), np.float64)
         lib().pong_oracle_get_state(self._h, _p(s))
         return s
+
+    def set_state(self, state):
+        """Write (N, 10) game states in get_state()'s layout, as crl_pong_set_state does on the GPU: integer fields take
+        the C (int) truncation, vx / vy are stored as given; Bat._current_move, the serve counter, ClipRewardEnv's step
+        count, the MaxAndSkip buffers and the FrameStack deque keep what they held.  No domain check: the caller keeps
+        the rows inside state_in_domain()."""
+        s = np.asarray(state, np.float64).reshape(self.n, 10)
+        for i in range(self.n):
+            g = lib().pong_oracle_game_ptr(self._h, i).contents
+            for k, name in enumerate(STATE_FIELDS):
+                setattr(g, name, float(s[i, k]) if k in (2, 3) else int(s[i, k]))
 
     def render_raw(self, i):
         f0 = np.empty((210, 160, 3), np.uint8)
