@@ -28,6 +28,7 @@ EXPORTS = [
     "crl_obs_alloc", "crl_obs_free",
     "crl_pong_opp_create", "crl_pong_opp_destroy", "crl_pong_opp_seed", "crl_pong_opp_load_net", "crl_pong_opp_set_pool",
     "crl_pong_opp_assign", "crl_pong_opp_restart", "crl_pong_opp_act", "crl_pong_opp_get_ids", "crl_pong_opp_get_stats",
+    "crl_pong_opp_set_pairs", "crl_pong_opp_act_pairs", "crl_pong_opp_get_pair_stats",
 ]
 
 
@@ -157,6 +158,9 @@ def load():
     L.crl_pong_opp_act.argtypes = [vp, vp, vp, vp, i32, vp, vp, vp]
     L.crl_pong_opp_get_ids.argtypes = [vp, vp, vp]
     L.crl_pong_opp_get_stats.argtypes = [vp, vp, vp]
+    L.crl_pong_opp_set_pairs.argtypes = [vp, vp, i32, vp]
+    L.crl_pong_opp_act_pairs.argtypes = [vp] * 8
+    L.crl_pong_opp_get_pair_stats.argtypes = [vp, vp, i32, vp]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("crl_last_error", "crl_launch_count"):

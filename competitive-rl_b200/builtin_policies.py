@@ -189,6 +189,42 @@ def is_light_agent(agent_name):
     return agent_name in _CHECKPOINTS and _CHECKPOINTS[agent_name][1]
 
 
+def light_network_image(name, added=None, resource_dir=None):
+    """The packed LightActorCritic image (pack_light_actor_critic) of the network pool entry `name`, as the opponent
+    kernel loads it: added[name] when `added` (name -> packed image) has it, else the built-in agent's checkpoint.
+    ValueError for an ActorCritic agent (STRONG / ALPHA_PONG) and for a name with neither."""
+    if added and name in added:
+        return added[name]
+    if name in BUILTIN_AGENT_NAMES and not is_light_agent(name):
+        raise ValueError("%s is an ActorCritic agent: per-env pools take RULE_BASED, RANDOM and LightActorCritic "
+                         "networks (WEAK, MEDIUM or add_opponent) only" % name)
+    path = find_checkpoint(name, resource_dir)
+    if path is None:
+        raise ValueError("unknown opponent %r: not RULE_BASED / RANDOM, not added with add_opponent, and no "
+                         "checkpoint found" % (name,))
+    return pack_light_actor_critic(torch.load(path, map_location="cpu", weights_only=True))
+
+
+def resolve_pool(pool, added=None, resource_dir=None):
+    """A pool of names as the opponent kernel takes it (include/crl_b200.h, crl_pong_opp_set_pool): (names, kinds,
+    images).  kinds[k] is entry k's kind: CRL_PONG_OPP_RULE_BASED, CRL_PONG_OPP_RANDOM or a network slot.  Networks
+    take slots 0, 1, ... in pool order, and images[s] is slot s's image (light_network_image, `added` first).
+    ValueError, before anything is loaded, for a pool that is not 1 to 16 distinct names, for more than 8 networks and
+    for a name light_network_image refuses."""
+    from . import _native
+    ext = _native.ext()
+    names = [str(p) for p in pool]
+    if not 1 <= len(names) <= ext.OPP_MAX_POOL or len(set(names)) != len(names):
+        raise ValueError("a pool is 1 to %d distinct names" % ext.OPP_MAX_POOL)
+    nets = [p for p in names if p not in ("RULE_BASED", "RANDOM")]
+    if len(nets) > ext.OPP_SLOTS:
+        raise ValueError("a pool holds at most %d networks" % ext.OPP_SLOTS)
+    images = [light_network_image(p, added, resource_dir) for p in nets]
+    kinds = [ext.OPP_RULE_BASED if p == "RULE_BASED" else ext.OPP_RANDOM if p == "RANDOM" else nets.index(p)
+             for p in names]
+    return names, kinds, images
+
+
 def get_compute_action_function(agent_name, num_envs=1, device="cuda", resource_dir=None):
     """Callable obs -> int32 [num_envs] device tensor (pong/builtin_policies.py:61-91)."""
     device = torch.device(device)

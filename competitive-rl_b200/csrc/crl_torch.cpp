@@ -316,6 +316,28 @@ struct PongOpponents {
         check_rc(crl_pong_opp_get_stats(handle(), s.data(), stream_of(device)));
         return s;
     }
+    // league mode.  pairs: int32 CPU tensor [P][2] of pool indices (seat 0, seat 1)
+    void set_pairs(const at::Tensor& pairs) {
+        TORCH_CHECK(pairs.dim() == 2 && pairs.size(1) == 2, "pairs: expected shape (P, 2)");
+        check_rc(crl_pong_opp_set_pairs(handle(), host_ptr<int32_t>(pairs, at::kInt, "pairs"), (int32_t)pairs.size(0),
+                                        stream_of(device)));
+    }
+    void act_pairs(const at::Tensor& obs0, const at::Tensor& obs1, const c10::optional<at::Tensor>& rew,
+                   const c10::optional<at::Tensor>& done, const at::Tensor& actions, const c10::optional<at::Tensor>& logits) {
+        check_rc(crl_pong_opp_act_pairs(handle(), dev_ptr<uint8_t>(obs0, at::kByte, device, n() * 42 * 42, "obs0"),
+                                        dev_ptr<uint8_t>(obs1, at::kByte, device, n() * 42 * 42, "obs1"),
+                                        opt_dev_ptr<float>(rew, at::kFloat, device, 2 * n(), "rew"),
+                                        opt_dev_ptr<uint8_t>(done, at::kBool, device, n(), "done"),
+                                        dev_ptr<int32_t>(actions, at::kInt, device, 2 * n(), "actions"),
+                                        opt_dev_ptr<float>(logits, at::kFloat, device, 6 * n(), "logits"), stream_of(device)));
+    }
+    // [P * 4]: episodes, wins, draws, losses of seat 0 per pairing
+    std::vector<uint64_t> pair_stats(int64_t num_pairs) {
+        TORCH_CHECK(num_pairs >= 1 && num_pairs <= CRL_PONG_OPP_MAX_PAIRS, "num_pairs must be in [1, ", CRL_PONG_OPP_MAX_PAIRS, "]");
+        std::vector<uint64_t> s(4 * num_pairs);
+        check_rc(crl_pong_opp_get_pair_stats(handle(), s.data(), (int32_t)num_pairs, stream_of(device)));
+        return s;
+    }
 };
 
 // An uninitialised observation buffer: crl_obs_alloc's memory (compressible where the device grants it) viewed as a tensor
@@ -390,6 +412,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
     m.attr("OPP_MAX_POOL") = CRL_PONG_OPP_MAX_POOL;
     m.attr("OPP_RULE_BASED") = CRL_PONG_OPP_RULE_BASED;
     m.attr("OPP_RANDOM") = CRL_PONG_OPP_RANDOM;
+    m.attr("OPP_MAX_PAIRS") = CRL_PONG_OPP_MAX_PAIRS;
     py::class_<PongOpponents>(m, "PongOpponents")
         .def(py::init<int64_t, int64_t, uint64_t, int64_t>())
         .def("close", &PongOpponents::close)
@@ -400,5 +423,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
         .def("restart", &PongOpponents::restart)
         .def("act", &PongOpponents::act)
         .def("ids", &PongOpponents::ids)
-        .def("stats", &PongOpponents::stats);
+        .def("stats", &PongOpponents::stats)
+        .def("set_pairs", &PongOpponents::set_pairs)
+        .def("act_pairs", &PongOpponents::act_pairs)
+        .def("pair_stats", &PongOpponents::pair_stats);
 }

@@ -12,6 +12,11 @@
 // The networks run on the SIMT fp32 pipe with explicit __fmaf_rn (the library is compiled with -fmad=false).  Each CTA
 // owns a contiguous range of envs; it sorts them by network slot in shared memory and then runs every slot present
 // with that slot's weights staged once in shared memory, one env at a time over all its threads.
+//
+// League mode (crl_pong_opp_set_pairs / crl_pong_opp_act_pairs) is the same kernel instantiated for two seats: env g
+// plays pairing g mod P, both seats act from their own stack (seat 0 from agent 0's frames, seat 1 from agent 1's),
+// and a finished episode is credited to the pairing.  The per-env thread files one work item per network seat, so a
+// slot's weights are still staged once per 64-env chunk whichever seats use it.
 #include <string.h>
 
 #include <cmath>
@@ -57,7 +62,11 @@ static_assert(SD_END == CRL_PONG_OPP_NET_FLOATS, "flat layout of the header");
 // shared memory of the act kernel (floats unless noted); h2 reuses the input stack, which conv1 is done with
 constexpr int SM_W = 0, SM_X = SM_W + NET_DEV, SM_H1 = SM_X + STACK * FRAME, SM_LUT = SM_H1 + C1 * H1 * H1,
               SM_RED = SM_LUT + 256, SM_FLOATS = SM_RED + 8 * 3;
-constexpr size_t SMEM_BYTES = SM_FLOATS * sizeof(float) + CRL_PONG_OPP_SLOTS * SUB + 16 * sizeof(int);
+// + the work list uint8 [slot][SEATS * SUB] and its counts int [16]
+template <int SEATS>
+constexpr size_t smem_bytes() { return SM_FLOATS * sizeof(float) + CRL_PONG_OPP_SLOTS * SUB * SEATS + 16 * sizeof(int); }
+constexpr size_t SMEM_BYTES = smem_bytes<1>();
+static_assert(SUB <= 64, "a league work item is (env in chunk) | seat << 6");
 
 constexpr int KIND_RULE = CRL_PONG_OPP_RULE_BASED;   // CRL_PONG_OPP_RANDOM is the other negative kind
 
@@ -80,11 +89,17 @@ struct OppArgs {
     uint8_t* stack;           // [n][4][1764]
     float* ret;               // [n] agent 0's summed clipped reward of the episode in progress
     uint32_t* episodes;       // [n] episodes finished since the handle was created (the draw counter)
-    unsigned long long* stats;   // [16][4] episodes, wins, draws, losses of agent 0
+    unsigned long long* stats;   // [16][4] (league: [P][4]) episodes, wins, draws, losses of agent 0
     const float* nets;        // [8][NET_DEV]
+    // league mode only (SEATS == 2); the fields above keep their offsets in the parameter block
+    int num_pairs;
+    uint8_t pairs[CRL_PONG_OPP_MAX_PAIRS][2];   // pool index of seat 0, seat 1
+    const uint8_t* obs0;      // [n][1764] agent 0's observation of the previous step
+    uint8_t* stack0;          // [n][4][1764] seat 0's stacks; `stack` holds seat 1's
 };
 
-// Philox streams: (global env, tag) x counter, keyed by the seed.  tag 1 = RANDOM's actions, tag 2 = opponent draws.
+// Philox streams: (global env, tag) x counter, keyed by the seed.  tag 1 = RANDOM's actions (seat 1), tag 2 = opponent
+// draws, tag 3 = RANDOM's actions in seat 0 (league mode).
 __device__ __forceinline__ uint32_t opp_rand(uint64_t seed, int64_t g, uint32_t tag, uint64_t ctr) {
     uint32_t r[4];
     philox4x32_10((uint32_t)g, (uint32_t)((uint64_t)g >> 32) ^ (tag << 24), (uint32_t)ctr, (uint32_t)(ctr >> 32),
@@ -99,6 +114,8 @@ __device__ __forceinline__ int opp_draw(const OppArgs& a, int64_t g, uint32_t ep
     return k;
 }
 
+// SEATS == 1: column 1 of the step buffer (the per-env opponents); SEATS == 2: both columns (league mode)
+template <int SEATS>
 __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs a) {
     extern __shared__ __align__(16) float sm[];
     float* const w = sm + SM_W;
@@ -107,8 +124,8 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
     float* const h2 = xs;
     float* const lut = sm + SM_LUT;
     float* const red = sm + SM_RED;
-    uint8_t* const list = (uint8_t*)(sm + SM_FLOATS);             // [slot][SUB]
-    int* const cnt = (int*)(list + CRL_PONG_OPP_SLOTS * SUB);   // [slot]
+    uint8_t* const list = (uint8_t*)(sm + SM_FLOATS);                     // [slot][SEATS * SUB]
+    int* const cnt = (int*)(list + CRL_PONG_OPP_SLOTS * SUB * SEATS);   // [slot]
     const int tid = threadIdx.x;
 
     for (int b = tid; b < 256; b += THREADS) lut[b] = (float)b / 255.0f;
@@ -118,7 +135,7 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
         if (tid < CRL_PONG_OPP_SLOTS) cnt[tid] = 0;
         __syncthreads();
         // ---- per env: bookkeeping of the step before, redraw, actions of the non-network kinds, sort by slot
-        if (tid < ne) {
+        if (SEATS == 1 && tid < ne) {
             const int i = e0 + tid;
             const int64_t g = a.first_env + i;
             int id = a.ids[i];
@@ -147,10 +164,43 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
                 if (a.logits) a.logits[3 * i] = a.logits[3 * i + 1] = a.logits[3 * i + 2] = 0.f;
             }
         }
-        // ---- the newest frame into ring slot `phase` of every env of the range
-        {
-            const uint32_t* src = (const uint32_t*)(a.obs1 + (size_t)e0 * FRAME);
-            uint32_t* dst = (uint32_t*)(a.stack + (size_t)e0 * STACK * FRAME + (size_t)a.phase * FRAME);
+        if (SEATS == 2 && tid < ne) {   // league: the env's pairing is fixed by its global index
+            const int i = e0 + tid;
+            const int64_t g = a.first_env + i;
+            int64_t pr = g % a.num_pairs;
+            if (pr < 0) pr += a.num_pairs;
+            const int p = (int)pr;
+            if (a.rew) {
+                float r = a.ret[i] + a.rew[2 * i];
+                if (a.done[i]) {
+                    unsigned long long* st = a.stats + 4 * p;
+                    atomicAdd(st, 1ull);
+                    atomicAdd(st + (r > 0.f ? 1 : r == 0.f ? 2 : 3), 1ull);
+                    r = 0.f;
+                }
+                a.ret[i] = r;
+            }
+#pragma unroll
+            for (int seat = 0; seat < 2; ++seat) {
+                const int kind = a.kind[a.pairs[p][seat]];
+                if (kind >= 0) {
+                    list[kind * 2 * SUB + atomicAdd(&cnt[kind], 1)] = (uint8_t)(tid | seat << 6);
+                } else {
+                    a.actions[2 * i + seat] =
+                        kind == KIND_RULE ? CHEAT_CODES
+                                          : (int32_t)(((uint64_t)opp_rand(a.seed, g, seat ? 1u : 3u, a.step) * 3u) >> 32);
+                    if (a.logits) {
+                        float* lg = a.logits + 6 * i + 3 * seat;
+                        lg[0] = lg[1] = lg[2] = 0.f;
+                    }
+                }
+            }
+        }
+        // ---- the newest frame into ring slot `phase` of every env of the range (league: of both seats' stacks)
+#pragma unroll
+        for (int seat = 2 - SEATS; seat < 2; ++seat) {
+            const uint32_t* src = (const uint32_t*)((seat ? a.obs1 : a.obs0) + (size_t)e0 * FRAME);
+            uint32_t* dst = (uint32_t*)((seat ? a.stack : a.stack0) + (size_t)e0 * STACK * FRAME + (size_t)a.phase * FRAME);
             for (int k = tid; k < ne * FRAME_WORDS; k += THREADS) {
                 const int e = k / FRAME_WORDS, j = k - e * FRAME_WORDS;
                 dst[(size_t)e * STACK * FRAME_WORDS + j] = src[k];
@@ -166,9 +216,11 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
                 for (int k = tid; k < NET_DEV / 4; k += THREADS) ((float4*)w)[k] = src[k];
             }
             for (int q = 0; q < m; ++q) {
-                const int i = e0 + list[s * SUB + q];
+                const int item = list[s * SEATS * SUB + q];
+                const int i = e0 + (SEATS == 1 ? item : item & (SUB - 1));
+                const int seat = SEATS == 1 ? 1 : item >> 6;
                 {   // stack / 255 -> xs[ci][42][42], ci 0 = oldest
-                    const uint32_t* src = (const uint32_t*)(a.stack + (size_t)i * STACK * FRAME);
+                    const uint32_t* src = (const uint32_t*)((SEATS == 1 || seat ? a.stack : a.stack0) + (size_t)i * STACK * FRAME);
                     for (int k = tid; k < STACK * FRAME_WORDS; k += THREADS) {
                         const int ci = k / FRAME_WORDS, j = k - ci * FRAME_WORDS;
                         const uint32_t v = src[((a.phase + 1 + ci) & 3) * FRAME_WORDS + j];
@@ -266,8 +318,11 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
                     float best = l[0];
                     if (l[1] > best) { act = 1; best = l[1]; }
                     if (l[2] > best) act = 2;
-                    a.actions[2 * i + 1] = act;
-                    if (a.logits) { a.logits[3 * i] = l[0]; a.logits[3 * i + 1] = l[1]; a.logits[3 * i + 2] = l[2]; }
+                    a.actions[2 * i + seat] = act;
+                    if (a.logits) {
+                        float* lg = a.logits + (SEATS == 1 ? 3 * i : 6 * i + 3 * seat);
+                        lg[0] = l[0]; lg[1] = l[1]; lg[2] = l[2];
+                    }
                 }
             }
             __syncthreads();   // thread 0 is done with this slot's bias before the next slot's weights arrive
@@ -287,7 +342,7 @@ __global__ void pong_opp_draw_kernel(const OppArgs a) {
 using namespace crl::opp;
 
 struct crl_pong_opp {
-    int n = 0, device = 0, grid = 0;
+    int n = 0, device = 0, grid = 0, grid_league = 0;
     uint64_t seed = 0;
     int64_t first_env = 0;
     uint64_t steps = 0;
@@ -304,6 +359,12 @@ struct crl_pong_opp {
     float* ret = nullptr;
     uint32_t* episodes = nullptr;
     unsigned long long* stats = nullptr;
+    // league mode
+    bool league = false;
+    int num_pairs = 0;
+    uint8_t pairs[CRL_PONG_OPP_MAX_PAIRS][2] = {};
+    uint8_t* stack0 = nullptr;                 // allocated by the first crl_pong_opp_set_pairs
+    unsigned long long* pair_stats = nullptr;  // [CRL_PONG_OPP_MAX_PAIRS][4], allocated with stack0
 };
 
 static OppArgs opp_args(const crl_pong_opp* h) {
@@ -336,15 +397,19 @@ int crl_pong_opp_create(int32_t num_envs, int32_t device, uint64_t seed, int64_t
     crl_pong_opp* h = new crl_pong_opp();
     h->n = num_envs; h->device = device; h->seed = seed; h->first_env = first_env;
     const size_t n = (size_t)num_envs;
-    int sms = 0, per_sm = 0;
+    int sms = 0, per_sm = 0, per_sm_league = 0;
     cudaError_t err = cudaSuccess;
     auto alloc = [&](auto** p, size_t count) { if (err == cudaSuccess) err = h->allocs.alloc(p, count); };
     alloc(&h->nets, (size_t)NET_DEV * CRL_PONG_OPP_SLOTS);
     alloc(&h->ids, n); alloc(&h->stack, (size_t)STACK * FRAME * n); alloc(&h->ret, n); alloc(&h->episodes, n);
     alloc(&h->stats, 4 * CRL_PONG_OPP_MAX_POOL);
-    if (err == cudaSuccess) err = cudaFuncSetAttribute(pong_opp_act_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(pong_opp_act_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
+    if (err == cudaSuccess)
+        err = cudaFuncSetAttribute(pong_opp_act_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes<2>());
     if (err == cudaSuccess) err = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-    if (err == cudaSuccess) err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pong_opp_act_kernel, THREADS, SMEM_BYTES);
+    if (err == cudaSuccess) err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pong_opp_act_kernel<1>, THREADS, SMEM_BYTES);
+    if (err == cudaSuccess)
+        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_league, pong_opp_act_kernel<2>, THREADS, smem_bytes<2>());
     if (err == cudaSuccess) err = cudaDeviceSynchronize();
     if (err != cudaSuccess) {
         crl_pong_opp_destroy(h);
@@ -352,6 +417,7 @@ int crl_pong_opp_create(int32_t num_envs, int32_t device, uint64_t seed, int64_t
     }
     // one resident wave: every CTA owns an equal contiguous range of envs
     h->grid = (int)std::min<int64_t>((int64_t)std::max(per_sm, 1) * sms, num_envs);
+    h->grid_league = (int)std::min<int64_t>((int64_t)std::max(per_sm_league, 1) * sms, num_envs);
     *out = h;
     return CRL_OK;
 }
@@ -414,6 +480,12 @@ int crl_pong_opp_set_pool(crl_pong_opp* h, const int32_t* kinds_host, const doub
     h->pool_size = pool_size;
     h->assigned = false;
     CUDA_TRY(cudaMemsetAsync(h->stats, 0, sizeof(unsigned long long) * 4 * CRL_PONG_OPP_MAX_POOL, (cudaStream_t)stream));
+    if (h->league) {   // leaving league mode: the per-env opponents start as on a fresh handle (the act count runs on)
+        h->league = false;
+        CUDA_TRY(cudaMemsetAsync(h->ret, 0, sizeof(float) * h->n, (cudaStream_t)stream));
+        CUDA_TRY(cudaMemsetAsync(h->stack, 0, (size_t)STACK * FRAME * h->n, (cudaStream_t)stream));
+        h->phase = 0;
+    }
     return CRL_OK;
 }
 
@@ -438,6 +510,7 @@ int crl_pong_opp_restart(crl_pong_opp* h, int32_t clear_stacks, void* stream) {
     CUDA_TRY(cudaMemsetAsync(h->ret, 0, sizeof(float) * h->n, (cudaStream_t)stream));
     if (clear_stacks) {
         CUDA_TRY(cudaMemsetAsync(h->stack, 0, (size_t)STACK * FRAME * h->n, (cudaStream_t)stream));
+        if (h->stack0) CUDA_TRY(cudaMemsetAsync(h->stack0, 0, (size_t)STACK * FRAME * h->n, (cudaStream_t)stream));
         h->phase = 0;
     }
     return CRL_OK;
@@ -446,6 +519,7 @@ int crl_pong_opp_restart(crl_pong_opp* h, int32_t clear_stacks, void* stream) {
 int crl_pong_opp_act(crl_pong_opp* h, const uint8_t* obs1_dev, const float* rew_dev, const uint8_t* done_dev, int32_t resample,
                      int32_t* actions_dev, float* logits_dev, void* stream) {
     CHECK_HANDLE(h, h->device);
+    if (h->league) return crl_set_error(CRL_E_STATE, "league mode: use crl_pong_opp_act_pairs (crl_pong_opp_set_pool leaves it)");
     if (!h->assigned) return crl_set_error(CRL_E_STATE, "crl_pong_opp_assign after every crl_pong_opp_set_pool");
     if (!obs1_dev || !actions_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
     if ((rew_dev == nullptr) != (done_dev == nullptr)) return crl_set_error(CRL_E_INVALID, "rew_dev and done_dev go together");
@@ -453,10 +527,72 @@ int crl_pong_opp_act(crl_pong_opp* h, const uint8_t* obs1_dev, const float* rew_
     OppArgs a = opp_args(h);
     a.resample = resample ? 1 : 0;
     a.obs1 = obs1_dev; a.rew = rew_dev; a.done = done_dev; a.actions = actions_dev; a.logits = logits_dev;
-    LAUNCH((pong_opp_act_kernel<<<h->grid, THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(a), cudaGetLastError()), 1);
+    LAUNCH((pong_opp_act_kernel<1><<<h->grid, THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(a), cudaGetLastError()), 1);
     h->phase = (h->phase + 1) & 3;
     h->steps += 1;
     return CRL_OK;
+}
+
+int crl_pong_opp_set_pairs(crl_pong_opp* h, const int32_t* pairs_host, int32_t num_pairs, void* stream) {
+    CHECK_HANDLE(h, h->device);
+    if (h->pool_size == 0) return crl_set_error(CRL_E_STATE, "crl_pong_opp_set_pool first");
+    if (!pairs_host || num_pairs < 1 || num_pairs > CRL_PONG_OPP_MAX_PAIRS)
+        return crl_set_error(CRL_E_INVALID, "a league has 1 to %d pairings", CRL_PONG_OPP_MAX_PAIRS);
+    for (int p = 0; p < num_pairs; ++p)
+        for (int seat = 0; seat < 2; ++seat)
+            if (pairs_host[2 * p + seat] < 0 || pairs_host[2 * p + seat] >= h->pool_size)
+                return crl_set_error(CRL_E_INVALID, "pairing %d, seat %d: pool index %d is not in [0, %d)", p, seat,
+                                     pairs_host[2 * p + seat], h->pool_size);
+    if (!h->stack0) {
+        cudaError_t err = h->allocs.alloc(&h->pair_stats, 4 * CRL_PONG_OPP_MAX_PAIRS);
+        if (err == cudaSuccess) err = h->allocs.alloc(&h->stack0, (size_t)STACK * FRAME * h->n);
+        if (err != cudaSuccess) {   // both or neither: a failed call leaves the handle as it was
+            h->allocs.free(h->pair_stats);
+            h->pair_stats = nullptr;
+            h->stack0 = nullptr;
+            return crl_set_error(CRL_E_CUDA, "crl_pong_opp_set_pairs: %s", cudaGetErrorString(err));
+        }
+    }
+    const cudaStream_t s = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemsetAsync(h->pair_stats, 0, sizeof(unsigned long long) * 4 * CRL_PONG_OPP_MAX_PAIRS, s));
+    CUDA_TRY(cudaMemsetAsync(h->ret, 0, sizeof(float) * h->n, s));
+    CUDA_TRY(cudaMemsetAsync(h->stack, 0, (size_t)STACK * FRAME * h->n, s));
+    CUDA_TRY(cudaMemsetAsync(h->stack0, 0, (size_t)STACK * FRAME * h->n, s));
+    for (int p = 0; p < CRL_PONG_OPP_MAX_PAIRS; ++p)
+        for (int seat = 0; seat < 2; ++seat) h->pairs[p][seat] = p < num_pairs ? (uint8_t)pairs_host[2 * p + seat] : 0;
+    h->num_pairs = num_pairs;
+    h->phase = 0;
+    h->league = true;
+    return CRL_OK;
+}
+
+int crl_pong_opp_act_pairs(crl_pong_opp* h, const uint8_t* obs0_dev, const uint8_t* obs1_dev, const float* rew_dev,
+                           const uint8_t* done_dev, int32_t* actions_dev, float* logits_dev, void* stream) {
+    CHECK_HANDLE(h, h->device);
+    if (!h->league) return crl_set_error(CRL_E_STATE, "crl_pong_opp_set_pairs first (league mode)");
+    if (!obs0_dev || !obs1_dev || !actions_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
+    if ((rew_dev == nullptr) != (done_dev == nullptr)) return crl_set_error(CRL_E_INVALID, "rew_dev and done_dev go together");
+    if (((uintptr_t)obs0_dev & 3) != 0 || ((uintptr_t)obs1_dev & 3) != 0)
+        return crl_set_error(CRL_E_INVALID, "obs0_dev and obs1_dev must be 4-byte aligned");
+    OppArgs a = opp_args(h);
+    a.stats = h->pair_stats;
+    a.num_pairs = h->num_pairs;
+    memcpy(a.pairs, h->pairs, sizeof a.pairs);
+    a.obs0 = obs0_dev; a.obs1 = obs1_dev; a.stack0 = h->stack0;
+    a.rew = rew_dev; a.done = done_dev; a.actions = actions_dev; a.logits = logits_dev;
+    LAUNCH((pong_opp_act_kernel<2><<<h->grid_league, THREADS, smem_bytes<2>(), (cudaStream_t)stream>>>(a), cudaGetLastError()), 1);
+    h->phase = (h->phase + 1) & 3;
+    h->steps += 1;
+    return CRL_OK;
+}
+
+int crl_pong_opp_get_pair_stats(crl_pong_opp* h, uint64_t* stats_host, int32_t num_pairs, void* stream) {
+    CHECK_HANDLE(h, h->device);
+    if (!stats_host) return crl_set_error(CRL_E_INVALID, "null buffer");
+    if (num_pairs < 1 || num_pairs > CRL_PONG_OPP_MAX_PAIRS)
+        return crl_set_error(CRL_E_INVALID, "num_pairs must be in [1, %d]", CRL_PONG_OPP_MAX_PAIRS);
+    if (!h->pair_stats) return crl_set_error(CRL_E_STATE, "crl_pong_opp_set_pairs first (league mode)");
+    return crl_read_counters(h->pair_stats, stats_host, 4 * num_pairs, (cudaStream_t)stream);
 }
 
 int crl_pong_opp_get_ids(crl_pong_opp* h, int32_t* ids_dev, void* stream) {

@@ -1,10 +1,12 @@
-"""evaluate_two_policies_in_batch on the device (competitive_rl/pong/evaluate.py:53-88; SURVEY section 8 row f3).
+"""evaluate_two_policies_in_batch on the device (competitive_rl/pong/evaluate.py:53-88; SURVEY section 8 row f3), and
+evaluate_pool_in_batch, which plays every pairing of an opponent pool in one batch.
 
 Same contract as the reference: two action functions play each other on a cPongDouble vec-env until `num_episodes`
 episodes have finished; returns ([win, draw, lose, cumulative reward] of agent 0, the same for agent 1).  The per-env
 bookkeeping (episode returns, win / draw / lose classification on done, zeroing finished envs) is tensor arithmetic on
 the device instead of a Python loop over envs; the only host traffic per step is the finished-episode count that the
 stopping rule needs."""
+import numpy as np
 import torch
 
 
@@ -32,3 +34,95 @@ def evaluate_two_policies_in_batch(compute_action0, compute_action1, envs, num_e
             break
     w, d, l, s0, s1 = [float(x) for x in tally.tolist()]
     return [int(w), int(d), int(l), s0], [int(l), int(d), int(w), s1]
+
+
+def evaluate_pool_in_batch(pool, envs, episodes_per_pair, pairs=None, networks=None, seed=0, resource_dir=None,
+                           check_every=64, max_steps=None):
+    """Win / draw / loss table of pool entries playing each other, every pairing in one batch.
+
+    Both agents of every env are played by the league mode of the per-env opponent kernel (csrc/pong_opponent.cu,
+    include/crl_b200.h crl_pong_opp_set_pairs): one launch per step evaluates both seats of every env, and env g plays
+    pairing g mod P for the whole run.
+
+    pool: up to 16 distinct names, resolved as TournamentEnvWrapper.set_opponents resolves them: "RULE_BASED", "RANDOM"
+        and up to 8 LightActorCritic networks (WEAK / MEDIUM from their checkpoints, or names given in `networks`).
+    envs: a 42x42 cPongDouble vec-env with frame_stack None and uint8 observations, at least one env per pairing.
+        It is reset first.
+    episodes_per_pair: the run stops once every pairing has at least this many finished episodes (checked every
+        `check_every` steps, one host synchronisation each) or after `max_steps` steps.
+    pairs: (seat 0, seat 1) pool indices or names; None = all M^2 ordered pairings, self-play included.  At most 256.
+    networks: {name: state dict | module | checkpoint dict | path} of extra LightActorCritic networks.
+    seed: keys RANDOM's actions.
+
+    Returns {"pool", "pairs", "episodes", "wins", "draws", "losses", "steps"}: the tallies are int64 (M, M) arrays,
+    row = seat 0's entry, column = seat 1's, counted from seat 0's side (> 0, == 0, < 0 summed clipped reward, as in
+    evaluate_two_policies_in_batch); repeated pairings add up, pairings not played are 0."""
+    from . import _native
+    from .builtin_policies import pack_light_actor_critic, resolve_pool
+    if envs.dim != 42 or envs.c != 1 or envs.f32 or envs.ring or getattr(envs, "n_agents", 2) != 2:
+        raise ValueError("league evaluation needs a cPongDouble env with resized_dim=42, frame_stack=None and uint8 "
+                         "observations")
+    ext = _native.ext()
+    added = {}
+    for name, state in (networks or {}).items():
+        if name in ("RULE_BASED", "RANDOM"):
+            raise ValueError("%s is not a network" % name)
+        if isinstance(state, str):
+            state = torch.load(state, map_location="cpu", weights_only=True)
+        added[name] = pack_light_actor_critic(state)
+    pool, kinds, images = resolve_pool(pool, added, resource_dir)
+    m = len(pool)
+    if pairs is None:
+        pairs = [(a, b) for a in range(m) for b in range(m)]
+    idx = []
+    for pr in pairs:
+        pr = list(pr)
+        if len(pr) != 2:
+            raise ValueError("a pairing is (seat 0, seat 1)")
+        for x in pr:
+            if isinstance(x, str) and x not in pool:
+                raise ValueError("pairing %r: %r is not in the pool" % (tuple(pr), x))
+        k = [pool.index(x) if isinstance(x, str) else int(x) for x in pr]
+        if not all(0 <= v < m for v in k):
+            raise ValueError("pairing %r: pool indices must be in [0, %d)" % (tuple(pr), m))
+        idx.append(k)
+    p = len(idx)
+    if not 1 <= p <= ext.OPP_MAX_PAIRS:
+        raise ValueError("a league has 1 to %d pairings (got %d)" % (ext.OPP_MAX_PAIRS, p))
+    n = envs.num_envs
+    if n < p:
+        raise ValueError("%d pairings need at least as many envs (got %d)" % (p, n))
+    if episodes_per_pair < 1 or check_every < 1 or (max_steps is not None and max_steps < 1):
+        raise ValueError("episodes_per_pair, check_every and max_steps must be positive")
+
+    dev = envs.device
+    opp = ext.PongOpponents(n, int(dev.index), int(seed) & (2 ** 64 - 1), int(envs.first_env))
+    try:
+        for slot, image in enumerate(images):
+            opp.load_net(slot, image)
+        opp.set_pool(torch.tensor(kinds, dtype=torch.int32), None)
+        opp.set_pairs(torch.tensor(idx, dtype=torch.int32))
+        both = torch.zeros((n, 2), dtype=torch.int32, device=dev)
+        envs.reset()
+        rew = done = None
+        steps = 0
+        while True:
+            # credits the episodes that the previous step ended, then acts for both seats
+            opp.act_pairs(envs._obs[0], envs._obs[1], rew, done, both, None)
+            if steps > 0 and (steps % check_every == 0 or steps == max_steps):
+                st = np.array(opp.pair_stats(p), dtype=np.int64).reshape(p, 4)
+                if st[:, 0].min() >= episodes_per_pair or steps == max_steps:
+                    break
+            envs.step(both)
+            rew, done = envs._rew, envs._done
+            steps += 1
+    finally:
+        torch.cuda.synchronize(dev)
+        opp.close()
+    out = {"pool": pool, "pairs": [tuple(k) for k in idx], "steps": steps}
+    ab = np.array(idx, dtype=np.int64)
+    for col, key in enumerate(("episodes", "wins", "draws", "losses")):
+        t = np.zeros((m, m), np.int64)
+        np.add.at(t, (ab[:, 0], ab[:, 1]), st[:, col])
+        out[key] = t
+    return out

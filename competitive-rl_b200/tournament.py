@@ -12,8 +12,8 @@ import numpy as np
 import torch
 
 from . import _native
-from .builtin_policies import (BUILTIN_AGENT_NAMES, find_checkpoint, get_builtin_agent_names, get_compute_action_function,
-                               is_light_agent, pack_light_actor_critic)
+from .builtin_policies import (get_builtin_agent_names, get_compute_action_function, is_light_agent,
+                               pack_light_actor_critic, resolve_pool)
 
 
 class TournamentEnvWrapper(object):
@@ -68,28 +68,13 @@ class TournamentEnvWrapper(object):
         if self.per_env and name in self._pool:
             self._load_pool_nets()
 
-    def _net_image(self, name):
-        if name in self._added:
-            return self._added[name]
-        if name in BUILTIN_AGENT_NAMES and not is_light_agent(name):
-            raise ValueError("%s is an ActorCritic agent: per-env pools take RULE_BASED, RANDOM and LightActorCritic "
-                             "networks (WEAK, MEDIUM or add_opponent) only" % name)
-        path = find_checkpoint(name, self._resource_dir)
-        if path is None:
-            raise ValueError("unknown opponent %r: not RULE_BASED / RANDOM, not added with add_opponent, and no "
-                             "checkpoint found" % (name,))
-        return pack_light_actor_critic(torch.load(path, map_location="cpu", weights_only=True))
-
     def _default_pool(self):
         pool = ["RULE_BASED", "RANDOM"] + [n for n in self.agent_names if is_light_agent(n) and n not in self._added]
         return pool + list(self._added)
 
     def _load_pool_nets(self):
-        slot = 0
-        for name in self._pool:
-            if name not in ("RULE_BASED", "RANDOM"):
-                self._opp.load_net(slot, self._net_image(name))
-                slot += 1
+        for slot, image in enumerate(resolve_pool(self._pool, self._added, self._resource_dir)[2]):
+            self._opp.load_net(slot, image)
 
     def set_opponents(self, assignment=None, pool=None, weights=None, resample_on_done=False, seed=None):
         """Enter (or re-configure) per-env mode: every env plays its own opponent, chosen from `pool`.
@@ -114,29 +99,15 @@ class TournamentEnvWrapper(object):
             raise ValueError("per-env opponents need resized_dim=42, frame_stack=None and uint8 observations")
         if pool is None:
             pool = self._pool if self.per_env else self._default_pool()
-        pool = [str(p) for p in pool]
-        if not 1 <= len(pool) <= _native.ext().OPP_MAX_POOL or len(set(pool)) != len(pool):
-            raise ValueError("a pool is 1 to %d distinct names" % _native.ext().OPP_MAX_POOL)
-        nets = [p for p in pool if p not in ("RULE_BASED", "RANDOM")]
-        if len(nets) > _native.ext().OPP_SLOTS:
-            raise ValueError("a pool holds at most %d networks" % _native.ext().OPP_SLOTS)
-        images = [self._net_image(p) for p in nets]            # refuses unknown and ActorCritic names before any change
+        pool, kinds, images = resolve_pool(pool, self._added, self._resource_dir)   # refuses bad pools before any change
         if seed is not None:
             self._seed = int(seed) & (2 ** 64 - 1)
         ext = _native.ext()
         if self._opp is None:
             self._opp = ext.PongOpponents(self.num_envs, int(self.env.device.index), self._seed, int(self.env.first_env))
         self._opp.seed(self._seed)
-        kinds, slot = [], 0
-        for p in pool:
-            if p == "RULE_BASED":
-                kinds.append(ext.OPP_RULE_BASED)
-            elif p == "RANDOM":
-                kinds.append(ext.OPP_RANDOM)
-            else:
-                self._opp.load_net(slot, images[slot])
-                kinds.append(slot)
-                slot += 1
+        for slot, image in enumerate(images):
+            self._opp.load_net(slot, image)
         w = None
         if weights is not None:
             w = torch.as_tensor(np.asarray(weights, np.float64).reshape(-1))

@@ -233,11 +233,35 @@ int crl_obs_free(void* ptr);
  *   Episodes    act receives the previous step's reward and done.  Agent 0's clipped rewards are summed per env; an env
  *               that finished credits the episode to the pool entry it played (agent 0 wins when the sum is > 0,
  *               draws at 0, loses below: pong/evaluate.py:53-88) and, with resample != 0, draws a new id.
+ *
+ * League mode (crl_pong_opp_set_pairs, crl_pong_opp_act_pairs, crl_pong_opp_get_pair_stats): both agents of every env
+ * are played from the pool, so one launch per step evaluates every pairing of the pool in one batch.
+ *   Pool        as above (crl_pong_opp_load_net, crl_pong_opp_set_pool); the pool's weights are not used.
+ *   Pairings    pairs[P][2] = (pool index of seat 0, pool index of seat 1), 1 <= P <= CRL_PONG_OPP_MAX_PAIRS; repeated
+ *               pairings and self-pairings (a, a) are allowed.  The env of global index g = first_env + i plays pairing
+ *               g mod P (the non-negative remainder) for the whole run: nothing is redrawn, so the assignment does not
+ *               depend on the sharding.
+ *   Stacks      two uint8 [4][42][42] stacks per env, oldest -> newest.  Seat 0 is fed agent 0's observation, seat 1
+ *               agent 1's (already mirrored by the env, so a network plays either seat as it was trained).  Both are
+ *               zeroed by crl_pong_opp_set_pairs; done does not clear them, restart(clear_stacks != 0) does.
+ *   Actions     every act_pairs writes both columns of the int32 [num_envs][2] step buffer: RULE_BASED 999 (the step
+ *               accepts it for either bat); RANDOM a Philox-uniform draw from {0, 1, 2} keyed by (seed, global env
+ *               index, act count), seat 1 on the stream of crl_pong_opp_act's RANDOM and seat 0 on a stream of its own;
+ *               a network the argmax (ties: lowest index) of its fp32 actor logits over its seat's stack / 255, computed
+ *               exactly as crl_pong_opp_act computes them.
+ *   Episodes    agent 0's (seat 0's) clipped rewards are summed per env; an env that finished credits the episode to its
+ *               pairing: [episodes, wins, draws, losses] of seat 0 (> 0, == 0, < 0).  As with crl_pong_opp_act, an
+ *               episode is credited by the act_pairs call that follows the step that ended it.
+ *   Modes       crl_pong_opp_act returns CRL_E_STATE in league mode and crl_pong_opp_act_pairs outside it.
+ *               crl_pong_opp_set_pool leaves league mode: it zeroes the per-env reward sums and agent 1's stacks (the act
+ *               count runs on), and crl_pong_opp_assign must follow it as always.  League mode does not change the
+ *               opponent ids, the episode counts of the draws or the per-entry statistics of crl_pong_opp_get_stats.
  * ====================================================================================== */
 #define CRL_PONG_OPP_MAX_POOL 16
 #define CRL_PONG_OPP_SLOTS 8
 #define CRL_PONG_OPP_RULE_BASED (-1)   /* pool entry kinds; 0 .. CRL_PONG_OPP_SLOTS-1 = network slot */
 #define CRL_PONG_OPP_RANDOM (-2)
+#define CRL_PONG_OPP_MAX_PAIRS 256    /* pairings of league mode */
 /* LightActorCritic parameters in state-dict order, each row-major: conv1.weight [16][4][4][4], conv1.bias [16],
  * conv2.weight [16][16][2][2], conv2.bias [16], critic_linear.weight [1][1600], critic_linear.bias [1],
  * actor_linear.weight [3][1600], actor_linear.bias [3] (the critic is carried but not evaluated) */
@@ -274,6 +298,22 @@ int crl_pong_opp_get_ids(crl_pong_opp* h, int32_t* ids_dev, void* stream);
 /* stats_host uint64 [16][4]: per pool entry, episodes finished against it, agent 0's wins, draws, losses (since the
  * last crl_pong_opp_set_pool).  Synchronises the stream. */
 int crl_pong_opp_get_stats(crl_pong_opp* h, uint64_t* stats_host, void* stream);
+/* Enters (or re-enters) league mode: pairs_host int32 [num_pairs][2] pool indices (seat 0, seat 1), every one validated
+ * against the current pool (CRL_E_STATE without a pool).  Zeroes the pairing statistics, the per-env reward sums and
+ * both stacks of every env, and restarts the ring.  Seat 0's stacks (num_envs * 7056 bytes) are allocated by the first
+ * call, so a handle that never enters league mode does not pay for them. */
+int crl_pong_opp_set_pairs(crl_pong_opp* h, const int32_t* pairs_host, int32_t num_pairs, void* stream);
+/* One league step, before crl_pong_step:
+ *   obs0_dev, obs1_dev  uint8 [num_envs][42][42] agent 0's and agent 1's observations of the previous step, 4-byte aligned
+ *   rew_dev, done_dev   as crl_pong_opp_act (both NULL for the first act after a reset)
+ *   actions_dev         int32 [num_envs][2]: both columns receive the seats' actions
+ *   logits_dev          float32 [num_envs][2][3] or NULL: each network seat's actor logits (0 for the other kinds) */
+int crl_pong_opp_act_pairs(crl_pong_opp* h, const uint8_t* obs0_dev, const uint8_t* obs1_dev, const float* rew_dev,
+                           const uint8_t* done_dev, int32_t* actions_dev, float* logits_dev, void* stream);
+/* stats_host uint64 [num_pairs][4]: per pairing, episodes finished, seat 0's wins, draws, losses (since the last
+ * crl_pong_opp_set_pairs).  1 <= num_pairs <= CRL_PONG_OPP_MAX_PAIRS; rows past the league's P read 0.  Synchronises
+ * the stream. */
+int crl_pong_opp_get_pair_stats(crl_pong_opp* h, uint64_t* stats_host, int32_t num_pairs, void* stream);
 
 /* ======================================================================================
  * cCarRacing-v0 / cCarRacingDouble-v0
