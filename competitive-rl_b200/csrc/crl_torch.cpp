@@ -331,6 +331,24 @@ struct PongOpponents {
                                         dev_ptr<int32_t>(actions, at::kInt, device, 2 * n(), "actions"),
                                         opt_dev_ptr<float>(logits, at::kFloat, device, 6 * n(), "logits"), stream_of(device)));
     }
+    // learner mode.  params: as load_net, the whole image (the critic is evaluated)
+    void load_learner(const at::Tensor& params) {
+        check_rc(crl_pong_opp_load_learner(handle(), host_ptr<float>(params, at::kFloat, "params"), (size_t)params.numel(),
+                                           stream_of(device)));
+    }
+    void act_learner(const at::Tensor& obs0, const at::Tensor& obs1, const c10::optional<at::Tensor>& rew,
+                     const c10::optional<at::Tensor>& done, bool resample, bool sample, const at::Tensor& actions,
+                     const at::Tensor& logp_value, const c10::optional<at::Tensor>& logits, const at::Tensor& stack_out) {
+        check_rc(crl_pong_opp_act_learner(handle(), dev_ptr<uint8_t>(obs0, at::kByte, device, n() * 42 * 42, "obs0"),
+                                          dev_ptr<uint8_t>(obs1, at::kByte, device, n() * 42 * 42, "obs1"),
+                                          opt_dev_ptr<float>(rew, at::kFloat, device, 2 * n(), "rew"),
+                                          opt_dev_ptr<uint8_t>(done, at::kBool, device, n(), "done"), resample ? 1 : 0,
+                                          sample ? 1 : 0, dev_ptr<int32_t>(actions, at::kInt, device, 2 * n(), "actions"),
+                                          dev_ptr<float>(logp_value, at::kFloat, device, 2 * n(), "logp_value"),
+                                          opt_dev_ptr<float>(logits, at::kFloat, device, 3 * n(), "logits"),
+                                          dev_ptr<uint8_t>(stack_out, at::kByte, device, n() * 4 * 42 * 42, "stack_out"),
+                                          stream_of(device)));
+    }
     // [P * 4]: episodes, wins, draws, losses of seat 0 per pairing
     std::vector<uint64_t> pair_stats(int64_t num_pairs) {
         TORCH_CHECK(num_pairs >= 1 && num_pairs <= CRL_PONG_OPP_MAX_PAIRS, "num_pairs must be in [1, ", CRL_PONG_OPP_MAX_PAIRS, "]");
@@ -426,5 +444,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
         .def("stats", &PongOpponents::stats)
         .def("set_pairs", &PongOpponents::set_pairs)
         .def("act_pairs", &PongOpponents::act_pairs)
-        .def("pair_stats", &PongOpponents::pair_stats);
+        .def("pair_stats", &PongOpponents::pair_stats)
+        .def("load_learner", &PongOpponents::load_learner)
+        .def("act_learner", &PongOpponents::act_learner);
 }

@@ -17,6 +17,12 @@
 // plays pairing g mod P, both seats act from their own stack (seat 0 from agent 0's frames, seat 1 from agent 1's),
 // and a finished episode is credited to the pairing.  The per-env thread files one work item per network seat, so a
 // slot's weights are still staged once per 64-env chunk whichever seats use it.
+//
+// Learner mode (crl_pong_opp_load_learner / crl_pong_opp_act_learner) is the one-seat kernel with LEARNER set: seat 1
+// is played exactly as above, and seat 0 is a LightActorCritic learner with its own weights (actor and critic) staged
+// like a ninth slot, run for every env of the chunk after the pool's slots.  It acts on a FrameStackTensor ring of agent
+// 0's frames (zeroed on done), samples its action from the softmax of its logits (or takes the argmax) and writes what
+// a PPO rollout stores: the action, its log-probability, the value and the stack it acted on.
 #include <string.h>
 
 #include <cmath>
@@ -58,13 +64,22 @@ static_assert(NET_DEV % 4 == 0, "slot image is copied as float4");
 constexpr int SD_W1 = 0, SD_B1 = SD_W1 + C1 * STACK * 16, SD_W2 = SD_B1 + C1, SD_B2 = SD_W2 + C2 * C1 * 4,
               SD_WC = SD_B2 + C2, SD_BC = SD_WC + FEATS, SD_WA = SD_BC + 1, SD_BA = SD_WA + 3 * FEATS, SD_END = SD_BA + 3;
 static_assert(SD_END == CRL_PONG_OPP_NET_FLOATS, "flat layout of the header");
+// the learner's image: a slot image followed by critic_linear
+//   WC[1600]    feature (c*100 + y*10 + x)
+//   BC[4]       1 used
+constexpr int OFF_WC = NET_DEV, OFF_BC = OFF_WC + FEATS, NET_LRN = OFF_BC + 4;
+static_assert(NET_LRN % 4 == 0, "learner image is copied as float4");
 
-// shared memory of the act kernel (floats unless noted); h2 reuses the input stack, which conv1 is done with
-constexpr int SM_W = 0, SM_X = SM_W + NET_DEV, SM_H1 = SM_X + STACK * FRAME, SM_LUT = SM_H1 + C1 * H1 * H1,
-              SM_RED = SM_LUT + 256, SM_FLOATS = SM_RED + 8 * 3;
+// shared memory of the act kernel (floats unless noted); h2 reuses the input stack, which conv1 is done with.  The
+// learner kernel stages the larger learner image and reduces 4 sums (3 logits, the value) per warp.
+template <bool LEARNER>
+struct Smem {
+    static constexpr int W = 0, X = W + (LEARNER ? NET_LRN : NET_DEV), HID = X + STACK * FRAME, LUT = HID + C1 * H1 * H1,
+                         RS = LEARNER ? 4 : 3, RED = LUT + 256, FLOATS = RED + 8 * RS;
+};
 // + the work list uint8 [slot][SEATS * SUB] and its counts int [16]
-template <int SEATS>
-constexpr size_t smem_bytes() { return SM_FLOATS * sizeof(float) + CRL_PONG_OPP_SLOTS * SUB * SEATS + 16 * sizeof(int); }
+template <int SEATS, bool LEARNER = false>
+constexpr size_t smem_bytes() { return Smem<LEARNER>::FLOATS * sizeof(float) + CRL_PONG_OPP_SLOTS * SUB * SEATS + 16 * sizeof(int); }
 constexpr size_t SMEM_BYTES = smem_bytes<1>();
 static_assert(SUB <= 64, "a league work item is (env in chunk) | seat << 6");
 
@@ -96,10 +111,16 @@ struct OppArgs {
     uint8_t pairs[CRL_PONG_OPP_MAX_PAIRS][2];   // pool index of seat 0, seat 1
     const uint8_t* obs0;      // [n][1764] agent 0's observation of the previous step
     uint8_t* stack0;          // [n][4][1764] seat 0's stacks; `stack` holds seat 1's
+    // learner mode only (SEATS == 1, LEARNER): obs0 and stack0 above are agent 0's frames and the learner's ring
+    int sample;               // != 0: sample the action from the softmax, else the argmax
+    const float* learner;     // [NET_LRN]
+    float* logp_value;        // [n][2]
+    float* learner_logits;    // [n][3] or nullptr
+    uint8_t* stack_out;       // [n][4][1764] the stack the learner acted on, oldest -> newest
 };
 
 // Philox streams: (global env, tag) x counter, keyed by the seed.  tag 1 = RANDOM's actions (seat 1), tag 2 = opponent
-// draws, tag 3 = RANDOM's actions in seat 0 (league mode).
+// draws, tag 3 = RANDOM's actions in seat 0 (league mode), tag 4 = the learner's sampled actions (learner mode).
 __device__ __forceinline__ uint32_t opp_rand(uint64_t seed, int64_t g, uint32_t tag, uint64_t ctr) {
     uint32_t r[4];
     philox4x32_10((uint32_t)g, (uint32_t)((uint64_t)g >> 32) ^ (tag << 24), (uint32_t)ctr, (uint32_t)(ctr >> 32),
@@ -114,17 +135,47 @@ __device__ __forceinline__ int opp_draw(const OppArgs& a, int64_t g, uint32_t ep
     return k;
 }
 
-// SEATS == 1: column 1 of the step buffer (the per-env opponents); SEATS == 2: both columns (league mode)
-template <int SEATS>
+// The learner's outputs from its fp32 logits l and value v (thread 0): the action (a draw u = r32 * 2^-32 from the tag 4
+// stream, the first k with u < c_k of the cumulative softmax, or the argmax), log pi(action) and the value.
+__device__ __forceinline__ void learner_out(const OppArgs& a, int i, const float (&l)[3], float v) {
+    const float mx = fmaxf(fmaxf(l[0], l[1]), l[2]);
+    const float e0 = expf(l[0] - mx), e1 = expf(l[1] - mx), e2 = expf(l[2] - mx);
+    const float s = (e0 + e1) + e2;
+    int act = 0;
+    if (a.sample) {
+        const float c0 = e0 / s, c1 = c0 + e1 / s;   // action 2 takes the rest, whatever c_2 rounds to
+        const double u = (double)opp_rand(a.seed, a.first_env + i, 4u, a.step) * 0x1p-32;   // exact, and so is the compare
+        act = u < (double)c0 ? 0 : u < (double)c1 ? 1 : 2;
+    } else {
+        float best = l[0];                     // argmax, ties to the lowest index
+        if (l[1] > best) { act = 1; best = l[1]; }
+        if (l[2] > best) act = 2;
+    }
+    const float la = act == 0 ? l[0] : act == 1 ? l[1] : l[2];
+    a.logp_value[2 * i] = la - (mx + logf(s));   // log softmax: l_a - logsumexp(l)
+    a.logp_value[2 * i + 1] = v;
+    a.actions[2 * i] = act;
+    if (a.learner_logits) {
+        float* lg = a.learner_logits + 3 * i;
+        lg[0] = l[0]; lg[1] = l[1]; lg[2] = l[2];
+    }
+}
+
+// SEATS == 1: column 1 of the step buffer (the per-env opponents); SEATS == 2: both columns (league mode).
+// LEARNER (SEATS == 1 only): column 0 too, from the learner's network (learner mode).
+template <int SEATS, bool LEARNER>
 __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs a) {
+    static_assert(!LEARNER || SEATS == 1, "the learner plays seat 0 of the one-seat kernel");
+    using L = Smem<LEARNER>;
+    constexpr int NS = CRL_PONG_OPP_SLOTS + (LEARNER ? 1 : 0);   // the learner is slot CRL_PONG_OPP_SLOTS
     extern __shared__ __align__(16) float sm[];
-    float* const w = sm + SM_W;
-    float* const xs = sm + SM_X;
-    float* const h1 = sm + SM_H1;
+    float* const w = sm + L::W;
+    float* const xs = sm + L::X;
+    float* const h1 = sm + L::HID;
     float* const h2 = xs;
-    float* const lut = sm + SM_LUT;
-    float* const red = sm + SM_RED;
-    uint8_t* const list = (uint8_t*)(sm + SM_FLOATS);                     // [slot][SEATS * SUB]
+    float* const lut = sm + L::LUT;
+    float* const red = sm + L::RED;
+    uint8_t* const list = (uint8_t*)(sm + L::FLOATS);                     // [slot][SEATS * SUB]
     int* const cnt = (int*)(list + CRL_PONG_OPP_SLOTS * SUB * SEATS);   // [slot]
     const int tid = threadIdx.x;
 
@@ -196,34 +247,45 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
                 }
             }
         }
-        // ---- the newest frame into ring slot `phase` of every env of the range (league: of both seats' stacks)
+        // ---- the newest frame into ring slot `phase` of every env of the range (league: of both seats' stacks;
+        //      learner: of both, and an env whose previous step ended has its learner ring zeroed first)
 #pragma unroll
-        for (int seat = 2 - SEATS; seat < 2; ++seat) {
+        for (int seat = SEATS == 2 || LEARNER ? 0 : 1; seat < 2; ++seat) {
             const uint32_t* src = (const uint32_t*)((seat ? a.obs1 : a.obs0) + (size_t)e0 * FRAME);
             uint32_t* dst = (uint32_t*)((seat ? a.stack : a.stack0) + (size_t)e0 * STACK * FRAME + (size_t)a.phase * FRAME);
             for (int k = tid; k < ne * FRAME_WORDS; k += THREADS) {
                 const int e = k / FRAME_WORDS, j = k - e * FRAME_WORDS;
                 dst[(size_t)e * STACK * FRAME_WORDS + j] = src[k];
+                if (LEARNER && seat == 0 && a.done && a.done[e0 + e]) {
+                    uint32_t* ring = (uint32_t*)(a.stack0 + (size_t)(e0 + e) * STACK * FRAME);
+#pragma unroll
+                    for (int d = 1; d < STACK; ++d) ring[((a.phase + d) & 3) * FRAME_WORDS + j] = 0u;
+                }
             }
         }
         __syncthreads();
-        // ---- networks, slot by slot
-        for (int s = 0; s < CRL_PONG_OPP_SLOTS; ++s) {
-            const int m = cnt[s];
+        // ---- networks, slot by slot (learner mode: then the learner, for every env of the range)
+        for (int s = 0; s < NS; ++s) {
+            const bool lrn = LEARNER && s == CRL_PONG_OPP_SLOTS;
+            const int m = lrn ? ne : cnt[s];
             if (m == 0) continue;
-            {
+            if (lrn) {
+                const float4* src = (const float4*)a.learner;
+                for (int k = tid; k < NET_LRN / 4; k += THREADS) ((float4*)w)[k] = src[k];
+            } else {
                 const float4* src = (const float4*)(a.nets + (size_t)s * NET_DEV);
                 for (int k = tid; k < NET_DEV / 4; k += THREADS) ((float4*)w)[k] = src[k];
             }
             for (int q = 0; q < m; ++q) {
-                const int item = list[s * SEATS * SUB + q];
+                const int item = lrn ? q : list[s * SEATS * SUB + q];
                 const int i = e0 + (SEATS == 1 ? item : item & (SUB - 1));
-                const int seat = SEATS == 1 ? 1 : item >> 6;
-                {   // stack / 255 -> xs[ci][42][42], ci 0 = oldest
-                    const uint32_t* src = (const uint32_t*)((SEATS == 1 || seat ? a.stack : a.stack0) + (size_t)i * STACK * FRAME);
+                const int seat = lrn ? 0 : SEATS == 1 ? 1 : item >> 6;
+                {   // stack / 255 -> xs[ci][42][42], ci 0 = oldest (the learner's bytes also go to stack_out)
+                    const uint32_t* src = (const uint32_t*)(((SEATS == 1 && !LEARNER) || seat ? a.stack : a.stack0) + (size_t)i * STACK * FRAME);
                     for (int k = tid; k < STACK * FRAME_WORDS; k += THREADS) {
                         const int ci = k / FRAME_WORDS, j = k - ci * FRAME_WORDS;
                         const uint32_t v = src[((a.phase + 1 + ci) & 3) * FRAME_WORDS + j];
+                        if (lrn) ((uint32_t*)a.stack_out)[(size_t)i * STACK * FRAME_WORDS + k] = v;
                         float4 f;
                         f.x = lut[v & 255]; f.y = lut[(v >> 8) & 255]; f.z = lut[(v >> 16) & 255]; f.w = lut[v >> 24];
                         *(float4*)&xs[ci * FRAME + 4 * j] = f;
@@ -287,22 +349,25 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
                     for (int c = 0; c < 8; ++c) h2[(half * 8 + c) * H2 * H2 + p] = fmaxf(acc[c], 0.f);
                 }
                 __syncthreads();
-                {   // actor_linear: strided partial sums, warp tree, then 7 warp sums in order
-                    float s0 = 0.f, s1 = 0.f, s2 = 0.f;
+                {   // actor_linear (learner: and critic_linear): strided partial sums, warp tree, then 7 warp sums in order
+                    float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
                     for (int f = tid; f < FEATS; f += THREADS) {
                         const float x = h2[f];
                         s0 = __fmaf_rn(w[OFF_WA + f], x, s0);
                         s1 = __fmaf_rn(w[OFF_WA + FEATS + f], x, s1);
                         s2 = __fmaf_rn(w[OFF_WA + 2 * FEATS + f], x, s2);
+                        if (lrn) s3 = __fmaf_rn(w[OFF_WC + f], x, s3);
                     }
 #pragma unroll
                     for (int o = 16; o > 0; o >>= 1) {
                         s0 += __shfl_xor_sync(0xffffffffu, s0, o);
                         s1 += __shfl_xor_sync(0xffffffffu, s1, o);
                         s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+                        if (lrn) s3 += __shfl_xor_sync(0xffffffffu, s3, o);
                     }
                     if ((tid & 31) == 0) {
-                        red[3 * (tid >> 5)] = s0; red[3 * (tid >> 5) + 1] = s1; red[3 * (tid >> 5) + 2] = s2;
+                        red[L::RS * (tid >> 5)] = s0; red[L::RS * (tid >> 5) + 1] = s1; red[L::RS * (tid >> 5) + 2] = s2;
+                        if (lrn) red[L::RS * (tid >> 5) + 3] = s3;
                     }
                 }
                 __syncthreads();
@@ -311,8 +376,14 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
 #pragma unroll
                     for (int k = 0; k < 3; ++k) {
                         float v = 0.f;
-                        for (int wi = 0; wi < THREADS / 32; ++wi) v += red[3 * wi + k];
+                        for (int wi = 0; wi < THREADS / 32; ++wi) v += red[L::RS * wi + k];
                         l[k] = v + w[OFF_BA + k];
+                    }
+                    if (lrn) {
+                        float v = 0.f;
+                        for (int wi = 0; wi < THREADS / 32; ++wi) v += red[L::RS * wi + 3];
+                        learner_out(a, i, l, v + w[OFF_BC]);
+                        continue;      // the rest of this block is a pool network's; thread 0 joins the next barrier
                     }
                     int act = 0;                       // argmax, ties to the lowest index
                     float best = l[0];
@@ -342,7 +413,7 @@ __global__ void pong_opp_draw_kernel(const OppArgs a) {
 using namespace crl::opp;
 
 struct crl_pong_opp {
-    int n = 0, device = 0, grid = 0, grid_league = 0;
+    int n = 0, device = 0, grid = 0, grid_league = 0, grid_learner = 0;
     uint64_t seed = 0;
     int64_t first_env = 0;
     uint64_t steps = 0;
@@ -363,8 +434,12 @@ struct crl_pong_opp {
     bool league = false;
     int num_pairs = 0;
     uint8_t pairs[CRL_PONG_OPP_MAX_PAIRS][2] = {};
-    uint8_t* stack0 = nullptr;                 // allocated by the first crl_pong_opp_set_pairs
-    unsigned long long* pair_stats = nullptr;  // [CRL_PONG_OPP_MAX_PAIRS][4], allocated with stack0
+    uint8_t* stack0 = nullptr;                 // seat 0's stacks (league) or the learner's rings, allocated on first use
+    unsigned long long* pair_stats = nullptr;  // [CRL_PONG_OPP_MAX_PAIRS][4], allocated by the first crl_pong_opp_set_pairs
+    // learner mode
+    bool learner = false;
+    bool learner_loaded = false;
+    float* learner_net = nullptr;              // [NET_LRN]
 };
 
 static OppArgs opp_args(const crl_pong_opp* h) {
@@ -397,19 +472,26 @@ int crl_pong_opp_create(int32_t num_envs, int32_t device, uint64_t seed, int64_t
     crl_pong_opp* h = new crl_pong_opp();
     h->n = num_envs; h->device = device; h->seed = seed; h->first_env = first_env;
     const size_t n = (size_t)num_envs;
-    int sms = 0, per_sm = 0, per_sm_league = 0;
+    int sms = 0, per_sm = 0, per_sm_league = 0, per_sm_learner = 0;
     cudaError_t err = cudaSuccess;
     auto alloc = [&](auto** p, size_t count) { if (err == cudaSuccess) err = h->allocs.alloc(p, count); };
     alloc(&h->nets, (size_t)NET_DEV * CRL_PONG_OPP_SLOTS);
+    alloc(&h->learner_net, (size_t)NET_LRN);
     alloc(&h->ids, n); alloc(&h->stack, (size_t)STACK * FRAME * n); alloc(&h->ret, n); alloc(&h->episodes, n);
     alloc(&h->stats, 4 * CRL_PONG_OPP_MAX_POOL);
-    if (err == cudaSuccess) err = cudaFuncSetAttribute(pong_opp_act_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(pong_opp_act_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
     if (err == cudaSuccess)
-        err = cudaFuncSetAttribute(pong_opp_act_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes<2>());
+        err = cudaFuncSetAttribute(pong_opp_act_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes<2>());
+    if (err == cudaSuccess)
+        err = cudaFuncSetAttribute(pong_opp_act_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)smem_bytes<1, true>());
     if (err == cudaSuccess) err = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-    if (err == cudaSuccess) err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pong_opp_act_kernel<1>, THREADS, SMEM_BYTES);
+    if (err == cudaSuccess) err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pong_opp_act_kernel<1, false>, THREADS, SMEM_BYTES);
     if (err == cudaSuccess)
-        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_league, pong_opp_act_kernel<2>, THREADS, smem_bytes<2>());
+        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_league, pong_opp_act_kernel<2, false>, THREADS, smem_bytes<2>());
+    if (err == cudaSuccess)
+        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_learner, pong_opp_act_kernel<1, true>, THREADS,
+                                                            smem_bytes<1, true>());
     if (err == cudaSuccess) err = cudaDeviceSynchronize();
     if (err != cudaSuccess) {
         crl_pong_opp_destroy(h);
@@ -418,6 +500,7 @@ int crl_pong_opp_create(int32_t num_envs, int32_t device, uint64_t seed, int64_t
     // one resident wave: every CTA owns an equal contiguous range of envs
     h->grid = (int)std::min<int64_t>((int64_t)std::max(per_sm, 1) * sms, num_envs);
     h->grid_league = (int)std::min<int64_t>((int64_t)std::max(per_sm_league, 1) * sms, num_envs);
+    h->grid_learner = (int)std::min<int64_t>((int64_t)std::max(per_sm_learner, 1) * sms, num_envs);
     *out = h;
     return CRL_OK;
 }
@@ -428,14 +511,14 @@ int crl_pong_opp_seed(crl_pong_opp* h, uint64_t seed) {
     return CRL_OK;
 }
 
-int crl_pong_opp_load_net(crl_pong_opp* h, int32_t slot, const float* params_host, size_t count, void* stream) {
-    CHECK_HANDLE(h, h->device);
-    if (slot < 0 || slot >= CRL_PONG_OPP_SLOTS) return crl_set_error(CRL_E_INVALID, "network slot must be in [0, %d)", CRL_PONG_OPP_SLOTS);
+// checks a state-dict image and copies it to dst in the device layout: a slot image (NET_DEV floats) or, with the
+// critic, the learner's (NET_LRN).  Synchronises the stream.
+static int load_image(float* dst, int floats, const float* params_host, size_t count, void* stream) {
     if (!params_host || count != (size_t)CRL_PONG_OPP_NET_FLOATS)
         return crl_set_error(CRL_E_INVALID, "a LightActorCritic parameter image has %d floats (got %zu)", CRL_PONG_OPP_NET_FLOATS, count);
     for (size_t k = 0; k < count; ++k)
         if (!std::isfinite(params_host[k])) return crl_set_error(CRL_E_INVALID, "network parameter %zu is not finite", k);
-    std::vector<float> img(NET_DEV, 0.f);
+    std::vector<float> img(floats, 0.f);
     const float* p = params_host;
     for (int co = 0; co < C1; ++co)
         for (int t = 0; t < 64; ++t) img[OFF_W1 + t * C1 + co] = p[SD_W1 + co * 64 + t];     // [co][ci][kh][kw] -> [tap][co]
@@ -445,10 +528,27 @@ int crl_pong_opp_load_net(crl_pong_opp* h, int32_t slot, const float* params_hos
     for (int co = 0; co < C2; ++co) img[OFF_B2 + co] = p[SD_B2 + co];
     for (int k = 0; k < 3 * FEATS; ++k) img[OFF_WA + k] = p[SD_WA + k];
     for (int k = 0; k < 3; ++k) img[OFF_BA + k] = p[SD_BA + k];
-    CUDA_TRY(cudaMemcpyAsync(h->nets + (size_t)slot * NET_DEV, img.data(), sizeof(float) * NET_DEV, cudaMemcpyHostToDevice,
-                             (cudaStream_t)stream));
+    if (floats == NET_LRN) {
+        for (int k = 0; k < FEATS; ++k) img[OFF_WC + k] = p[SD_WC + k];
+        img[OFF_BC] = p[SD_BC];
+    }
+    CUDA_TRY(cudaMemcpyAsync(dst, img.data(), sizeof(float) * floats, cudaMemcpyHostToDevice, (cudaStream_t)stream));
     CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
+    return CRL_OK;
+}
+
+int crl_pong_opp_load_net(crl_pong_opp* h, int32_t slot, const float* params_host, size_t count, void* stream) {
+    CHECK_HANDLE(h, h->device);
+    if (slot < 0 || slot >= CRL_PONG_OPP_SLOTS) return crl_set_error(CRL_E_INVALID, "network slot must be in [0, %d)", CRL_PONG_OPP_SLOTS);
+    if (int r = load_image(h->nets + (size_t)slot * NET_DEV, NET_DEV, params_host, count, stream)) return r;
     h->loaded[slot] = true;
+    return CRL_OK;
+}
+
+int crl_pong_opp_load_learner(crl_pong_opp* h, const float* params_host, size_t count, void* stream) {
+    CHECK_HANDLE(h, h->device);
+    if (int r = load_image(h->learner_net, NET_LRN, params_host, count, stream)) return r;
+    h->learner_loaded = true;
     return CRL_OK;
 }
 
@@ -479,6 +579,7 @@ int crl_pong_opp_set_pool(crl_pong_opp* h, const int32_t* kinds_host, const doub
     }
     h->pool_size = pool_size;
     h->assigned = false;
+    h->learner = false;
     CUDA_TRY(cudaMemsetAsync(h->stats, 0, sizeof(unsigned long long) * 4 * CRL_PONG_OPP_MAX_POOL, (cudaStream_t)stream));
     if (h->league) {   // leaving league mode: the per-env opponents start as on a fresh handle (the act count runs on)
         h->league = false;
@@ -512,6 +613,8 @@ int crl_pong_opp_restart(crl_pong_opp* h, int32_t clear_stacks, void* stream) {
         CUDA_TRY(cudaMemsetAsync(h->stack, 0, (size_t)STACK * FRAME * h->n, (cudaStream_t)stream));
         if (h->stack0) CUDA_TRY(cudaMemsetAsync(h->stack0, 0, (size_t)STACK * FRAME * h->n, (cudaStream_t)stream));
         h->phase = 0;
+    } else if (h->learner) {   // a reset starts every learner episode afresh (FrameStackTensor.reset)
+        CUDA_TRY(cudaMemsetAsync(h->stack0, 0, (size_t)STACK * FRAME * h->n, (cudaStream_t)stream));
     }
     return CRL_OK;
 }
@@ -520,6 +623,7 @@ int crl_pong_opp_act(crl_pong_opp* h, const uint8_t* obs1_dev, const float* rew_
                      int32_t* actions_dev, float* logits_dev, void* stream) {
     CHECK_HANDLE(h, h->device);
     if (h->league) return crl_set_error(CRL_E_STATE, "league mode: use crl_pong_opp_act_pairs (crl_pong_opp_set_pool leaves it)");
+    if (h->learner) return crl_set_error(CRL_E_STATE, "learner mode: use crl_pong_opp_act_learner (crl_pong_opp_set_pool leaves it)");
     if (!h->assigned) return crl_set_error(CRL_E_STATE, "crl_pong_opp_assign after every crl_pong_opp_set_pool");
     if (!obs1_dev || !actions_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
     if ((rew_dev == nullptr) != (done_dev == nullptr)) return crl_set_error(CRL_E_INVALID, "rew_dev and done_dev go together");
@@ -527,7 +631,7 @@ int crl_pong_opp_act(crl_pong_opp* h, const uint8_t* obs1_dev, const float* rew_
     OppArgs a = opp_args(h);
     a.resample = resample ? 1 : 0;
     a.obs1 = obs1_dev; a.rew = rew_dev; a.done = done_dev; a.actions = actions_dev; a.logits = logits_dev;
-    LAUNCH((pong_opp_act_kernel<1><<<h->grid, THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(a), cudaGetLastError()), 1);
+    LAUNCH((pong_opp_act_kernel<1, false><<<h->grid, THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(a), cudaGetLastError()), 1);
     h->phase = (h->phase + 1) & 3;
     h->steps += 1;
     return CRL_OK;
@@ -543,13 +647,14 @@ int crl_pong_opp_set_pairs(crl_pong_opp* h, const int32_t* pairs_host, int32_t n
             if (pairs_host[2 * p + seat] < 0 || pairs_host[2 * p + seat] >= h->pool_size)
                 return crl_set_error(CRL_E_INVALID, "pairing %d, seat %d: pool index %d is not in [0, %d)", p, seat,
                                      pairs_host[2 * p + seat], h->pool_size);
-    if (!h->stack0) {
+    if (!h->pair_stats) {
+        const bool had_stack0 = h->stack0 != nullptr;   // learner mode came first
         cudaError_t err = h->allocs.alloc(&h->pair_stats, 4 * CRL_PONG_OPP_MAX_PAIRS);
-        if (err == cudaSuccess) err = h->allocs.alloc(&h->stack0, (size_t)STACK * FRAME * h->n);
+        if (err == cudaSuccess && !had_stack0) err = h->allocs.alloc(&h->stack0, (size_t)STACK * FRAME * h->n);
         if (err != cudaSuccess) {   // both or neither: a failed call leaves the handle as it was
             h->allocs.free(h->pair_stats);
             h->pair_stats = nullptr;
-            h->stack0 = nullptr;
+            if (!had_stack0) h->stack0 = nullptr;
             return crl_set_error(CRL_E_CUDA, "crl_pong_opp_set_pairs: %s", cudaGetErrorString(err));
         }
     }
@@ -563,6 +668,7 @@ int crl_pong_opp_set_pairs(crl_pong_opp* h, const int32_t* pairs_host, int32_t n
     h->num_pairs = num_pairs;
     h->phase = 0;
     h->league = true;
+    h->learner = false;
     return CRL_OK;
 }
 
@@ -580,7 +686,42 @@ int crl_pong_opp_act_pairs(crl_pong_opp* h, const uint8_t* obs0_dev, const uint8
     memcpy(a.pairs, h->pairs, sizeof a.pairs);
     a.obs0 = obs0_dev; a.obs1 = obs1_dev; a.stack0 = h->stack0;
     a.rew = rew_dev; a.done = done_dev; a.actions = actions_dev; a.logits = logits_dev;
-    LAUNCH((pong_opp_act_kernel<2><<<h->grid_league, THREADS, smem_bytes<2>(), (cudaStream_t)stream>>>(a), cudaGetLastError()), 1);
+    LAUNCH((pong_opp_act_kernel<2, false><<<h->grid_league, THREADS, smem_bytes<2>(), (cudaStream_t)stream>>>(a), cudaGetLastError()), 1);
+    h->phase = (h->phase + 1) & 3;
+    h->steps += 1;
+    return CRL_OK;
+}
+
+int crl_pong_opp_act_learner(crl_pong_opp* h, const uint8_t* obs0_dev, const uint8_t* obs1_dev, const float* rew_dev,
+                             const uint8_t* done_dev, int32_t resample, int32_t sample, int32_t* actions_dev,
+                             float* logp_value_dev, float* logits_dev, uint8_t* stack_out_dev, void* stream) {
+    CHECK_HANDLE(h, h->device);
+    if (!h->learner_loaded) return crl_set_error(CRL_E_STATE, "crl_pong_opp_load_learner first");
+    if (h->league) return crl_set_error(CRL_E_STATE, "league mode: use crl_pong_opp_act_pairs (crl_pong_opp_set_pool leaves it)");
+    if (!h->assigned) return crl_set_error(CRL_E_STATE, "crl_pong_opp_assign after every crl_pong_opp_set_pool");
+    if (!obs0_dev || !obs1_dev || !actions_dev || !logp_value_dev || !stack_out_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
+    if ((rew_dev == nullptr) != (done_dev == nullptr)) return crl_set_error(CRL_E_INVALID, "rew_dev and done_dev go together");
+    if (((uintptr_t)obs0_dev & 3) != 0 || ((uintptr_t)obs1_dev & 3) != 0 || ((uintptr_t)stack_out_dev & 3) != 0)
+        return crl_set_error(CRL_E_INVALID, "obs0_dev, obs1_dev and stack_out_dev must be 4-byte aligned");
+    const cudaStream_t s = (cudaStream_t)stream;
+    if (!h->learner) {   // entering learner mode: fresh rings
+        if (!h->stack0) {
+            const cudaError_t err = h->allocs.alloc(&h->stack0, (size_t)STACK * FRAME * h->n);
+            if (err != cudaSuccess) {
+                h->stack0 = nullptr;
+                return crl_set_error(CRL_E_CUDA, "crl_pong_opp_act_learner: %s", cudaGetErrorString(err));
+            }
+        }
+        CUDA_TRY(cudaMemsetAsync(h->stack0, 0, (size_t)STACK * FRAME * h->n, s));
+        h->learner = true;
+    }
+    OppArgs a = opp_args(h);
+    a.resample = resample ? 1 : 0;
+    a.sample = sample ? 1 : 0;
+    a.obs0 = obs0_dev; a.obs1 = obs1_dev; a.stack0 = h->stack0; a.learner = h->learner_net;
+    a.rew = rew_dev; a.done = done_dev; a.actions = actions_dev;
+    a.logp_value = logp_value_dev; a.learner_logits = logits_dev; a.stack_out = stack_out_dev;
+    LAUNCH((pong_opp_act_kernel<1, true><<<h->grid_learner, THREADS, smem_bytes<1, true>(), s>>>(a), cudaGetLastError()), 1);
     h->phase = (h->phase + 1) & 3;
     h->steps += 1;
     return CRL_OK;

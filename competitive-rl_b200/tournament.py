@@ -7,7 +7,11 @@ Two modes:
   * uniform (the reference's): one opponent plays every env; `reset_opponent(name)` switches it for the whole batch.
   * per-env (`set_opponents`): every env plays its own opponent from a pool, evaluated for the whole batch by one CUDA
     kernel per step (csrc/pong_opponent.cu, include/crl_b200.h crl_pong_opp_*).  See `set_opponents` for the rules.
-    `reset_opponent` returns to uniform mode."""
+    `reset_opponent` returns to uniform mode.
+
+In per-env mode a LightActorCritic learner can also act in the same launch (`set_learner`, `learner_step`): it samples
+its action and returns its log-probability, its value and the stacked observation it acted on, as a PPO rollout
+stores them."""
 import numpy as np
 import torch
 
@@ -36,6 +40,9 @@ class TournamentEnvWrapper(object):
         self._pool, self._resample, self._seed = None, False, 0
         self._have_prev = False               # env._rew / env._done hold the outputs of a step played in per-env mode
         self._both = None                     # int32 (N, 2) step buffer of per-env mode: learner | opponent
+        # learner
+        self.learner_logits = None            # float32 (N, 3) device tensor: learner steps write the learner's logits here
+        self._sample = None                   # set_learner's `sample`; None until a learner is loaded
 
     def _agent(self, name):
         if name not in self.agents:
@@ -149,6 +156,43 @@ class TournamentEnvWrapper(object):
         return {name: dict(episodes=int(s[4 * k]), wins=int(s[4 * k + 1]), draws=int(s[4 * k + 2]), losses=int(s[4 * k + 3]))
                 for k, name in enumerate(self._pool)}
 
+    # ------------------------------------------------------------------ learner
+    def set_learner(self, module_or_state_dict, sample=True):
+        """Load the learner's weights for learner_step: a LightActorCritic module, its state dict or a checkpoint dict
+        ({"model": state_dict}); ActorCritic layouts are refused.  Needs per-env mode (set_opponents).  Call it again
+        after every update to refresh the weights (one host synchronisation); they take effect on the next
+        learner_step.  sample: sample the action from the softmax of the logits, else take the argmax."""
+        if not self.per_env:
+            raise RuntimeError("set_learner needs per-env opponents: call set_opponents first")
+        self._opp.load_learner(pack_light_actor_critic(module_or_state_dict))
+        self._sample = bool(sample)
+
+    def learner_step(self, stack_out=None):
+        """One step in which the learner (set_learner) acts for agent 0 and the per-env opponents for agent 1, both in one
+        kernel launch, then the env steps.  Returns (stack, action, log_prob, value, obs, reward, done, info):
+          stack     uint8 (N, 4, 42, 42): the learner's last 4 observations, oldest first, that it acted on (zeroed
+                    before the newest frame after a done, like FrameStackTensor); written into `stack_out` if given
+          action    int32 (N,); log_prob and value float32 (N,)
+          obs, reward, done, info   as step() returns them.
+        The learner's frames are stacked by the kernel (include/crl_b200.h, learner mode); step() is refused once
+        learner steps have started, until set_opponents is called again.  learner_logits, if set, receives the
+        learner's logits; opponent_logits is not written by learner steps."""
+        if not self.per_env or self._sample is None:
+            raise RuntimeError("no learner: call set_opponents, then set_learner")
+        env = self.env
+        dev = env.device
+        n = self.num_envs
+        if stack_out is None:
+            stack_out = torch.empty((n, 4, 42, 42), dtype=torch.uint8, device=dev)
+        both = torch.empty((n, 2), dtype=torch.int32, device=dev)
+        lpv = torch.empty((n, 2), dtype=torch.float32, device=dev)
+        prev = (env._rew, env._done) if self._have_prev else (None, None)
+        self._opp.act_learner(env._obs[0], env._obs[1], prev[0], prev[1], self._resample, self._sample, both, lpv,
+                              self.learner_logits, stack_out)
+        self._both = both
+        out = self._env_step(both)
+        return (stack_out, both[:, 0], lpv[:, 0], lpv[:, 1]) + out
+
     # ------------------------------------------------------------------ VecEnv protocol
     def step(self, action):
         a = torch.as_tensor(np.asarray(action) if not isinstance(action, torch.Tensor) else action)
@@ -161,6 +205,9 @@ class TournamentEnvWrapper(object):
             both = self._both
         else:
             both = torch.stack([a, self.current_agent(self.prev_opponent_obs).reshape(-1)], dim=1)
+        return self._env_step(both)
+
+    def _env_step(self, both):
         obs, rew, done, info = self.env.step(both)
         self._have_prev = self.per_env
         self.prev_opponent_obs = obs[1]

@@ -256,6 +256,33 @@ int crl_obs_free(void* ptr);
  *               crl_pong_opp_set_pool leaves league mode: it zeroes the per-env reward sums and agent 1's stacks (the act
  *               count runs on), and crl_pong_opp_assign must follow it as always.  League mode does not change the
  *               opponent ids, the episode counts of the draws or the per-entry statistics of crl_pong_opp_get_stats.
+ *
+ * Learner mode (crl_pong_opp_load_learner, crl_pong_opp_act_learner): per-env opponents as above in seat 1, and in seat 0
+ * a LightActorCritic learner whose network runs in the same launch, returning what a PPO rollout stores for the step.
+ *   Learner     its own weights (crl_pong_opp_load_learner: the whole image, critic included), not one of the 8 slots,
+ *               so a pool keeps all of them.  Every env runs it, whatever its opponent.
+ *   Seat 1      exactly as crl_pong_opp_act: bookkeeping, redraws, pool actions, agent 1's stack, the act count, the
+ *               per-entry statistics.  Only the opponents' logits are not returned.
+ *   Ring        a uint8 [4][42][42] stack per env of agent 0's observations, oldest -> newest, with FrameStackTensor's
+ *               semantics (utils/utils.py:145-173): every act_learner pushes agent 0's observation of the previous step,
+ *               and when that step's done is set the env's ring is zeroed first, so that only the newest slot is
+ *               non-zero.  All rings are zeroed on entering learner mode (the first act_learner after create,
+ *               crl_pong_opp_set_pool or crl_pong_opp_set_pairs) and by every crl_pong_opp_restart in learner mode,
+ *               whatever clear_stacks (a VecEnv reset starts every episode afresh).  They take num_envs * 7056 bytes,
+ *               allocated by the first act_learner (shared with league mode's seat-0 stacks).
+ *   Network     conv1 / conv2 / actor exactly as for a pool network (fp32 over stack / 255), and critic_linear
+ *               (1600 -> 1) as one more sum of the same kind.
+ *   Action      sample != 0: u = r32 * 2^-32 from Philox keyed by (seed, global env index, act count) with tag 4, a
+ *               stream of its own, so it does not depend on the sharding or the batch; with m = max(l) and
+ *               e_k = expf(l_k - m), s = (e_0 + e_1) + e_2, c_0 = e_0 / s and c_1 = c_0 + e_1 / s in fp32, the action
+ *               is 0 if u < c_0, 1 if u < c_1, else 2 (u and c_k compared exactly).  sample == 0: the argmax of the
+ *               logits, ties to the lowest index.
+ *   Outputs     the action in column 0 of the step buffer; log pi(action) = l_a - (m + logf(s)) and the value; the
+ *               logits if asked; the stack the learner acted on (the ring after the push, oldest -> newest).
+ *   Modes       crl_pong_opp_act returns CRL_E_STATE in learner mode, so the two cannot be mixed: a frame of agent 0
+ *               would be missing from the rings.  crl_pong_opp_set_pool and crl_pong_opp_set_pairs leave learner mode;
+ *               crl_pong_opp_act_learner returns CRL_E_STATE in league mode, before crl_pong_opp_load_learner and before
+ *               crl_pong_opp_assign.  Reloading the learner's weights does not leave learner mode.
  * ====================================================================================== */
 #define CRL_PONG_OPP_MAX_POOL 16
 #define CRL_PONG_OPP_SLOTS 8
@@ -264,7 +291,7 @@ int crl_obs_free(void* ptr);
 #define CRL_PONG_OPP_MAX_PAIRS 256    /* pairings of league mode */
 /* LightActorCritic parameters in state-dict order, each row-major: conv1.weight [16][4][4][4], conv1.bias [16],
  * conv2.weight [16][16][2][2], conv2.bias [16], critic_linear.weight [1][1600], critic_linear.bias [1],
- * actor_linear.weight [3][1600], actor_linear.bias [3] (the critic is carried but not evaluated) */
+ * actor_linear.weight [3][1600], actor_linear.bias [3] (the critic is evaluated for the learner only) */
 #define CRL_PONG_OPP_NET_FLOATS 8484
 
 typedef struct crl_pong_opp crl_pong_opp; /* opaque handle: the opponents of one shard of envs on one GPU */
@@ -314,6 +341,21 @@ int crl_pong_opp_act_pairs(crl_pong_opp* h, const uint8_t* obs0_dev, const uint8
  * crl_pong_opp_set_pairs).  1 <= num_pairs <= CRL_PONG_OPP_MAX_PAIRS; rows past the league's P read 0.  Synchronises
  * the stream. */
 int crl_pong_opp_get_pair_stats(crl_pong_opp* h, uint64_t* stats_host, int32_t num_pairs, void* stream);
+/* learner <- params_host[CRL_PONG_OPP_NET_FLOATS] (finite), the whole image (pack_light_actor_critic order), critic
+ * included; checked as crl_pong_opp_load_net.  Synchronises the stream: call it once per update, not per step. */
+int crl_pong_opp_load_learner(crl_pong_opp* h, const float* params_host, size_t count, void* stream);
+/* One learner-mode step, before crl_pong_step (enters learner mode, see above):
+ *   obs0_dev, obs1_dev  uint8 [num_envs][42][42] agent 0's and agent 1's observations of the previous step, 4-byte aligned
+ *   rew_dev, done_dev   as crl_pong_opp_act (both NULL for the first act after a reset)
+ *   resample            as crl_pong_opp_act
+ *   sample              != 0: sample the learner's action from its softmax; 0: the argmax
+ *   actions_dev         int32 [num_envs][2]: column 0 the learner's action, column 1 the opponent's
+ *   logp_value_dev      float32 [num_envs][2]: log pi(action), value
+ *   logits_dev          float32 [num_envs][3] or NULL: the learner's logits
+ *   stack_out_dev       uint8 [num_envs][4][42][42], 4-byte aligned: the stack the learner acted on, oldest first */
+int crl_pong_opp_act_learner(crl_pong_opp* h, const uint8_t* obs0_dev, const uint8_t* obs1_dev, const float* rew_dev,
+                             const uint8_t* done_dev, int32_t resample, int32_t sample, int32_t* actions_dev,
+                             float* logp_value_dev, float* logits_dev, uint8_t* stack_out_dev, void* stream);
 
 /* ======================================================================================
  * cCarRacing-v0 / cCarRacingDouble-v0
