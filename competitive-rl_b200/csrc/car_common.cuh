@@ -32,6 +32,13 @@ constexpr int CAR_MAP_BLOCK = 16, CAR_MAP_GRID = 128, CAR_MAP_ORIGIN = 5000 - 10
 constexpr int CAR_MAP_MAX_BLOCKS = 768;     // blocks a track may paint (standard tracks: 260-450); 192 KB per track slot
 constexpr int CAR_MAX_CONTACTS = 8;         // touching car-car fixture pairs kept per env (of 48 possible)
 constexpr int CAR_RAW_RING = 1024;          // raw points of the curve follower kept while it walks (last lap + tail)
+// Tiles of a track that the wheel-tile prefilter's constant radii do not cover (sensor_wheel_overlaps): a vertex farther
+// than CAR_WIDE_REACH from the tile's track point, or a track point farther than CAR_WIDE_GROUP from its group's sample
+// point.  Generated tracks have one, the seam tile 0 (its gap along the track is up to ~14.5 units against 3.5 elsewhere);
+// recorded tracks with more than CAR_MAX_WIDE are refused by crl_car_load_tracks.
+constexpr int CAR_MAX_WIDE = 4;
+constexpr float CAR_WIDE_REACH = 8.3f;      // 9 (wheel radius of the prefilter) - 0.6083 (wheel circumradius) - 2 skins, less slack
+constexpr float CAR_WIDE_GROUP = 24.9f;     // 36 (sample radius) - 11 (track point to hull of a touching wheel), less slack
 
 // A road tile, 124 bytes: for the physics the convex hull (CCW, fp32) of the reference's 5 listed
 // vertices, with the edge normals the sensor-overlap test needs; for the renderer the listed vertices and the kerb quad in ROAD-MAP PIXELS, i.e.
@@ -148,6 +155,7 @@ struct CarDev {
     uint8_t* map_blocks;
     const uint8_t* chk;       // [2][2048] 0xFF where map column (axis 0) / row (axis 1) CAR_MAP_ORIGIN + i lies in a checker square (:733-746)
     float2* tile_centres;     // [2n][CAR_MAX_TRACK] tile centres (= CarTile::cx, cy), contiguous for the step kernel's candidate search
+    float4* wide_tiles;       // [2n][CAR_MAX_WIDE] tiles the prefilter radii miss: track point x, y, reach, tile id (reach < 0: unused)
     // ---- per frame (env * players + player): written by car_frame_setup_kernel, read by car_render_kernel ----
     FrameMap* frame_map;      // [n*players]
     uint8_t* frame_aux;       // [n*players] FrameAux records (car polygon span tables, road-map block list)

@@ -346,6 +346,26 @@ __device__ int generate_track_warp(const CarDev& p, int e, int slot, bool for_pr
     __syncwarp();
     for (int i = lane; i < n; i += 32) build_tile(pts, n, i, tiles[i].flags, tiles, centres);
     for (int i = n + lane; i < CAR_MAX_TRACK; i += 32) tiles[i].flags = 0;
+    // the tiles the prefilter's constant radii do not cover (CAR_WIDE_REACH / CAR_WIDE_GROUP), listed with their reach
+    float4* wide = p.wide_tiles + (size_t)slot * CAR_MAX_WIDE;
+    int n_wide = 0;
+    for (int base = 0; base < n; base += 32) {
+        const int i = base + lane;                       // the lane that built tile i above
+        float4 w = make_float4(0.f, 0.f, -1.f, 0.f);
+        if (i < n) {
+            const CarTile& T = tiles[i];
+            float reach = 0.f;
+            for (int k = 0; k < T.n; ++k) reach = fmaxf(reach, sqrtf((T.px[k] - T.cx) * (T.px[k] - T.cx) + (T.py[k] - T.cy) * (T.py[k] - T.cy)));
+            const int s = i - i % CAR_SAMPLE_STRIDE;
+            const float gx = T.cx - (float)pts[3 * s + 1], gy = T.cy - (float)pts[3 * s + 2];
+            if (reach > CAR_WIDE_REACH || gx * gx + gy * gy > CAR_WIDE_GROUP * CAR_WIDE_GROUP) w = make_float4(T.cx, T.cy, reach, (float)i);
+        }
+        const unsigned m = __ballot_sync(0xffffffffu, w.z >= 0.f);
+        const int k = n_wide + __popc(m & ((1u << lane) - 1u));
+        if (w.z >= 0.f && k < CAR_MAX_WIDE) wide[k] = w;   // more cannot come from a generated track; load_tracks refuses them
+        n_wide += __popc(m);
+    }
+    for (int k = n_wide + lane; k < CAR_MAX_WIDE; k += 32) wide[k] = make_float4(0.f, 0.f, -1.f, 0.f);
     for (int s = lane; s < CAR_MAX_SAMPLES; s += 32) {
         const int i = s * CAR_SAMPLE_STRIDE;
         p.samples[(size_t)s * (2 * p.n) + slot] = (i < n) ? make_float2((float)pts[3 * i + 1], (float)pts[3 * i + 2])
@@ -605,8 +625,8 @@ __device__ __forceinline__ bool cars_near(const float (*pose)[3], float hull_lcx
 
 // b2ContactManager::Collide for the tile sensors of ONE wheel: the road tiles whose fixture overlaps the wheel box (SAT
 // with the b2_polygonRadius skins), as a 512-bit set in now16[16] (global memory).  Candidates: every 8th track point
-// within 36 units of the hull (transposed array: coalesced), then tile centres within 11.5 of the hull and 9 of the wheel.
-// `near_samples`: bit s set = track point 8 s lies within 36 units of the hull (0 = not known: scanned here).
+// within 36 units of the hull (transposed array: coalesced), then tile centres within 11.5 of the hull and 9 of the wheel;
+// plus the slot's wide tiles (generate_track_warp), which those radii would miss.  `near_samples`: bit s set = track point 8 s lies within 36 units of the hull (0 = not known: scanned here).
 __device__ void sensor_wheel_overlaps(const CarDev& p, int slot, int n_track, F2 hp, F2 wc, float wa, uint32_t* __restrict__ now16,
                                       unsigned long long near_samples, bool have_near) {
     const CarTile* tiles = p.tiles + (size_t)slot * CAR_MAX_TRACK;
@@ -677,6 +697,18 @@ __device__ void sensor_wheel_overlaps(const CarDev& p, int slot, int n_track, F2
             if (n_cand < 6) { cand |= (unsigned long long)t << (10 * n_cand); ++n_cand; }
             else test_tile(t);                                     // more candidates than the word holds: on the spot
         }
+    }
+    // tiles that reach farther than the radii above assume (the seam tile of every generated track): candidates whenever
+    // the wheel box (circumradius 0.6083, two skins 0.02) can reach the tile's far vertex; a repeated test only sets its
+    // bit again
+    const float4* wide = p.wide_tiles + (size_t)slot * CAR_MAX_WIDE;
+    for (int j = 0; j < CAR_MAX_WIDE; ++j) {
+        const float4 wt = wide[j];
+        if (!(wt.z >= 0.f)) break;
+        const float dx = wt.x - wc.x, dy = wt.y - wc.y, r = wt.z + 0.65f;
+        if (!(dx * dx + dy * dy <= r * r)) continue;
+        if (n_cand < 6) { cand |= (unsigned long long)(int)wt.w << (10 * n_cand); ++n_cand; }
+        else test_tile((int)wt.w);
     }
     for (int j = 0; j < n_cand; ++j) test_tile((int)((cand >> (10 * j)) & 1023ull));
 }

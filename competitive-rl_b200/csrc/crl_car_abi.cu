@@ -334,7 +334,7 @@ int crl_car_create(const crl_car_config* cfg, crl_car** out) {
         alloc(&d.frame_aux, nc * car_frame_aux_bytes());
     }
     alloc(&d.map_index, 2 * n * CAR_MAP_GRID * CAR_MAP_GRID); alloc(&d.map_blocks, 2 * n * CAR_MAP_MAX_BLOCKS * 256);
-    alloc(&d.tile_centres, 2 * n * CAR_MAX_TRACK);
+    alloc(&d.tile_centres, 2 * n * CAR_MAX_TRACK); alloc(&d.wide_tiles, 2 * n * CAR_MAX_WIDE);
     alloc(&h->actions_stage, nc * 2); alloc(&h->rew_stage, nc); alloc(&h->done_stage, n); alloc(&h->steps_stage, n); alloc(&h->trunc_stage, n);
     if (P == 2) { alloc(&d.contacts, n * CAR_MAX_CONTACTS); alloc(&d.n_contacts, n); alloc(&d.n_contacts_step, n); alloc(&d.slow_list, n); alloc(&d.slow_count, 2); d.near_count = d.slow_count + 1; alloc(&d.near_list, n); }
     alloc(&d.deferred, n);
@@ -417,6 +417,24 @@ int crl_car_inject_tracks(crl_car* h, const double* draws_host, int32_t k_draws,
     return CRL_OK;
 }
 
+// Tiles of a recorded track (beta, x, y per point) that the kernel would list in wide_tiles (generate_track_warp), counted
+// in fp64 with 0.05 units of margin on the kernel's fp32 thresholds, over the 5 listed vertices (the hull is a subset).
+static int count_wide_tiles(const double* pts, int n) {
+    const double w = 40.0 / 6.0, pi = 3.141592653589793;
+    int wide = 0;
+    for (int i = 0; i < n; ++i) {
+        const double *p1 = pts + 3 * i, *p2 = pts + 3 * ((i - 1 + n) % n), *ps = pts + 3 * (i - i % CAR_SAMPLE_STRIDE);
+        const double vx[5] = {p1[1] - w * cos(p1[0]), p1[1] - w / 2 * cos(p1[0] - pi / 2), p1[1] + w * cos(p1[0]),
+                              p2[1] + w * cos(p2[0]), p2[1] - w * cos(p2[0])};
+        const double vy[5] = {p1[2] - w * sin(p1[0]), p1[2] - w / 2 * sin(p1[0] - pi / 2), p1[2] + w * sin(p1[0]),
+                              p2[2] + w * sin(p2[0]), p2[2] - w * sin(p2[0])};
+        double reach = 0.0;
+        for (int k = 0; k < 5; ++k) reach = fmax(reach, hypot(vx[k] - p1[1], vy[k] - p1[2]));
+        if (reach > CAR_WIDE_REACH - 0.05 || hypot(p1[1] - ps[1], p1[2] - ps[2]) > CAR_WIDE_GROUP - 0.05) ++wide;
+    }
+    return wide;
+}
+
 int crl_car_load_tracks(crl_car* h, const double* pts_host, const int32_t* counts_host, int32_t n_tracks, void* stream) {
     CHECK_HANDLE(h, h->cfg.device);
     cudaStream_t s = (cudaStream_t)stream;
@@ -432,6 +450,12 @@ int crl_car_load_tracks(crl_car* h, const double* pts_host, const int32_t* count
     for (int k = 0; k < n_tracks; ++k)
         if (counts_host[k] < 9 || counts_host[k] > CAR_MAX_TRACK)
             return crl_set_error(CRL_E_INVALID, "track %d has %d points; need 9..%d", k, counts_host[k], CAR_MAX_TRACK);
+    for (int k = 0; k < n_tracks; ++k) {
+        const int wide = count_wide_tiles(pts_host + (size_t)k * CAR_MAX_TRACK * 3, counts_host[k]);
+        if (wide > CAR_MAX_WIDE)
+            return crl_set_error(CRL_E_INVALID, "track %d: %d tiles reach farther from their track point than the wheel-tile "
+                                 "contact search covers (at most %d per track; points too far apart?)", k, wide, CAR_MAX_WIDE);
+    }
     double* dp = nullptr;
     int32_t* dc = nullptr;
     CUDA_TRY(h->allocs.alloc(&dp, (size_t)n_tracks * CAR_MAX_TRACK * 3));
