@@ -29,7 +29,7 @@ EXPORTS = [
     "crl_pong_opp_create", "crl_pong_opp_destroy", "crl_pong_opp_seed", "crl_pong_opp_load_net", "crl_pong_opp_set_pool",
     "crl_pong_opp_assign", "crl_pong_opp_restart", "crl_pong_opp_act", "crl_pong_opp_get_ids", "crl_pong_opp_get_stats",
     "crl_pong_opp_set_pairs", "crl_pong_opp_act_pairs", "crl_pong_opp_get_pair_stats", "crl_pong_opp_load_learner",
-    "crl_pong_opp_act_learner",
+    "crl_pong_opp_act_learner", "crl_pong_opp_set_selfplay", "crl_pong_opp_act_selfplay",
 ]
 
 
@@ -164,6 +164,8 @@ def load():
     L.crl_pong_opp_get_pair_stats.argtypes = [vp, vp, i32, vp]
     L.crl_pong_opp_load_learner.argtypes = [vp, vp, ctypes.c_size_t, vp]
     L.crl_pong_opp_act_learner.argtypes = [vp, vp, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp]
+    L.crl_pong_opp_set_selfplay.argtypes = [vp, vp, i32, vp]
+    L.crl_pong_opp_act_selfplay.argtypes = [vp, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("crl_last_error", "crl_launch_count"):

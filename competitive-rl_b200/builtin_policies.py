@@ -225,6 +225,38 @@ def resolve_pool(pool, added=None, resource_dir=None):
     return names, kinds, images
 
 
+LEARNER = "LEARNER"   # a learner seat of a self-play pairing (selfplay.SelfPlayEnvWrapper); not a pool name there
+
+
+def resolve_pairs(pairs, pool, learner=False):
+    """Pairings as the opponent kernel takes them (include/crl_b200.h, crl_pong_opp_set_pairs and
+    crl_pong_opp_set_selfplay): a list of [seat 0, seat 1].  Each seat of `pairs` is a name in `pool` (the names
+    resolve_pool returned) or an index into it; with learner=True, "LEARNER" is a learner seat (CRL_PONG_OPP_LEARNER)
+    and may not also be a pool name.  ValueError, before anything is loaded, for a pairing that is not two seats, a name
+    not in the pool, an index out of range and for other than 1 to 256 pairings."""
+    from . import _native
+    ext = _native.ext()
+    m = len(pool)
+    if learner and LEARNER in pool:
+        raise ValueError("%s is reserved for the learner's seats: it cannot be a pool name" % LEARNER)
+    idx = []
+    for pr in pairs:
+        pr = list(pr)
+        if len(pr) != 2:
+            raise ValueError("a pairing is (seat 0, seat 1)")
+        for x in pr:
+            if isinstance(x, str) and x not in pool and not (learner and x == LEARNER):
+                raise ValueError("pairing %r: %r is not in the pool" % (tuple(pr), x))
+        is_lrn = [learner and isinstance(x, str) and x == LEARNER for x in pr]
+        k = [ext.OPP_LEARNER if lr else pool.index(x) if isinstance(x, str) else int(x) for x, lr in zip(pr, is_lrn)]
+        if not all(lr or 0 <= v < m for v, lr in zip(k, is_lrn)):
+            raise ValueError("pairing %r: pool indices must be in [0, %d)" % (tuple(pr), m))
+        idx.append(k)
+    if not 1 <= len(idx) <= ext.OPP_MAX_PAIRS:
+        raise ValueError("a league has 1 to %d pairings (got %d)" % (ext.OPP_MAX_PAIRS, len(idx)))
+    return idx
+
+
 def get_compute_action_function(agent_name, num_envs=1, device="cuda", resource_dir=None):
     """Callable obs -> int32 [num_envs] device tensor (pong/builtin_policies.py:61-91)."""
     device = torch.device(device)

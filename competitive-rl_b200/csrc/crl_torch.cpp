@@ -349,6 +349,25 @@ struct PongOpponents {
                                           dev_ptr<uint8_t>(stack_out, at::kByte, device, n() * 4 * 42 * 42, "stack_out"),
                                           stream_of(device)));
     }
+    // self-play mode.  pairs: int32 CPU tensor [P][2] of pool indices or CRL_PONG_OPP_LEARNER (seat 0, seat 1)
+    void set_selfplay(const at::Tensor& pairs) {
+        TORCH_CHECK(pairs.dim() == 2 && pairs.size(1) == 2, "pairs: expected shape (P, 2)");
+        check_rc(crl_pong_opp_set_selfplay(handle(), host_ptr<int32_t>(pairs, at::kInt, "pairs"), (int32_t)pairs.size(0),
+                                           stream_of(device)));
+    }
+    void act_selfplay(const at::Tensor& obs0, const at::Tensor& obs1, const c10::optional<at::Tensor>& rew,
+                      const c10::optional<at::Tensor>& done, bool sample, const at::Tensor& actions,
+                      const at::Tensor& logp_value, const c10::optional<at::Tensor>& logits, const at::Tensor& stack_out) {
+        check_rc(crl_pong_opp_act_selfplay(handle(), dev_ptr<uint8_t>(obs0, at::kByte, device, n() * 42 * 42, "obs0"),
+                                           dev_ptr<uint8_t>(obs1, at::kByte, device, n() * 42 * 42, "obs1"),
+                                           opt_dev_ptr<float>(rew, at::kFloat, device, 2 * n(), "rew"),
+                                           opt_dev_ptr<uint8_t>(done, at::kBool, device, n(), "done"), sample ? 1 : 0,
+                                           dev_ptr<int32_t>(actions, at::kInt, device, 2 * n(), "actions"),
+                                           dev_ptr<float>(logp_value, at::kFloat, device, 4 * n(), "logp_value"),
+                                           opt_dev_ptr<float>(logits, at::kFloat, device, 6 * n(), "logits"),
+                                           dev_ptr<uint8_t>(stack_out, at::kByte, device, n() * 2 * 4 * 42 * 42, "stack_out"),
+                                           stream_of(device)));
+    }
     // [P * 4]: episodes, wins, draws, losses of seat 0 per pairing
     std::vector<uint64_t> pair_stats(int64_t num_pairs) {
         TORCH_CHECK(num_pairs >= 1 && num_pairs <= CRL_PONG_OPP_MAX_PAIRS, "num_pairs must be in [1, ", CRL_PONG_OPP_MAX_PAIRS, "]");
@@ -431,6 +450,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
     m.attr("OPP_RULE_BASED") = CRL_PONG_OPP_RULE_BASED;
     m.attr("OPP_RANDOM") = CRL_PONG_OPP_RANDOM;
     m.attr("OPP_MAX_PAIRS") = CRL_PONG_OPP_MAX_PAIRS;
+    m.attr("OPP_LEARNER") = CRL_PONG_OPP_LEARNER;
     py::class_<PongOpponents>(m, "PongOpponents")
         .def(py::init<int64_t, int64_t, uint64_t, int64_t>())
         .def("close", &PongOpponents::close)
@@ -446,5 +466,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
         .def("act_pairs", &PongOpponents::act_pairs)
         .def("pair_stats", &PongOpponents::pair_stats)
         .def("load_learner", &PongOpponents::load_learner)
-        .def("act_learner", &PongOpponents::act_learner);
+        .def("act_learner", &PongOpponents::act_learner)
+        .def("set_selfplay", &PongOpponents::set_selfplay)
+        .def("act_selfplay", &PongOpponents::act_selfplay);
 }

@@ -23,6 +23,11 @@
 // like a ninth slot, run for every env of the chunk after the pool's slots.  It acts on a FrameStackTensor ring of agent
 // 0's frames (zeroed on done), samples its action from the softmax of its logits (or takes the argmax) and writes what
 // a PPO rollout stores: the action, its log-probability, the value and the stack it acted on.
+//
+// Self-play mode (crl_pong_opp_set_selfplay / crl_pong_opp_act_selfplay) is the two-seat kernel with LEARNER set: league
+// mode in which a pairing's seat may be the learner instead of a pool entry.  The per-env thread files learner seats in a
+// ninth work list, so the learner's image is still staged once per 64-env chunk, and the learner acts on that seat's own
+// ring with learner mode's zeroing and sampling (seat 1 draws from a Philox stream of its own).
 #include <string.h>
 
 #include <cmath>
@@ -77,13 +82,21 @@ struct Smem {
     static constexpr int W = 0, X = W + (LEARNER ? NET_LRN : NET_DEV), HID = X + STACK * FRAME, LUT = HID + C1 * H1 * H1,
                          RS = LEARNER ? 4 : 3, RED = LUT + 256, FLOATS = RED + 8 * RS;
 };
-// + the work list uint8 [slot][SEATS * SUB] and its counts int [16]
+// + the work list uint8 [slot][SEATS * SUB] and its counts int [16]; self-play (SEATS == 2, LEARNER) adds a ninth list,
+// the learner's, and a byte per env of the chunk: bit `seat` set = zero that seat's ring before the push
+template <int SEATS, bool LEARNER>
+__host__ __device__ constexpr int work_lists() { return CRL_PONG_OPP_SLOTS + (SEATS == 2 && LEARNER ? 1 : 0); }
 template <int SEATS, bool LEARNER = false>
-constexpr size_t smem_bytes() { return Smem<LEARNER>::FLOATS * sizeof(float) + CRL_PONG_OPP_SLOTS * SUB * SEATS + 16 * sizeof(int); }
+constexpr size_t smem_bytes() {
+    return Smem<LEARNER>::FLOATS * sizeof(float) + work_lists<SEATS, LEARNER>() * SUB * SEATS + 16 * sizeof(int) +
+           (SEATS == 2 && LEARNER ? SUB : 0);
+}
 constexpr size_t SMEM_BYTES = smem_bytes<1>();
 static_assert(SUB <= 64, "a league work item is (env in chunk) | seat << 6");
 
 constexpr int KIND_RULE = CRL_PONG_OPP_RULE_BASED;   // CRL_PONG_OPP_RANDOM is the other negative kind
+constexpr uint8_t PAIR_LEARNER = 255;                 // a learner seat (CRL_PONG_OPP_LEARNER) in the uint8 pairing table
+static_assert(CRL_PONG_OPP_MAX_POOL < PAIR_LEARNER, "pool indices and the learner sentinel are distinct");
 
 struct OppArgs {
     int n;
@@ -114,13 +127,17 @@ struct OppArgs {
     // learner mode only (SEATS == 1, LEARNER): obs0 and stack0 above are agent 0's frames and the learner's ring
     int sample;               // != 0: sample the action from the softmax, else the argmax
     const float* learner;     // [NET_LRN]
-    float* logp_value;        // [n][2]
+    float* logp_value;        // [n][2] (self-play: [n][2][2])
     float* learner_logits;    // [n][3] or nullptr
-    uint8_t* stack_out;       // [n][4][1764] the stack the learner acted on, oldest -> newest
+    uint8_t* stack_out;       // [n][4][1764] the stack the learner acted on, oldest -> newest (self-play: [n][2][4][1764])
+    // self-play mode only (SEATS == 2, LEARNER): pairs[p][seat] == PAIR_LEARNER is a learner seat, whose logits go to
+    // `logits` [n][2][3] like a pool network's
+    int clear_rings;          // != 0: every learner seat's ring is zeroed before this act's push (a restart)
 };
 
 // Philox streams: (global env, tag) x counter, keyed by the seed.  tag 1 = RANDOM's actions (seat 1), tag 2 = opponent
-// draws, tag 3 = RANDOM's actions in seat 0 (league mode), tag 4 = the learner's sampled actions (learner mode).
+// draws, tag 3 = RANDOM's actions in seat 0 (league mode), tag 4 = the learner's sampled actions (learner mode, and seat 0
+// in self-play mode), tag 5 = the learner's sampled actions in seat 1 (self-play mode).
 __device__ __forceinline__ uint32_t opp_rand(uint64_t seed, int64_t g, uint32_t tag, uint64_t ctr) {
     uint32_t r[4];
     philox4x32_10((uint32_t)g, (uint32_t)((uint64_t)g >> 32) ^ (tag << 24), (uint32_t)ctr, (uint32_t)(ctr >> 32),
@@ -136,15 +153,18 @@ __device__ __forceinline__ int opp_draw(const OppArgs& a, int64_t g, uint32_t ep
 }
 
 // The learner's outputs from its fp32 logits l and value v (thread 0): the action (a draw u = r32 * 2^-32 from the tag 4
-// stream, the first k with u < c_k of the cumulative softmax, or the argmax), log pi(action) and the value.
-__device__ __forceinline__ void learner_out(const OppArgs& a, int i, const float (&l)[3], float v) {
+// stream, or tag 5 for seat 1 in self-play, the first k with u < c_k of the cumulative softmax, or the argmax),
+// log pi(action) and the value.  SEATS == 1: seat 0 of learner mode; SEATS == 2: `seat` of self-play mode.
+template <int SEATS>
+__device__ __forceinline__ void learner_out(const OppArgs& a, int i, int seat, const float (&l)[3], float v) {
     const float mx = fmaxf(fmaxf(l[0], l[1]), l[2]);
     const float e0 = expf(l[0] - mx), e1 = expf(l[1] - mx), e2 = expf(l[2] - mx);
     const float s = (e0 + e1) + e2;
     int act = 0;
     if (a.sample) {
         const float c0 = e0 / s, c1 = c0 + e1 / s;   // action 2 takes the rest, whatever c_2 rounds to
-        const double u = (double)opp_rand(a.seed, a.first_env + i, 4u, a.step) * 0x1p-32;   // exact, and so is the compare
+        const uint32_t tag = SEATS == 1 || seat == 0 ? 4u : 5u;
+        const double u = (double)opp_rand(a.seed, a.first_env + i, tag, a.step) * 0x1p-32;   // exact, and so is the compare
         act = u < (double)c0 ? 0 : u < (double)c1 ? 1 : 2;
     } else {
         float best = l[0];                     // argmax, ties to the lowest index
@@ -152,22 +172,26 @@ __device__ __forceinline__ void learner_out(const OppArgs& a, int i, const float
         if (l[2] > best) act = 2;
     }
     const float la = act == 0 ? l[0] : act == 1 ? l[1] : l[2];
-    a.logp_value[2 * i] = la - (mx + logf(s));   // log softmax: l_a - logsumexp(l)
-    a.logp_value[2 * i + 1] = v;
-    a.actions[2 * i] = act;
-    if (a.learner_logits) {
-        float* lg = a.learner_logits + 3 * i;
+    const int o = SEATS == 1 ? i : 2 * i + seat;   // the (env, seat) row
+    a.logp_value[2 * o] = la - (mx + logf(s));   // log softmax: l_a - logsumexp(l)
+    a.logp_value[2 * o + 1] = v;
+    a.actions[SEATS == 1 ? 2 * i : o] = act;
+    float* const lgs = SEATS == 1 ? a.learner_logits : a.logits;
+    if (lgs) {
+        float* lg = lgs + 3 * o;
         lg[0] = l[0]; lg[1] = l[1]; lg[2] = l[2];
     }
 }
 
 // SEATS == 1: column 1 of the step buffer (the per-env opponents); SEATS == 2: both columns (league mode).
-// LEARNER (SEATS == 1 only): column 0 too, from the learner's network (learner mode).
+// LEARNER, SEATS == 1: column 0 too, from the learner's network (learner mode).
+// LEARNER, SEATS == 2: a seat of any pairing may be the learner's (self-play mode).
 template <int SEATS, bool LEARNER>
 __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs a) {
-    static_assert(!LEARNER || SEATS == 1, "the learner plays seat 0 of the one-seat kernel");
     using L = Smem<LEARNER>;
+    constexpr bool SELF = SEATS == 2 && LEARNER;
     constexpr int NS = CRL_PONG_OPP_SLOTS + (LEARNER ? 1 : 0);   // the learner is slot CRL_PONG_OPP_SLOTS
+    constexpr int NL = work_lists<SEATS, LEARNER>();
     extern __shared__ __align__(16) float sm[];
     float* const w = sm + L::W;
     float* const xs = sm + L::X;
@@ -176,14 +200,15 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
     float* const lut = sm + L::LUT;
     float* const red = sm + L::RED;
     uint8_t* const list = (uint8_t*)(sm + L::FLOATS);                     // [slot][SEATS * SUB]
-    int* const cnt = (int*)(list + CRL_PONG_OPP_SLOTS * SUB * SEATS);   // [slot]
+    int* const cnt = (int*)(list + NL * SUB * SEATS);                   // [slot]
+    uint8_t* const zero = (uint8_t*)(cnt + 16);                          // self-play: [SUB] rings to zero, bit per seat
     const int tid = threadIdx.x;
 
     for (int b = tid; b < 256; b += THREADS) lut[b] = (float)b / 255.0f;
     const int r0 = (int)((int64_t)a.n * blockIdx.x / gridDim.x), r1 = (int)((int64_t)a.n * (blockIdx.x + 1) / gridDim.x);
     for (int e0 = r0; e0 < r1; e0 += SUB) {
         const int ne = min(SUB, r1 - e0);
-        if (tid < CRL_PONG_OPP_SLOTS) cnt[tid] = 0;
+        if (tid < NL) cnt[tid] = 0;
         __syncthreads();
         // ---- per env: bookkeeping of the step before, redraw, actions of the non-network kinds, sort by slot
         if (SEATS == 1 && tid < ne) {
@@ -231,8 +256,15 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
                 }
                 a.ret[i] = r;
             }
+            int zm = 0;
 #pragma unroll
             for (int seat = 0; seat < 2; ++seat) {
+                if (SELF && a.pairs[p][seat] == PAIR_LEARNER) {   // before kind[] is indexed
+                    list[CRL_PONG_OPP_SLOTS * 2 * SUB + atomicAdd(&cnt[CRL_PONG_OPP_SLOTS], 1)] = (uint8_t)(tid | seat << 6);
+                    if (a.clear_rings || (a.done && a.done[i])) zm |= 1 << seat;
+                    continue;
+                }
+                if (SELF) a.logp_value[4 * i + 2 * seat] = a.logp_value[4 * i + 2 * seat + 1] = 0.f;
                 const int kind = a.kind[a.pairs[p][seat]];
                 if (kind >= 0) {
                     list[kind * 2 * SUB + atomicAdd(&cnt[kind], 1)] = (uint8_t)(tid | seat << 6);
@@ -246,9 +278,12 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
                     }
                 }
             }
+            if (SELF) zero[tid] = (uint8_t)zm;
         }
+        if (SELF) __syncthreads();   // the push below reads `zero`
         // ---- the newest frame into ring slot `phase` of every env of the range (league: of both seats' stacks;
-        //      learner: of both, and an env whose previous step ended has its learner ring zeroed first)
+        //      learner: of both, and an env whose previous step ended has its learner ring zeroed first; self-play: of
+        //      both, and a learner seat's ring is zeroed first after a done or a restart)
 #pragma unroll
         for (int seat = SEATS == 2 || LEARNER ? 0 : 1; seat < 2; ++seat) {
             const uint32_t* src = (const uint32_t*)((seat ? a.obs1 : a.obs0) + (size_t)e0 * FRAME);
@@ -256,8 +291,8 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
             for (int k = tid; k < ne * FRAME_WORDS; k += THREADS) {
                 const int e = k / FRAME_WORDS, j = k - e * FRAME_WORDS;
                 dst[(size_t)e * STACK * FRAME_WORDS + j] = src[k];
-                if (LEARNER && seat == 0 && a.done && a.done[e0 + e]) {
-                    uint32_t* ring = (uint32_t*)(a.stack0 + (size_t)(e0 + e) * STACK * FRAME);
+                if (LEARNER && (SELF ? (zero[e] >> seat & 1) != 0 : seat == 0 && a.done && a.done[e0 + e])) {
+                    uint32_t* ring = (uint32_t*)((seat ? a.stack : a.stack0) + (size_t)(e0 + e) * STACK * FRAME);
 #pragma unroll
                     for (int d = 1; d < STACK; ++d) ring[((a.phase + d) & 3) * FRAME_WORDS + j] = 0u;
                 }
@@ -267,7 +302,7 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
         // ---- networks, slot by slot (learner mode: then the learner, for every env of the range)
         for (int s = 0; s < NS; ++s) {
             const bool lrn = LEARNER && s == CRL_PONG_OPP_SLOTS;
-            const int m = lrn ? ne : cnt[s];
+            const int m = lrn && !SELF ? ne : cnt[s];
             if (m == 0) continue;
             if (lrn) {
                 const float4* src = (const float4*)a.learner;
@@ -277,15 +312,15 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
                 for (int k = tid; k < NET_DEV / 4; k += THREADS) ((float4*)w)[k] = src[k];
             }
             for (int q = 0; q < m; ++q) {
-                const int item = lrn ? q : list[s * SEATS * SUB + q];
+                const int item = lrn && !SELF ? q : list[s * SEATS * SUB + q];
                 const int i = e0 + (SEATS == 1 ? item : item & (SUB - 1));
-                const int seat = lrn ? 0 : SEATS == 1 ? 1 : item >> 6;
+                const int seat = lrn && !SELF ? 0 : SEATS == 1 ? 1 : item >> 6;
                 {   // stack / 255 -> xs[ci][42][42], ci 0 = oldest (the learner's bytes also go to stack_out)
                     const uint32_t* src = (const uint32_t*)(((SEATS == 1 && !LEARNER) || seat ? a.stack : a.stack0) + (size_t)i * STACK * FRAME);
                     for (int k = tid; k < STACK * FRAME_WORDS; k += THREADS) {
                         const int ci = k / FRAME_WORDS, j = k - ci * FRAME_WORDS;
                         const uint32_t v = src[((a.phase + 1 + ci) & 3) * FRAME_WORDS + j];
-                        if (lrn) ((uint32_t*)a.stack_out)[(size_t)i * STACK * FRAME_WORDS + k] = v;
+                        if (lrn) ((uint32_t*)a.stack_out)[(size_t)(SELF ? 2 * i + seat : i) * STACK * FRAME_WORDS + k] = v;
                         float4 f;
                         f.x = lut[v & 255]; f.y = lut[(v >> 8) & 255]; f.z = lut[(v >> 16) & 255]; f.w = lut[v >> 24];
                         *(float4*)&xs[ci * FRAME + 4 * j] = f;
@@ -382,7 +417,7 @@ __global__ void __launch_bounds__(THREADS, 2) pong_opp_act_kernel(const OppArgs 
                     if (lrn) {
                         float v = 0.f;
                         for (int wi = 0; wi < THREADS / 32; ++wi) v += red[L::RS * wi + 3];
-                        learner_out(a, i, l, v + w[OFF_BC]);
+                        learner_out<SEATS>(a, i, seat, l, v + w[OFF_BC]);
                         continue;      // the rest of this block is a pool network's; thread 0 joins the next barrier
                     }
                     int act = 0;                       // argmax, ties to the lowest index
@@ -413,7 +448,7 @@ __global__ void pong_opp_draw_kernel(const OppArgs a) {
 using namespace crl::opp;
 
 struct crl_pong_opp {
-    int n = 0, device = 0, grid = 0, grid_league = 0, grid_learner = 0;
+    int n = 0, device = 0, grid = 0, grid_league = 0, grid_learner = 0, grid_selfplay = 0;
     uint64_t seed = 0;
     int64_t first_env = 0;
     uint64_t steps = 0;
@@ -440,7 +475,12 @@ struct crl_pong_opp {
     bool learner = false;
     bool learner_loaded = false;
     float* learner_net = nullptr;              // [NET_LRN]
+    // self-play mode: league mode's pairings (a learner seat is PAIR_LEARNER), stacks and statistics
+    bool selfplay = false;
+    bool clear_rings = false;                  // a restart is pending: the next act zeroes every learner seat's ring
 };
+
+static const char* const SELFPLAY_REFUSAL = "self-play mode: use crl_pong_opp_act_selfplay (crl_pong_opp_set_pool leaves it)";
 
 static OppArgs opp_args(const crl_pong_opp* h) {
     OppArgs a;
@@ -472,7 +512,7 @@ int crl_pong_opp_create(int32_t num_envs, int32_t device, uint64_t seed, int64_t
     crl_pong_opp* h = new crl_pong_opp();
     h->n = num_envs; h->device = device; h->seed = seed; h->first_env = first_env;
     const size_t n = (size_t)num_envs;
-    int sms = 0, per_sm = 0, per_sm_league = 0, per_sm_learner = 0;
+    int sms = 0, per_sm = 0, per_sm_league = 0, per_sm_learner = 0, per_sm_selfplay = 0;
     cudaError_t err = cudaSuccess;
     auto alloc = [&](auto** p, size_t count) { if (err == cudaSuccess) err = h->allocs.alloc(p, count); };
     alloc(&h->nets, (size_t)NET_DEV * CRL_PONG_OPP_SLOTS);
@@ -485,6 +525,9 @@ int crl_pong_opp_create(int32_t num_envs, int32_t device, uint64_t seed, int64_t
     if (err == cudaSuccess)
         err = cudaFuncSetAttribute(pong_opp_act_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    (int)smem_bytes<1, true>());
+    if (err == cudaSuccess)
+        err = cudaFuncSetAttribute(pong_opp_act_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)smem_bytes<2, true>());
     if (err == cudaSuccess) err = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
     if (err == cudaSuccess) err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pong_opp_act_kernel<1, false>, THREADS, SMEM_BYTES);
     if (err == cudaSuccess)
@@ -492,6 +535,9 @@ int crl_pong_opp_create(int32_t num_envs, int32_t device, uint64_t seed, int64_t
     if (err == cudaSuccess)
         err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_learner, pong_opp_act_kernel<1, true>, THREADS,
                                                             smem_bytes<1, true>());
+    if (err == cudaSuccess)
+        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_selfplay, pong_opp_act_kernel<2, true>, THREADS,
+                                                            smem_bytes<2, true>());
     if (err == cudaSuccess) err = cudaDeviceSynchronize();
     if (err != cudaSuccess) {
         crl_pong_opp_destroy(h);
@@ -501,6 +547,7 @@ int crl_pong_opp_create(int32_t num_envs, int32_t device, uint64_t seed, int64_t
     h->grid = (int)std::min<int64_t>((int64_t)std::max(per_sm, 1) * sms, num_envs);
     h->grid_league = (int)std::min<int64_t>((int64_t)std::max(per_sm_league, 1) * sms, num_envs);
     h->grid_learner = (int)std::min<int64_t>((int64_t)std::max(per_sm_learner, 1) * sms, num_envs);
+    h->grid_selfplay = (int)std::min<int64_t>((int64_t)std::max(per_sm_selfplay, 1) * sms, num_envs);
     *out = h;
     return CRL_OK;
 }
@@ -581,8 +628,10 @@ int crl_pong_opp_set_pool(crl_pong_opp* h, const int32_t* kinds_host, const doub
     h->assigned = false;
     h->learner = false;
     CUDA_TRY(cudaMemsetAsync(h->stats, 0, sizeof(unsigned long long) * 4 * CRL_PONG_OPP_MAX_POOL, (cudaStream_t)stream));
-    if (h->league) {   // leaving league mode: the per-env opponents start as on a fresh handle (the act count runs on)
+    // leaving league or self-play mode: the per-env opponents start as on a fresh handle (the act count runs on)
+    if (h->league || h->selfplay) {
         h->league = false;
+        h->selfplay = false;
         CUDA_TRY(cudaMemsetAsync(h->ret, 0, sizeof(float) * h->n, (cudaStream_t)stream));
         CUDA_TRY(cudaMemsetAsync(h->stack, 0, (size_t)STACK * FRAME * h->n, (cudaStream_t)stream));
         h->phase = 0;
@@ -615,6 +664,8 @@ int crl_pong_opp_restart(crl_pong_opp* h, int32_t clear_stacks, void* stream) {
         h->phase = 0;
     } else if (h->learner) {   // a reset starts every learner episode afresh (FrameStackTensor.reset)
         CUDA_TRY(cudaMemsetAsync(h->stack0, 0, (size_t)STACK * FRAME * h->n, (cudaStream_t)stream));
+    } else if (h->selfplay) {  // the same for every learner seat; pool seats keep their stacks
+        h->clear_rings = true;
     }
     return CRL_OK;
 }
@@ -624,6 +675,7 @@ int crl_pong_opp_act(crl_pong_opp* h, const uint8_t* obs1_dev, const float* rew_
     CHECK_HANDLE(h, h->device);
     if (h->league) return crl_set_error(CRL_E_STATE, "league mode: use crl_pong_opp_act_pairs (crl_pong_opp_set_pool leaves it)");
     if (h->learner) return crl_set_error(CRL_E_STATE, "learner mode: use crl_pong_opp_act_learner (crl_pong_opp_set_pool leaves it)");
+    if (h->selfplay) return crl_set_error(CRL_E_STATE, SELFPLAY_REFUSAL);
     if (!h->assigned) return crl_set_error(CRL_E_STATE, "crl_pong_opp_assign after every crl_pong_opp_set_pool");
     if (!obs1_dev || !actions_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
     if ((rew_dev == nullptr) != (done_dev == nullptr)) return crl_set_error(CRL_E_INVALID, "rew_dev and done_dev go together");
@@ -637,6 +689,40 @@ int crl_pong_opp_act(crl_pong_opp* h, const uint8_t* obs1_dev, const float* rew_
     return CRL_OK;
 }
 
+// league and self-play modes: pairs_host validated by the caller (a learner seat is CRL_PONG_OPP_LEARNER).  Allocates
+// what the modes share on first use, zeroes the pairing statistics, the reward sums and both stacks of every env, and
+// stores the table; the caller sets the mode.
+static int enter_pairs(crl_pong_opp* h, const int32_t* pairs_host, int32_t num_pairs, void* stream, const char* who) {
+    if (!h->pair_stats) {
+        const bool had_stack0 = h->stack0 != nullptr;   // learner mode came first
+        cudaError_t err = h->allocs.alloc(&h->pair_stats, 4 * CRL_PONG_OPP_MAX_PAIRS);
+        if (err == cudaSuccess && !had_stack0) err = h->allocs.alloc(&h->stack0, (size_t)STACK * FRAME * h->n);
+        if (err != cudaSuccess) {   // both or neither: a failed call leaves the handle as it was
+            h->allocs.free(h->pair_stats);
+            h->pair_stats = nullptr;
+            if (!had_stack0) h->stack0 = nullptr;
+            return crl_set_error(CRL_E_CUDA, "%s: %s", who, cudaGetErrorString(err));
+        }
+    }
+    const cudaStream_t s = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemsetAsync(h->pair_stats, 0, sizeof(unsigned long long) * 4 * CRL_PONG_OPP_MAX_PAIRS, s));
+    CUDA_TRY(cudaMemsetAsync(h->ret, 0, sizeof(float) * h->n, s));
+    CUDA_TRY(cudaMemsetAsync(h->stack, 0, (size_t)STACK * FRAME * h->n, s));
+    CUDA_TRY(cudaMemsetAsync(h->stack0, 0, (size_t)STACK * FRAME * h->n, s));
+    for (int p = 0; p < CRL_PONG_OPP_MAX_PAIRS; ++p)
+        for (int seat = 0; seat < 2; ++seat) {
+            const int32_t v = p < num_pairs ? pairs_host[2 * p + seat] : 0;
+            h->pairs[p][seat] = v == CRL_PONG_OPP_LEARNER ? PAIR_LEARNER : (uint8_t)v;
+        }
+    h->num_pairs = num_pairs;
+    h->phase = 0;
+    h->league = false;
+    h->learner = false;
+    h->selfplay = false;
+    h->clear_rings = false;
+    return CRL_OK;
+}
+
 int crl_pong_opp_set_pairs(crl_pong_opp* h, const int32_t* pairs_host, int32_t num_pairs, void* stream) {
     CHECK_HANDLE(h, h->device);
     if (h->pool_size == 0) return crl_set_error(CRL_E_STATE, "crl_pong_opp_set_pool first");
@@ -647,34 +733,33 @@ int crl_pong_opp_set_pairs(crl_pong_opp* h, const int32_t* pairs_host, int32_t n
             if (pairs_host[2 * p + seat] < 0 || pairs_host[2 * p + seat] >= h->pool_size)
                 return crl_set_error(CRL_E_INVALID, "pairing %d, seat %d: pool index %d is not in [0, %d)", p, seat,
                                      pairs_host[2 * p + seat], h->pool_size);
-    if (!h->pair_stats) {
-        const bool had_stack0 = h->stack0 != nullptr;   // learner mode came first
-        cudaError_t err = h->allocs.alloc(&h->pair_stats, 4 * CRL_PONG_OPP_MAX_PAIRS);
-        if (err == cudaSuccess && !had_stack0) err = h->allocs.alloc(&h->stack0, (size_t)STACK * FRAME * h->n);
-        if (err != cudaSuccess) {   // both or neither: a failed call leaves the handle as it was
-            h->allocs.free(h->pair_stats);
-            h->pair_stats = nullptr;
-            if (!had_stack0) h->stack0 = nullptr;
-            return crl_set_error(CRL_E_CUDA, "crl_pong_opp_set_pairs: %s", cudaGetErrorString(err));
-        }
-    }
-    const cudaStream_t s = (cudaStream_t)stream;
-    CUDA_TRY(cudaMemsetAsync(h->pair_stats, 0, sizeof(unsigned long long) * 4 * CRL_PONG_OPP_MAX_PAIRS, s));
-    CUDA_TRY(cudaMemsetAsync(h->ret, 0, sizeof(float) * h->n, s));
-    CUDA_TRY(cudaMemsetAsync(h->stack, 0, (size_t)STACK * FRAME * h->n, s));
-    CUDA_TRY(cudaMemsetAsync(h->stack0, 0, (size_t)STACK * FRAME * h->n, s));
-    for (int p = 0; p < CRL_PONG_OPP_MAX_PAIRS; ++p)
-        for (int seat = 0; seat < 2; ++seat) h->pairs[p][seat] = p < num_pairs ? (uint8_t)pairs_host[2 * p + seat] : 0;
-    h->num_pairs = num_pairs;
-    h->phase = 0;
+    if (int r = enter_pairs(h, pairs_host, num_pairs, stream, "crl_pong_opp_set_pairs")) return r;
     h->league = true;
-    h->learner = false;
+    return CRL_OK;
+}
+
+int crl_pong_opp_set_selfplay(crl_pong_opp* h, const int32_t* pairs_host, int32_t num_pairs, void* stream) {
+    CHECK_HANDLE(h, h->device);
+    if (h->pool_size == 0) return crl_set_error(CRL_E_STATE, "crl_pong_opp_set_pool first");
+    if (!pairs_host || num_pairs < 1 || num_pairs > CRL_PONG_OPP_MAX_PAIRS)
+        return crl_set_error(CRL_E_INVALID, "a self-play table has 1 to %d pairings", CRL_PONG_OPP_MAX_PAIRS);
+    for (int p = 0; p < num_pairs; ++p)
+        for (int seat = 0; seat < 2; ++seat) {
+            const int32_t v = pairs_host[2 * p + seat];
+            if (v != CRL_PONG_OPP_LEARNER && (v < 0 || v >= h->pool_size))
+                return crl_set_error(CRL_E_INVALID,
+                                     "pairing %d, seat %d: %d is neither CRL_PONG_OPP_LEARNER nor a pool index in [0, %d)",
+                                     p, seat, v, h->pool_size);
+        }
+    if (int r = enter_pairs(h, pairs_host, num_pairs, stream, "crl_pong_opp_set_selfplay")) return r;
+    h->selfplay = true;
     return CRL_OK;
 }
 
 int crl_pong_opp_act_pairs(crl_pong_opp* h, const uint8_t* obs0_dev, const uint8_t* obs1_dev, const float* rew_dev,
                            const uint8_t* done_dev, int32_t* actions_dev, float* logits_dev, void* stream) {
     CHECK_HANDLE(h, h->device);
+    if (h->selfplay) return crl_set_error(CRL_E_STATE, SELFPLAY_REFUSAL);
     if (!h->league) return crl_set_error(CRL_E_STATE, "crl_pong_opp_set_pairs first (league mode)");
     if (!obs0_dev || !obs1_dev || !actions_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
     if ((rew_dev == nullptr) != (done_dev == nullptr)) return crl_set_error(CRL_E_INVALID, "rew_dev and done_dev go together");
@@ -698,6 +783,7 @@ int crl_pong_opp_act_learner(crl_pong_opp* h, const uint8_t* obs0_dev, const uin
     CHECK_HANDLE(h, h->device);
     if (!h->learner_loaded) return crl_set_error(CRL_E_STATE, "crl_pong_opp_load_learner first");
     if (h->league) return crl_set_error(CRL_E_STATE, "league mode: use crl_pong_opp_act_pairs (crl_pong_opp_set_pool leaves it)");
+    if (h->selfplay) return crl_set_error(CRL_E_STATE, SELFPLAY_REFUSAL);
     if (!h->assigned) return crl_set_error(CRL_E_STATE, "crl_pong_opp_assign after every crl_pong_opp_set_pool");
     if (!obs0_dev || !obs1_dev || !actions_dev || !logp_value_dev || !stack_out_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
     if ((rew_dev == nullptr) != (done_dev == nullptr)) return crl_set_error(CRL_E_INVALID, "rew_dev and done_dev go together");
@@ -722,6 +808,33 @@ int crl_pong_opp_act_learner(crl_pong_opp* h, const uint8_t* obs0_dev, const uin
     a.rew = rew_dev; a.done = done_dev; a.actions = actions_dev;
     a.logp_value = logp_value_dev; a.learner_logits = logits_dev; a.stack_out = stack_out_dev;
     LAUNCH((pong_opp_act_kernel<1, true><<<h->grid_learner, THREADS, smem_bytes<1, true>(), s>>>(a), cudaGetLastError()), 1);
+    h->phase = (h->phase + 1) & 3;
+    h->steps += 1;
+    return CRL_OK;
+}
+
+int crl_pong_opp_act_selfplay(crl_pong_opp* h, const uint8_t* obs0_dev, const uint8_t* obs1_dev, const float* rew_dev,
+                              const uint8_t* done_dev, int32_t sample, int32_t* actions_dev, float* logp_value_dev,
+                              float* logits_dev, uint8_t* stack_out_dev, void* stream) {
+    CHECK_HANDLE(h, h->device);
+    if (!h->selfplay) return crl_set_error(CRL_E_STATE, "crl_pong_opp_set_selfplay first (self-play mode)");
+    if (!h->learner_loaded) return crl_set_error(CRL_E_STATE, "crl_pong_opp_load_learner first");
+    if (!obs0_dev || !obs1_dev || !actions_dev || !logp_value_dev || !stack_out_dev) return crl_set_error(CRL_E_INVALID, "null buffer");
+    if ((rew_dev == nullptr) != (done_dev == nullptr)) return crl_set_error(CRL_E_INVALID, "rew_dev and done_dev go together");
+    if (((uintptr_t)obs0_dev & 3) != 0 || ((uintptr_t)obs1_dev & 3) != 0 || ((uintptr_t)stack_out_dev & 3) != 0)
+        return crl_set_error(CRL_E_INVALID, "obs0_dev, obs1_dev and stack_out_dev must be 4-byte aligned");
+    OppArgs a = opp_args(h);
+    a.stats = h->pair_stats;
+    a.num_pairs = h->num_pairs;
+    memcpy(a.pairs, h->pairs, sizeof a.pairs);
+    a.sample = sample ? 1 : 0;
+    a.clear_rings = h->clear_rings ? 1 : 0;
+    a.obs0 = obs0_dev; a.obs1 = obs1_dev; a.stack0 = h->stack0; a.learner = h->learner_net;
+    a.rew = rew_dev; a.done = done_dev; a.actions = actions_dev; a.logits = logits_dev;
+    a.logp_value = logp_value_dev; a.stack_out = stack_out_dev;
+    LAUNCH((pong_opp_act_kernel<2, true><<<h->grid_selfplay, THREADS, smem_bytes<2, true>(), (cudaStream_t)stream>>>(a),
+            cudaGetLastError()), 1);
+    h->clear_rings = false;
     h->phase = (h->phase + 1) & 3;
     h->steps += 1;
     return CRL_OK;

@@ -58,7 +58,7 @@ def evaluate_pool_in_batch(pool, envs, episodes_per_pair, pairs=None, networks=N
     row = seat 0's entry, column = seat 1's, counted from seat 0's side (> 0, == 0, < 0 summed clipped reward, as in
     evaluate_two_policies_in_batch); repeated pairings add up, pairings not played are 0."""
     from . import _native
-    from .builtin_policies import pack_light_actor_critic, resolve_pool
+    from .builtin_policies import pack_light_actor_critic, resolve_pairs, resolve_pool
     if envs.dim != 42 or envs.c != 1 or envs.f32 or envs.ring or getattr(envs, "n_agents", 2) != 2:
         raise ValueError("league evaluation needs a cPongDouble env with resized_dim=42, frame_stack=None and uint8 "
                          "observations")
@@ -74,21 +74,8 @@ def evaluate_pool_in_batch(pool, envs, episodes_per_pair, pairs=None, networks=N
     m = len(pool)
     if pairs is None:
         pairs = [(a, b) for a in range(m) for b in range(m)]
-    idx = []
-    for pr in pairs:
-        pr = list(pr)
-        if len(pr) != 2:
-            raise ValueError("a pairing is (seat 0, seat 1)")
-        for x in pr:
-            if isinstance(x, str) and x not in pool:
-                raise ValueError("pairing %r: %r is not in the pool" % (tuple(pr), x))
-        k = [pool.index(x) if isinstance(x, str) else int(x) for x in pr]
-        if not all(0 <= v < m for v in k):
-            raise ValueError("pairing %r: pool indices must be in [0, %d)" % (tuple(pr), m))
-        idx.append(k)
+    idx = resolve_pairs(pairs, pool)
     p = len(idx)
-    if not 1 <= p <= ext.OPP_MAX_PAIRS:
-        raise ValueError("a league has 1 to %d pairings (got %d)" % (ext.OPP_MAX_PAIRS, p))
     n = envs.num_envs
     if n < p:
         raise ValueError("%d pairings need at least as many envs (got %d)" % (p, n))

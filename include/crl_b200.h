@@ -283,12 +283,42 @@ int crl_obs_free(void* ptr);
  *               would be missing from the rings.  crl_pong_opp_set_pool and crl_pong_opp_set_pairs leave learner mode;
  *               crl_pong_opp_act_learner returns CRL_E_STATE in league mode, before crl_pong_opp_load_learner and before
  *               crl_pong_opp_assign.  Reloading the learner's weights does not leave learner mode.
+ *
+ * Self-play mode (crl_pong_opp_set_selfplay, crl_pong_opp_act_selfplay): league mode in which any seat of a pairing may
+ * be the learner of learner mode, so one launch per step plays the current policy against itself, frozen snapshots and
+ * built-in opponents, and returns what a PPO rollout stores for every learner seat.
+ *   Pairings    pairs[P][2], 1 <= P <= CRL_PONG_OPP_MAX_PAIRS; each seat is a pool index or CRL_PONG_OPP_LEARNER.  Env
+ *               g = first_env + i plays pairing g mod P for the whole run, as in league mode.  A pairing without a
+ *               learner seat is allowed; its envs play exactly as in league mode.
+ *   Learner     a learner seat runs the learner's image (crl_pong_opp_load_learner), computed as in learner mode: conv1 /
+ *               conv2 / actor / critic in fp32 over stack / 255.  sample != 0: u = r32 * 2^-32 from Philox keyed by
+ *               (seed, global env index, act count), tag 4 (learner mode's stream) in seat 0 and tag 5 in seat 1, and
+ *               learner mode's inverse-CDF rule; sample == 0: the argmax of the logits, ties to the lowest index.
+ *   Pool seats  as in league mode: RULE_BASED 999, RANDOM a draw from tag 3 in seat 0 and tag 1 in seat 1, a network the
+ *               argmax of its logits.
+ *   Rings       the two stacks of league mode, seat 0's fed agent 0's observations and seat 1's agent 1's: every act
+ *               pushes the agent's observation of the previous step.  A learner seat's ring has FrameStackTensor's
+ *               zeroing (when the previous step's done is set, the other three slots are zeroed first); a pool seat's is
+ *               never cleared on done.  crl_pong_opp_set_selfplay zeroes both rings of every env.  crl_pong_opp_restart
+ *               zeroes every learner seat's ring (before the next act's push), whatever clear_stacks; pool seats follow
+ *               league mode's rule (zeroed by clear_stacks != 0 only).
+ *   Episodes    credited per pairing from seat 0's side, as in league mode (crl_pong_opp_get_pair_stats).
+ *   Outputs     both columns of the step buffer; for each learner seat log pi(action) and the value (0 and 0 for a pool
+ *               seat); each seat's logits, learner or pool network (0 for RULE_BASED and RANDOM); for each learner seat
+ *               the stack it acted on, oldest first (a pool seat's rows of stack_out are not written).
+ *   Modes       crl_pong_opp_set_selfplay needs a pool (CRL_E_STATE otherwise), validates every seat and then enters
+ *               self-play mode, allocating seat 0's stacks on first use as crl_pong_opp_set_pairs does.
+ *               crl_pong_opp_act_selfplay returns CRL_E_STATE outside self-play mode and before crl_pong_opp_load_learner.
+ *               In self-play mode crl_pong_opp_act, crl_pong_opp_act_pairs and crl_pong_opp_act_learner return
+ *               CRL_E_STATE.  crl_pong_opp_set_pool and crl_pong_opp_set_pairs leave self-play mode; reloading the
+ *               learner does not.  crl_pong_opp_set_pairs refuses CRL_PONG_OPP_LEARNER.
  * ====================================================================================== */
 #define CRL_PONG_OPP_MAX_POOL 16
 #define CRL_PONG_OPP_SLOTS 8
 #define CRL_PONG_OPP_RULE_BASED (-1)   /* pool entry kinds; 0 .. CRL_PONG_OPP_SLOTS-1 = network slot */
 #define CRL_PONG_OPP_RANDOM (-2)
 #define CRL_PONG_OPP_MAX_PAIRS 256    /* pairings of league mode */
+#define CRL_PONG_OPP_LEARNER (-3)     /* a learner seat of a self-play pairing */
 /* LightActorCritic parameters in state-dict order, each row-major: conv1.weight [16][4][4][4], conv1.bias [16],
  * conv2.weight [16][16][2][2], conv2.bias [16], critic_linear.weight [1][1600], critic_linear.bias [1],
  * actor_linear.weight [3][1600], actor_linear.bias [3] (the critic is evaluated for the learner only) */
@@ -356,6 +386,21 @@ int crl_pong_opp_load_learner(crl_pong_opp* h, const float* params_host, size_t 
 int crl_pong_opp_act_learner(crl_pong_opp* h, const uint8_t* obs0_dev, const uint8_t* obs1_dev, const float* rew_dev,
                              const uint8_t* done_dev, int32_t resample, int32_t sample, int32_t* actions_dev,
                              float* logp_value_dev, float* logits_dev, uint8_t* stack_out_dev, void* stream);
+/* Enters (or re-enters) self-play mode: pairs_host int32 [num_pairs][2], each seat a pool index or CRL_PONG_OPP_LEARNER,
+ * every one validated (CRL_E_STATE without a pool).  Zeroes the pairing statistics, the per-env reward sums and both
+ * stacks of every env, and restarts the ring, as crl_pong_opp_set_pairs does. */
+int crl_pong_opp_set_selfplay(crl_pong_opp* h, const int32_t* pairs_host, int32_t num_pairs, void* stream);
+/* One self-play step, before crl_pong_step (see above):
+ *   obs0_dev, obs1_dev  uint8 [num_envs][42][42] agent 0's and agent 1's observations of the previous step, 4-byte aligned
+ *   rew_dev, done_dev   as crl_pong_opp_act (both NULL for the first act after a reset)
+ *   sample              != 0: sample the learner seats' actions from their softmax; 0: the argmax
+ *   actions_dev         int32 [num_envs][2]: both columns
+ *   logp_value_dev      float32 [num_envs][2][2]: per seat log pi(action), value (0, 0 for a pool seat)
+ *   logits_dev          float32 [num_envs][2][3] or NULL: each seat's logits (0 for RULE_BASED and RANDOM)
+ *   stack_out_dev       uint8 [num_envs][2][4][42][42], 4-byte aligned: each learner seat's stack, oldest first */
+int crl_pong_opp_act_selfplay(crl_pong_opp* h, const uint8_t* obs0_dev, const uint8_t* obs1_dev, const float* rew_dev,
+                              const uint8_t* done_dev, int32_t sample, int32_t* actions_dev, float* logp_value_dev,
+                              float* logits_dev, uint8_t* stack_out_dev, void* stream);
 
 /* ======================================================================================
  * cCarRacing-v0 / cCarRacingDouble-v0
